@@ -39,7 +39,7 @@ namespace dh {
 constexpr int kPlanThreads = 1024;
 constexpr int kPlanWarps = kPlanThreads / 32;
 constexpr int kPlanTab = 1024;          // per-warp counter table: source cells lo .. lo + 1023 of one destination bucket per pass
-constexpr int kLenClasses = 256;        // rows are ordered by min(length, 255), descending
+constexpr int kLenClasses = 256;        // rows are bucketed by min(length, 255), descending (class 255 is then ranked exactly)
 
 __global__ void __launch_bounds__(kPlanThreads) loss_plan_kernel(
     const int32_t* __restrict__ fg_src, const int32_t* __restrict__ fg_dst, int n_fg,
@@ -177,6 +177,27 @@ __global__ void __launch_bounds__(kPlanThreads) loss_plan_kernel(
         __syncwarp();
     }
     __syncthreads();
+    {   // the rows of class 255 (255 or more entries) lead the order in raster order: rank them by their exact length so that
+        // the whole order is descending, which plan_ent_cap relies on.  Such rows need a multiplicity split or more than
+        // 255 distinct sources, so there are at most n_fg / 255 of them (none in the plans of rigid edits).
+        int n_big = 0;
+        for (int w = 0; w < kPlanWarps; ++w) n_big += whist[w * kLenClasses + kLenClasses - 1];
+        if (n_big > 1) {
+            int* big = reinterpret_cast<int*>(tabs) + 2 * kPlanWarps * kLenClasses;      // (is_src below reuses it)
+            for (int r = tid; r < n_big; r += kPlanThreads) big[r] = order[r];
+            __syncthreads();
+            for (int r = tid; r < n_big; r += kPlanThreads) {
+                const int cell = big[r], len = ucount[cell];
+                int rank = 0;
+                for (int j = 0; j < n_big; ++j) {
+                    const int lj = ucount[big[j]];
+                    rank += (lj > len || (lj == len && j < r)) ? 1 : 0;
+                }
+                order[rank] = cell;
+            }
+            __syncthreads();
+        }
+    }
     {   // slice widths (longest row of the slice) and their exclusive scan
         int w = 0;
         if (tid < n_slices)
@@ -186,6 +207,9 @@ __global__ void __launch_bounds__(kPlanThreads) loss_plan_kernel(
         if (tid == 0) { soff[n_slices] = total; pv.ell_off[n_slices] = total; }
     }
     const int n_groups = total;
+    // the table must fit the space plan_layout reserved for it; if it ever does not, nothing is written to `ent` and the header
+    // flags the plan as unusable (dh_loss_plan_info refuses it)
+    const bool ell_fits = (size_t)n_groups * 32 <= plan_ent_cap(grid, n_fg);
     __syncthreads();
     // box of the cells that are the source or the destination of a pair (resized layers work inside it)
     __shared__ int box_sm[4];
@@ -211,7 +235,7 @@ __global__ void __launch_bounds__(kPlanThreads) loss_plan_kernel(
     for (int i = c0; i < c1; ++i)
         if (is_src[i]) { pv.usrc_cell[run] = (uint16_t)i; is_src[i] = ++run; }
     __syncthreads();
-    for (int sl = wid; sl < n_slices; sl += kPlanWarps) {
+    for (int sl = wid; sl < (ell_fits ? n_slices : 0); sl += kPlanWarps) {
         const int r = sl * 32 + lane;
         const int cell = r < n_rows ? order[r] : -1;
         const int len = cell >= 0 ? ucount[cell] : 0;
@@ -270,7 +294,8 @@ __global__ void __launch_bounds__(kPlanThreads) loss_plan_kernel(
         pv.own_masks[tid] = make_uint2(m_ot, m_cr);
     }
     __syncthreads();
-    if (tid == 0) pv.hdr->reserved = nonbin_sm ? 0 : 1;      // bit 0: every background multiplicity is 0 or 1
+    // bit 0: every background multiplicity is 0 or 1; bit 1: the sliced-ELL table did not fit (the plan is unusable)
+    if (tid == 0) pv.hdr->reserved = (nonbin_sm ? 0 : 1) | (ell_fits ? 0 : 2);
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -1069,8 +1094,12 @@ int dh_build_loss_plan(const int32_t* fg_src, const int32_t* fg_dst, int n_fg, c
     DH_REQUIRE(n_fg >= 0 && n_bg_orig >= 0 && n_bg_trans >= 0 && n_bg_common >= 0);
     DH_REQUIRE((fg_src && fg_dst) || n_fg == 0);
     DH_REQUIRE((bg_orig || n_bg_orig == 0) && (bg_trans || n_bg_trans == 0) && (bg_common || n_bg_common == 0));
-    if (plan_bytes < dh_loss_plan_bytes(grid, n_fg) || ws_bytes < dh_loss_plan_workspace_bytes(grid, n_fg)) return DH_ERR_WORKSPACE;
     const int cells = grid * grid;
+    // 16-bit fields of the plan: the per-cell background counts (a list longer than 65535 could repeat one cell that often)
+    // and the row length in row_desc (a row has at most min(n_fg, cells + n_fg / 255) entries)
+    if (n_bg_orig > 65535 || n_bg_trans > 65535 || n_bg_common > 65535) return DH_ERR_UNSUPPORTED;
+    if (std::min<long long>(n_fg, cells + n_fg / 255) > 65535) return DH_ERR_UNSUPPORTED;
+    if (plan_bytes < dh_loss_plan_bytes(grid, n_fg) || ws_bytes < dh_loss_plan_workspace_bytes(grid, n_fg)) return DH_ERR_WORKSPACE;
     size_t smem_ints = (size_t)3 * cells + 1 + (size_t)kPlanWarps * kPlanTab;
     if (smem_ints < (size_t)4 * cells) smem_ints = (size_t)4 * cells;
     const size_t smem = sizeof(int) * smem_ints;
@@ -1112,6 +1141,7 @@ int dh_build_loss_resize_tables(const void* plan, int n_fg, int grid, int h, int
 int dh_loss_plan_info(const void* plan_header_host, dh_loss_plan_desc* desc) {
     DH_REQUIRE(plan_header_host && desc);
     const PlanHeader* h = static_cast<const PlanHeader*>(plan_header_host);
+    if (h->reserved & 2) return DH_ERR_UNSUPPORTED;        // the builder found no room for the sliced-ELL table
     desc->n_pairs = h->n_pairs;
     desc->flags = h->reserved & 1;
     desc->box_cells = h->box_r1 >= h->box_r0 ? (h->box_r1 - h->box_r0 + 1) * (h->box_s1 - h->box_s0 + 1) : 0;

@@ -204,11 +204,15 @@ __global__ void __launch_bounds__(kPatchThreads, 1) loss_patch_kernel(const __gr
 
         // ---- the two maps at the loss-grid resolution ----
         if (native) {
-            for (int q = tid; q < cells / 4; q += kPatchThreads) {
+            // 128-bit accesses only when the planes and the shared-memory maps are 16-byte aligned: with a cell count that is not a
+            // multiple of four, plane c >= 1 and the map u2 (at psm + cells) start at offsets that are not
+            const bool vec = (cells & 3) == 0 && ((reinterpret_cast<uintptr_t>(vc) | reinterpret_cast<uintptr_t>(vo)) & 15) == 0;
+            const int n4 = vec ? cells / 4 : 0;
+            for (int q = tid; q < n4; q += kPatchThreads) {
                 reinterpret_cast<float4*>(u2)[q] = __ldg(reinterpret_cast<const float4*>(vc) + q);
                 reinterpret_cast<float4*>(u1)[q] = __ldg(reinterpret_cast<const float4*>(vo) + q);
             }
-            for (int q = (cells / 4) * 4 + tid; q < cells; q += kPatchThreads) { u2[q] = vc[q]; u1[q] = vo[q]; }
+            for (int q = n4 * 4 + tid; q < cells; q += kPatchThreads) { u2[q] = vc[q]; u1[q] = vo[q]; }
         } else {
             for (int q = tid; q < cells; q += kPatchThreads) {
                 const int Y = q / G, X = q - Y * G;

@@ -34,10 +34,10 @@ struct PlanView {
 
 __host__ __device__ inline size_t plan_ent_cap(int grid, int cap) {
     const size_t cells = (size_t)grid * grid, n = cap > 0 ? (size_t)cap : 1;
-    // sum over slices of 32 * (longest row of the slice) <= n_pairs + 32 * (longest row of all); a row has at most one entry
-    // per source cell plus the entries that a multiplicity > 255 is split into
-    // (+ the padding of every row to a multiple of four entries: at most 3 * 32 per slice)
-    return n + 32 * ((n < cells ? n : cells) + (n >> 8) + 1) + 96 * ((cells + 31) / 32);
+    // rows in descending order of length: sum over slices of 32 * (longest row of the slice) <= n_pairs + 32 * (longest row
+    // of all); a row has at most one entry per source cell plus the entries that multiplicities > 255 are split into
+    // (sum of floor((m - 1) / 255) <= n / 255) (+ the padding of every row to a multiple of four entries: at most 3 * 32 per slice)
+    return n + 32 * ((n < cells ? n : cells) + n / 255 + 1) + 96 * ((cells + 31) / 32);
 }
 
 struct PlanOffsets { size_t row, bg, pairs, ell_off, row_desc, ent, usrc_cell, own_masks, total; };

@@ -131,7 +131,10 @@ def _launch(curs: Sequence[torch.Tensor], origs: Sequence[torch.Tensor], want_gr
     shapes = tuple(tuple(c.shape) for c in curs)
     # maps smaller than grid/8 (e.g. 4x4) exceed the tap window of the specialised patch-1 kernels: the general kernel takes them
     # 'local_avg' on a layer smaller than the grid needs the whole up-sampled map: the general kernel takes it (no shipped config does)
+    # the patch-1 kernels move whole 16-byte groups of a plane: maps whose area is not a multiple of 4 (e.g. 9x9, 63x63) go to the
+    # general kernel too
     general = (patch != 1 or any(2 * -(-plan.grid // min(sh[1], sh[2])) > 16 for sh in shapes)
+               or any((sh[1] * sh[2]) % 4 for sh in shapes)
                or (bg_kind == _BG_LOCAL and any((sh[1], sh[2]) != (plan.grid, plan.grid) for sh in shapes)))
     key = (shapes, fg_kind, bg_kind, patch, general)
     runner = plan._runners.get(key)

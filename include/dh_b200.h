@@ -246,7 +246,9 @@ typedef struct dh_loss_layer {
 
 /* Loss plan, built once per edit from the process_correspondences lists (int32 cell ids y*grid+x): the
  * foreground pairs grouped by destination cell with duplicates collapsed into multiplicities, and the per-cell
- * multiplicities of the three background lists.  grid <= 64.  plan / ws sizes from the two queries. */
+ * multiplicities of the three background lists.  grid <= 64.  plan / ws sizes from the two queries.
+ * DH_ERR_UNSUPPORTED for a background list longer than 65535 entries, or an n_fg that could give one destination cell more
+ * than 65535 entries (16-bit plan fields). */
 size_t dh_loss_plan_bytes(int grid, int n_fg);
 size_t dh_loss_plan_workspace_bytes(int grid, int n_fg);
 int dh_build_loss_plan(const int32_t* fg_src, const int32_t* fg_dst, int n_fg,
@@ -270,6 +272,7 @@ typedef struct dh_loss_plan_desc {
     int32_t ell_groups;    /* ... and groups of 32 entries (sizes its shared-memory copy)                         */
     int32_t n_src_cells;   /* distinct source cells (sizes the per-plane buffers of the resized layers)           */
 } dh_loss_plan_desc;
+/* DH_ERR_UNSUPPORTED when the builder flagged the plan as unusable (its sliced-ELL table did not fit the plan buffer). */
 int dh_loss_plan_info(const void* plan_header_host, dh_loss_plan_desc* desc);
 /* n_* are the list lengths the plan was built from (they are the means' denominators).  ONE persistent launch for all
  * layers.  `ws` must be zero-filled once before its first use; the launch leaves its queue counters zeroed again, so the

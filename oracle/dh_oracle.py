@@ -657,12 +657,13 @@ def background_loss(cur: np.ndarray, orig: np.ndarray, pc: Dict[str, np.ndarray]
     if len(x2) == 0:
         return dtype(np.nan), np.zeros(cur.shape, dtype)          # NaN loss, nothing to scatter the gradient to
     if len(x1) == 0:
-        return dtype(np.nan), np.full(cur.shape, np.nan, dtype)
+        return dtype(np.nan), np.zeros(cur.shape, dtype)          # NaN difference: torch's abs backward takes sign(NaN) = 0
     delta = uo[:, y1, x1].mean(-1) - uc[:, y2, x2].mean(-1)
     loss = np.abs(delta).mean()
-    g_up = np.zeros((C, size[0], size[1]), dtype)
-    g_up[:, y2, x2] = (-np.sign(delta) / dtype(C * len(x2)))[:, None]
-    return dtype(loss), bilinear_resize_transpose(g_up, (h, w), dtype)
+    g_up = np.zeros((C, size[0] * size[1]), dtype)
+    # a cell listed k times receives k quanta (np.add.at accumulates over repeated indices, fancy assignment would not)
+    np.add.at(g_up, (slice(None), np.asarray(y2) * size[1] + np.asarray(x2)), (-np.sign(delta) / dtype(C * len(x2)))[:, None])
+    return dtype(loss), bilinear_resize_transpose(g_up.reshape(C, *size), (h, w), dtype)
 
 
 def loss_sign_ambiguity(cur: np.ndarray, orig: np.ndarray, pc: Dict[str, np.ndarray], size=(64, 64),
