@@ -51,6 +51,12 @@ class dh_loss_plan_desc(C.Structure):
                 ("ell_groups", C.c_int32), ("n_src_cells", C.c_int32)]
 
 
+class dh_loss_batch_edit(C.Structure):
+    _fields_ = [("layers", C.POINTER(dh_loss_layer)), ("n_layers", C.c_int32), ("plan", c_void_p), ("desc", dh_loss_plan_desc),
+                ("n_fg", C.c_int32), ("n_bg_orig", C.c_int32), ("n_bg_trans", C.c_int32), ("n_bg_common", C.c_int32),
+                ("loss_out", c_void_p)]
+
+
 _SIGNATURES = {
     "dh_status_string": (C.c_char_p, [c_int]),
     "dh_abi_version": (c_int, []),
@@ -110,6 +116,8 @@ _SIGNATURES = {
     "dh_loss_plan_info": (c_int, [c_void_p, C.POINTER(dh_loss_plan_desc)]),
     "dh_guidance_loss": (c_int, [C.POINTER(dh_loss_layer), c_int, c_int, c_void_p, C.POINTER(dh_loss_plan_desc), c_int, c_int, c_int, c_int,
                                  c_int, c_int, c_void_p, c_void_p, c_size_t, c_void_p]),
+    "dh_guidance_loss_batch_workspace_bytes": (c_size_t, [c_int, c_int, c_int]),
+    "dh_guidance_loss_batch": (c_int, [C.POINTER(dh_loss_batch_edit), c_int, c_int, c_int, c_int, c_void_p, c_size_t, c_void_p]),
     "dh_scale_inplace": (c_int, [c_void_p, c_size_t, c_void_p, c_void_p]),
     "dh_scale_inplace_many": (c_int, [C.POINTER(c_void_p), C.POINTER(c_size_t), c_int, c_void_p, c_void_p]),
     "dh_latent_step": (c_int, [c_void_p, c_void_p, c_float, c_void_p, c_size_t, c_void_p]),

@@ -395,12 +395,13 @@ __device__ __forceinline__ void block_sum(float (&v)[kN], float (*red)[8], int g
 
 // Called by the compute warps of every CTA when the queue is empty; the last CTA reduces the per-channel partials in a
 // fixed order -> loss_out[0] = total, [1+2l] = fg_l, [2+2l] = bg_l, and re-arms the counters.
-__device__ void loss_finish(const FusedParams& p, float (*red)[8], unsigned int* ticket) {
+template <class Cta>
+__device__ void loss_finish(const FusedParams& p, float (*red)[8], unsigned int* ticket, const Cta& cta) {
     __threadfence();
     __syncthreads();                      // every group of the CTA is done
     if (threadIdx.x == 0) *ticket = atomicAdd(p.counters + 1, 1u);
     __syncthreads();
-    if (*ticket != gridDim.x - 1 || threadIdx.x >= kLossThreads) return;
+    if (*ticket != cta.count() - 1 || threadIdx.x >= kLossThreads) return;
     __threadfence();
     // the first group of the last CTA: per-channel partials -> per-layer sums, four layers (eight sums) per pass; every thread
     // adds a fixed subset of the channels in a fixed order and the block tree is fixed, so the value is reproducible bit for bit
@@ -649,8 +650,24 @@ __device__ __forceinline__ void pair_term(float fm, float d, float& acc, float& 
 // kGroups: groups per CTA the kernel is compiled for.  3 (80 registers) is the general build; 4 (64 registers, 1024 threads) is
 // compiled WITHOUT the resized-layer path and is used for launches whose layers all have the loss-grid resolution - which is what
 // guided_inference issues with the reference's weight schedule (its only resized layer always has weight 0 and is skipped).
-template <int kG, bool kBinary, int kMem, int kGroups>
-__global__ void __launch_bounds__(kLossThreads * kGroups, 1) loss_fused_kernel(const __grid_constant__ FusedParams p) {
+// Where a CTA sits among the CTAs that serve its edit: the whole grid (loss_fused_kernel) or the edit's share of the grid
+// (loss_fused_batch_kernel).  The single-edit position reads blockIdx / gridDim where they are used, as a plain kernel would.
+struct WholeGrid {
+    __device__ __forceinline__ unsigned int index() const { return blockIdx.x; }
+    __device__ __forceinline__ unsigned int count() const { return gridDim.x; }
+};
+struct EditShare {
+    // shared memory: first CTA of the edit, CTAs of the edit (read where used rather than held in registers: the 3-group body
+    // runs at its 80-register cap, and two more live registers cost spills)
+    const unsigned int* first_n;
+    __device__ __forceinline__ unsigned int index() const { return blockIdx.x - first_n[0]; }
+    __device__ __forceinline__ unsigned int count() const { return first_n[1]; }
+};
+
+// The body of one edit's launch.  kBatch: the edit may have no sliced-ELL table while the batch's placement is kMem >= 1 (an
+// empty foreground list next to non-empty ones): its plan copy is then skipped.
+template <int kG, bool kBinary, int kMem, int kGroups, bool kBatch, class Cta>
+__device__ __forceinline__ void loss_fused_body(const FusedParams& p, const Cta& cta) {
     constexpr bool kHasSmall = kGroups < 4;
     extern __shared__ __align__(128) float fsm[];
     __shared__ __align__(16) FusedShared shg[kGroups];
@@ -684,14 +701,14 @@ __global__ void __launch_bounds__(kLossThreads * kGroups, 1) loss_fused_kernel(c
         tma_bulk_g2s(st_cur, L.cur + off, bytes, &sh.full);
         tma_bulk_g2s(st_org, L.orig + off, bytes, &sh.full);
     };
-    // The first item of every group is static (item b + gridDim.x * g for group g of CTA b: the longest items are spread over
+    // The first item of every group is static (item b + n * g for group g of CTA b of n: the longest items are spread over
     // the SMs first), so its planes are on their way before anything else happens; later items are drawn from the queue.
-    const int n_groups_total = (int)(gridDim.x * (blockDim.x / kLossThreads));
+    const int n_groups_total = (int)(cta.count() * (blockDim.x / kLossThreads));
     if (tid == 0) {
         mbar_init(&sh.full, 1);
         if (kMem && threadIdx.x == 0) mbar_init(&plan_bar, 1);
         mbar_fence_init();
-        stage_item((int)(blockIdx.x + gridDim.x * gid));
+        stage_item((int)(cta.index() + cta.count() * gid));
     }
 
     const int G = kG ? kG : p.G, GG = G * G;
@@ -706,9 +723,9 @@ __global__ void __launch_bounds__(kLossThreads * kGroups, 1) loss_fused_kernel(c
         uint32_t* const s_w = reinterpret_cast<uint32_t*>(fsm);
         const uint32_t b_off = (uint32_t)p.ell_desc_at * 4u, b_desc = (uint32_t)n_slices * 128u, b_ent = (uint32_t)p.ell_ent_cap * 4u;
         mbar_arrive_expect_tx(&plan_bar, b_off + b_desc + b_ent);
-        tma_bulk_g2s(s_w, pv.ell_off, b_off, &plan_bar);
-        tma_bulk_g2s(s_w + p.ell_desc_at, pv.row_desc, b_desc, &plan_bar);
-        tma_bulk_g2s(s_w + p.ell_ent_at, pv.ent, b_ent, &plan_bar);
+        if (!kBatch || b_off) tma_bulk_g2s(s_w, pv.ell_off, b_off, &plan_bar);
+        if (!kBatch || b_desc) tma_bulk_g2s(s_w + p.ell_desc_at, pv.row_desc, b_desc, &plan_bar);
+        if (!kBatch || b_ent) tma_bulk_g2s(s_w + p.ell_ent_at, pv.ent, b_ent, &plan_bar);
     }
     auto ell_off_of = [&](int sl) -> int { return kMem ? (int)s_words[sl] : __ldg(pv.ell_off + sl); };
     auto row_desc_of = [&](int i) -> uint32_t { return kMem ? s_words[p.ell_desc_at + i] : __ldg(pv.row_desc + i); };
@@ -1022,14 +1039,44 @@ __global__ void __launch_bounds__(kLossThreads * kGroups, 1) loss_fused_kernel(c
         unsigned int smid;
         asm volatile("mov.u64 %0, %globaltimer;" : "=l"(t1));
         asm volatile("mov.u32 %0, %smid;" : "=r"(smid));
-        const int slot = blockIdx.x * 4 + gid;
+        const int slot = cta.index() * 4 + gid;
         p.debug[4 * slot + 0] = dbg_t0; p.debug[4 * slot + 1] = t1;
         p.debug[4 * slot + 2] = dbg_items; p.debug[4 * slot + 3] = smid;
 #ifdef DH_LOSS_PHASE_TIMERS
         for (int i = 0; i < 8; ++i) p.debug[4 * 1024 + 8 * slot + i] = (unsigned long long)ph[i];
 #endif
     }
-    loss_finish(p, shg[0].red, &shg[0].ticket);
+    loss_finish(p, shg[0].red, &shg[0].ticket, cta);
+}
+
+template <int kG, bool kBinary, int kMem, int kGroups>
+__global__ void __launch_bounds__(kLossThreads * kGroups, 1) loss_fused_kernel(const __grid_constant__ FusedParams p) {
+    loss_fused_body<kG, kBinary, kMem, kGroups, false>(p, WholeGrid{});
+}
+
+// Several edits in one launch: CTAs [cta_begin[e], cta_begin[e + 1]) serve edit e with that edit's parameters, exactly as a
+// loss_fused_kernel launch of cta_begin[e + 1] - cta_begin[e] CTAs would (own queue, ticket, partials and loss_out; the last
+// CTA of the edit reduces it and re-arms its counters).  Launch-wide: the instantiation, the group count and the shared-memory
+// carve-out (ell_floats / tab_floats / scratch_floats are the maxima over the edits, so that the group bases line up).
+constexpr int kMaxBatchEdits = 16;
+struct FusedBatchParams {
+    FusedParams edit[kMaxBatchEdits];
+    int cta_begin[kMaxBatchEdits + 1];
+    int n_edits;
+};
+static_assert(sizeof(FusedBatchParams) <= 32764, "kernel parameters are limited to 32764 bytes");
+
+template <int kG, bool kBinary, int kMem, int kGroups>
+__global__ void __launch_bounds__(kLossThreads * kGroups, 1) loss_fused_batch_kernel(const __grid_constant__ FusedBatchParams bp) {
+    int e = 0;
+#pragma unroll
+    for (int i = 1; i < kMaxBatchEdits; ++i)
+        if (i < bp.n_edits && (int)blockIdx.x >= bp.cta_begin[i]) e = i;
+    __shared__ unsigned int first_n[2];
+    if (threadIdx.x == 0) { first_n[0] = (unsigned int)bp.cta_begin[e]; first_n[1] = (unsigned int)(bp.cta_begin[e + 1] - bp.cta_begin[e]); }
+    __syncthreads();
+    const EditShare cta{first_n};
+    loss_fused_body<kG, kBinary, kMem, kGroups, true>(bp.edit[e], cta);
 }
 
 __global__ void __launch_bounds__(256) scale_inplace_kernel(float* __restrict__ data, size_t n, const float* __restrict__ scale) {
@@ -1151,9 +1198,44 @@ int dh_loss_plan_info(const void* plan_header_host, dh_loss_plan_desc* desc) {
     return DH_OK;
 }
 
-int dh_guidance_loss(const dh_loss_layer* layers_host, int n_layers, int grid, const void* plan, const dh_loss_plan_desc* desc,
-                     int n_fg, int n_bg_orig, int n_bg_trans, int n_bg_common, int fg_kind, int bg_kind, float* loss_out,
-                     void* ws, size_t ws_bytes, void* stream) {
+// What the launch rule needs to know about one edit; prepare_edit fills it next to the edit's FusedParams.
+struct EditLaunchInfo {
+    int n_items;        // work items
+    int ell_words;      // size of the shared-memory copy of the sliced-ELL plan (0: the plan has none)
+    int tab_words;      // size of the shared-memory copy of the first resized layer's tables (0: no resized layer)
+    bool tab_ok;        // that copy can be used: exactly one resized layer, 64 x 64 grid
+    bool binary;        // bit 0 of the plan flags: every background multiplicity is 0 or 1
+};
+
+// developer knobs, read once per process: DH_LOSS_DEBUG_BUF (address of a device buffer for tools/k4_timeline.py),
+// DH_LOSS_NO_FOUR_GROUPS, DH_LOSS_MEM (cap the shared-memory placement: 0, 1, 2), DH_LOSS_GROUPS (cap the groups per CTA)
+struct LossKnobs {
+    unsigned long long* debug;
+    bool no_four;
+    int mem_cap, groups_cap;
+};
+static const LossKnobs& loss_knobs() {
+    static const LossKnobs knobs = [] {
+        LossKnobs k;
+        const char* e = getenv("DH_LOSS_DEBUG_BUF");
+        k.debug = e ? reinterpret_cast<unsigned long long*>(strtoull(e, nullptr, 0)) : nullptr;
+        k.no_four = getenv("DH_LOSS_NO_FOUR_GROUPS") != nullptr;
+        e = getenv("DH_LOSS_MEM");
+        k.mem_cap = e ? atoi(e) : 99;
+        e = getenv("DH_LOSS_GROUPS");
+        k.groups_cap = e && atoi(e) >= 1 ? atoi(e) : 99;
+        return k;
+    }();
+    return knobs;
+}
+
+// Validates one edit and builds its FusedParams (everything but the launch-wide shared-memory placement).  No CUDA call.
+// A zero source-cell or slice count in the descriptor is read as "unknown" (budget for the whole grid), except with
+// exact_if_empty for an edit without foreground pairs, whose counts are exactly zero: in a batch such an edit must not
+// raise the launch-wide shared-memory maxima of the other edits.
+static int prepare_edit(const dh_loss_layer* layers_host, int n_layers, int grid, const void* plan, const dh_loss_plan_desc* desc,
+                        int n_fg, int n_bg_orig, int n_bg_trans, int n_bg_common, int fg_kind, int bg_kind, float* loss_out,
+                        void* ws, size_t ws_bytes, bool exact_if_empty, FusedParams& fp, EditLaunchInfo& info) {
     DH_REQUIRE(desc);
     const int plan_flags = desc->flags, ell_slices = desc->ell_slices, ell_groups = desc->ell_groups;
     DH_REQUIRE(layers_host && n_layers >= 1 && n_layers <= kMaxLossLayers && loss_out && ws && plan);
@@ -1161,7 +1243,6 @@ int dh_guidance_loss(const dh_loss_layer* layers_host, int n_layers, int grid, c
     DH_REQUIRE(n_fg >= 0 && n_bg_orig >= 0 && n_bg_trans >= 0 && n_bg_common >= 0);
     if (bg_kind != 0 && bg_kind != 1 && bg_kind != 2) return DH_ERR_INVALID_ARGUMENT;
     if (fg_kind != 0 && fg_kind != 1) return DH_ERR_INVALID_ARGUMENT;
-    FusedParams fp;
     memset(&fp, 0, sizeof(fp));
     const int GG = grid * grid;
     int chan = 0, first_small = -1, n_small_layers = 0;
@@ -1211,32 +1292,15 @@ int dh_guidance_loss(const dh_loss_layer* layers_host, int n_layers, int grid, c
     fp.partial = static_cast<float*>(ws);
     fp.counters = reinterpret_cast<unsigned int*>(static_cast<char*>(ws) + o_counter);
     fp.loss_out = loss_out;
-    // developer knobs, read once per process: DH_LOSS_DEBUG_BUF (address of a device buffer for tools/k4_timeline.py),
-    // DH_LOSS_NO_FOUR_GROUPS, DH_LOSS_MEM (cap the shared-memory placement: 0, 1, 2), DH_LOSS_GROUPS (cap the groups per CTA)
-    struct Knobs {
-        unsigned long long* debug;
-        bool no_four;
-        int mem_cap, groups_cap;
-    };
-    static const Knobs knobs = [] {
-        Knobs k;
-        const char* e = getenv("DH_LOSS_DEBUG_BUF");
-        k.debug = e ? reinterpret_cast<unsigned long long*>(strtoull(e, nullptr, 0)) : nullptr;
-        k.no_four = getenv("DH_LOSS_NO_FOUR_GROUPS") != nullptr;
-        e = getenv("DH_LOSS_MEM");
-        k.mem_cap = e ? atoi(e) : 99;
-        e = getenv("DH_LOSS_GROUPS");
-        k.groups_cap = e && atoi(e) >= 1 ? atoi(e) : 99;
-        return k;
-    }();
-    fp.debug = knobs.debug;
+    fp.debug = loss_knobs().debug;
+    const bool exact = exact_if_empty && n_fg == 0;
     // scratch of a group: the slot arrays of a resized plane pair, overlaid with the sign counts of a flat plane
     auto up4 = [](int v) { return (v + 3) / 4 * 4; };
     ResizeLayout& lay = fp.lay;
     int o = 0;
     if (fp.n_small_items) {
-        const int n_src = fg_kind ? (desc->n_src_cells > 0 ? desc->n_src_cells : GG) : 0;
-        const int n_slots = fg_kind ? (ell_slices > 0 ? ell_slices * 32 : GG) : 0;
+        const int n_src = fg_kind ? (desc->n_src_cells > 0 || exact ? desc->n_src_cells : GG) : 0;
+        const int n_slots = fg_kind ? (ell_slices > 0 || exact ? ell_slices * 32 : GG) : 0;
         lay.cap_usrc = n_src; lay.cap_slots = n_slots;
         lay.uo = o; o += up4(2 * n_src);
         lay.uc = o; o += up4(2 * n_slots);
@@ -1245,26 +1309,6 @@ int dh_guidance_loss(const dh_loss_layer* layers_host, int n_layers, int grid, c
     if (fp.n_flat_items && GG > o) o = GG;
     lay.total = o;
     fp.scratch_floats = (up4(o) + 31) / 32 * 32;      // (groups stay 128-byte aligned)
-    cudaStream_t st = as_stream(stream);
-    // per-process caches of the launch geometry queries (this entry point runs every denoising step)
-    struct LaunchCache {
-        int sms, max_smem;
-        size_t smem_attr_set[10];
-    };
-    static LaunchCache caches[64];          // zero-initialised; one entry per device (function attributes are per device)
-    int dev = 0;
-    DH_CUDA_CHECK(cudaGetDevice(&dev));
-    if (dev < 0 || dev >= 64) return DH_ERR_UNSUPPORTED;
-    LaunchCache& lc = caches[dev];
-    if (!lc.sms) {
-        DH_CUDA_CHECK(cudaDeviceGetAttribute(&lc.sms, cudaDevAttrMultiProcessorCount, dev));
-        DH_CUDA_CHECK(cudaDeviceGetAttribute(&lc.max_smem, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev));
-    }
-    // shared memory: [one copy of the sliced-ELL plan][per group: stage + scratch]; as many groups (<= 3) as fit, the plan copy
-    // is dropped (entries then come through L1) before the group count goes below two
-    const size_t group_bytes = sizeof(float) * ((size_t)kStageFloats + fp.scratch_floats);
-    const size_t static_bytes = 2304;       // FusedShared x kMaxGroups and the driver's reservation, rounded up
-    const size_t budget = (size_t)lc.max_smem > static_bytes ? (size_t)lc.max_smem - static_bytes : 0;
     int ell_words = 0;
     if (fg_kind && ell_slices > 0 && ell_groups > 0) {
         fp.ell_desc_at = up4(ell_slices + 1);
@@ -1278,20 +1322,62 @@ int dh_guidance_loss(const dh_loss_layer* layers_host, int n_layers, int grid, c
     int tab_words = 0;
     if (first_small >= 0) {
         const dh_loss_layer& sl = layers_host[first_small];
-        const int n_src = fg_kind ? (desc->n_src_cells > 0 ? desc->n_src_cells : GG) : 0;
-        const int n_slots = fg_kind ? (ell_slices > 0 ? ell_slices * 32 : GG) : 0;
+        const int n_src = fg_kind ? (desc->n_src_cells > 0 || exact ? desc->n_src_cells : GG) : 0;
+        const int n_slots = fg_kind ? (ell_slices > 0 || exact ? ell_slices * 32 : GG) : 0;
         const int n_rows_max = n_slots;
         tab_words = 16 + 4 * n_src + 4 * n_slots + up4(sl.h * sl.w + 1) + up4(2 * (4 * n_rows_max + 3 * sl.h * sl.w));      // (everything in front of wo / wt; native lists padded to 4)
         tab_words = (tab_words + 31) / 32 * 32;
     }
-    // preference: three groups with the plan and the tables in shared memory, then without the tables, then two groups ...
     // (the tables of ONE resized layer fit; with several resized layers they all stay in global memory)
-    int groups = 0, mem = 0;
     fp.ell_floats = 0; fp.tab_floats = 0; fp.tab_layer = first_small >= 0 ? first_small : 0;
+    info.n_items = fp.n_flat_items + fp.n_small_items;
+    info.ell_words = ell_words;
+    info.tab_words = tab_words;
+    info.tab_ok = n_small_layers == 1 && tab_words > 0 && grid == 64;
+    info.binary = (plan_flags & 1) != 0;
+    return DH_OK;
+}
+
+// per-process caches of the launch geometry queries (the loss entry points run every denoising step)
+struct LaunchCache {
+    int sms, max_smem;
+    size_t smem_attr_set[20];      // per instantiation: [0, 10) loss_fused_kernel, [10, 20) loss_fused_batch_kernel
+};
+static int launch_cache(LaunchCache** out) {
+    static LaunchCache caches[64];          // zero-initialised; one entry per device (function attributes are per device)
+    int dev = 0;
+    DH_CUDA_CHECK(cudaGetDevice(&dev));
+    if (dev < 0 || dev >= 64) return DH_ERR_UNSUPPORTED;
+    LaunchCache& lc = caches[dev];
+    if (!lc.sms) {
+        DH_CUDA_CHECK(cudaDeviceGetAttribute(&lc.sms, cudaDevAttrMultiProcessorCount, dev));
+        DH_CUDA_CHECK(cudaDeviceGetAttribute(&lc.max_smem, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev));
+    }
+    *out = &lc;
+    return DH_OK;
+}
+
+struct LaunchChoice {
+    int groups, mem;    // groups of kLossThreads per CTA; shared-memory placement (the kMem of the instantiation)
+    int vi;             // instantiation, index into loss_variants
+    size_t smem;        // dynamic shared memory per CTA
+};
+
+// The launch rule: the group count, the shared-memory placement and the instantiation for a launch whose edits need at most
+// ell_words / tab_words / scratch_floats of shared memory and have n_items work items in all.
+static int choose_launch(const LaunchCache& lc, int grid, bool any_small, int n_items, int ell_words, int tab_words, bool tab_ok,
+                         int scratch_floats, bool binary, LaunchChoice& ch) {
+    const LossKnobs& knobs = loss_knobs();
+    // shared memory: [one copy of the sliced-ELL plan][per group: stage + scratch]; as many groups (<= 3) as fit, the plan copy
+    // is dropped (entries then come through L1) before the group count goes below two
+    const size_t group_bytes = sizeof(float) * ((size_t)kStageFloats + scratch_floats);
+    const size_t static_bytes = 2304;       // FusedShared x kMaxGroups and the driver's reservation, rounded up
+    const size_t budget = (size_t)lc.max_smem > static_bytes ? (size_t)lc.max_smem - static_bytes : 0;
+    // preference: three groups with the plan and the tables in shared memory, then without the tables, then two groups ...
+    int groups = 0, mem = 0;
     const size_t ellb = sizeof(float) * ell_words, tabb = sizeof(float) * tab_words;
-    const bool tab_ok = n_small_layers == 1 && tab_words > 0 && grid == 64;
     // launches without a resized layer use the 64-register build: up to four groups per SM
-    const bool flat_build = fp.n_small_items == 0 && grid == 64 && !knobs.no_four;
+    const bool flat_build = !any_small && grid == 64 && !knobs.no_four;
     for (int g = std::min(flat_build ? 4 : kMaxGroups, knobs.groups_cap); g >= 1 && !groups; --g) {
         if (ell_words && tab_ok && ellb + tabb + g * group_bytes <= budget) { groups = g; mem = 2; }
         else if (ell_words && grid == 64 && ellb + g * group_bytes <= budget && g >= 2) { groups = g; mem = 1; }
@@ -1302,31 +1388,116 @@ int dh_guidance_loss(const dh_loss_layer* layers_host, int n_layers, int grid, c
         groups = 1;
     }
     if (knobs.mem_cap >= 0 && knobs.mem_cap < mem) mem = knobs.mem_cap;
-    if (mem >= 1) fp.ell_floats = ell_words;
-    if (mem == 2) fp.tab_floats = tab_words;
     if (!(flat_build && mem == 1) && groups > kMaxGroups) groups = kMaxGroups;      // only the flat build runs four groups
-    const int n_items = fp.n_flat_items + fp.n_small_items;
     if (knobs.groups_cap < groups) groups = knobs.groups_cap;
     while (groups > 1 && lc.sms * (groups - 1) >= n_items) --groups;      // tiny problems: no idle groups
-    const size_t smem = sizeof(float) * ((size_t)fp.ell_floats + fp.tab_floats) + groups * group_bytes;
+    const size_t smem = sizeof(float) * ((size_t)(mem >= 1 ? ell_words : 0) + (mem == 2 ? tab_words : 0)) + groups * group_bytes;
     if (smem > budget + static_bytes) return DH_ERR_UNSUPPORTED;
-    // bit 0 of plan_flags: background multiplicities are all 0/1 (lists from np.nonzero) -> register bit masks
+    // bit 0 of the plan flags: background multiplicities are all 0/1 (lists from np.nonzero) -> register bit masks
     const bool four = flat_build && mem == 1;      // (the flat build is instantiated with the plan in shared memory)
     // (shared-memory placement is only instantiated for the reference's 64 x 64 grid)
-    const int vi = four ? 8 + ((plan_flags & 1) ? 1 : 0) : grid == 64 ? 2 + 2 * mem + ((plan_flags & 1) ? 1 : 0) : ((plan_flags & 1) ? 1 : 0);
-    void (*kernel)(const FusedParams) =
-        vi == 0 ? loss_fused_kernel<0, false, 0, kMaxGroups> : vi == 1 ? loss_fused_kernel<0, true, 0, kMaxGroups>
-        : vi == 2 ? loss_fused_kernel<64, false, 0, kMaxGroups> : vi == 3 ? loss_fused_kernel<64, true, 0, kMaxGroups>
-        : vi == 4 ? loss_fused_kernel<64, false, 1, kMaxGroups> : vi == 5 ? loss_fused_kernel<64, true, 1, kMaxGroups>
-        : vi == 6 ? loss_fused_kernel<64, false, 2, kMaxGroups> : vi == 7 ? loss_fused_kernel<64, true, 2, kMaxGroups>
-        : vi == 8 ? loss_fused_kernel<64, false, 1, 4> : loss_fused_kernel<64, true, 1, 4>;
-    if (smem > lc.smem_attr_set[vi]) {
-        DH_CUDA_CHECK(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        lc.smem_attr_set[vi] = smem;
+    ch.vi = four ? 8 + (binary ? 1 : 0) : grid == 64 ? 2 + 2 * mem + (binary ? 1 : 0) : (binary ? 1 : 0);
+    ch.groups = groups;
+    ch.mem = mem;
+    ch.smem = smem;
+    return DH_OK;
+}
+
+#define DH_LOSS_VARIANTS(K)                                                                                        \
+    { K<0, false, 0, kMaxGroups>, K<0, true, 0, kMaxGroups>, K<64, false, 0, kMaxGroups>, K<64, true, 0, kMaxGroups>, \
+      K<64, false, 1, kMaxGroups>, K<64, true, 1, kMaxGroups>, K<64, false, 2, kMaxGroups>, K<64, true, 2, kMaxGroups>, \
+      K<64, false, 1, 4>, K<64, true, 1, 4> }
+
+int dh_guidance_loss(const dh_loss_layer* layers_host, int n_layers, int grid, const void* plan, const dh_loss_plan_desc* desc,
+                     int n_fg, int n_bg_orig, int n_bg_trans, int n_bg_common, int fg_kind, int bg_kind, float* loss_out,
+                     void* ws, size_t ws_bytes, void* stream) {
+    FusedParams fp;
+    EditLaunchInfo info;
+    int rc = prepare_edit(layers_host, n_layers, grid, plan, desc, n_fg, n_bg_orig, n_bg_trans, n_bg_common, fg_kind, bg_kind, loss_out,
+                          ws, ws_bytes, false, fp, info);
+    if (rc != DH_OK) return rc;
+    LaunchCache* lc = nullptr;
+    if ((rc = launch_cache(&lc)) != DH_OK) return rc;
+    LaunchChoice ch;
+    rc = choose_launch(*lc, grid, fp.n_small_items > 0, info.n_items, info.ell_words, info.tab_words, info.tab_ok, fp.scratch_floats,
+                       info.binary, ch);
+    if (rc != DH_OK) return rc;
+    if (ch.mem >= 1) fp.ell_floats = info.ell_words;
+    if (ch.mem == 2) fp.tab_floats = info.tab_words;
+    static void (*const kernels[10])(const FusedParams) = DH_LOSS_VARIANTS(loss_fused_kernel);
+    void (*kernel)(const FusedParams) = kernels[ch.vi];
+    if (ch.smem > lc->smem_attr_set[ch.vi]) {
+        DH_CUDA_CHECK(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)ch.smem));
+        lc->smem_attr_set[ch.vi] = ch.smem;
     }
-    int grid_x = lc.sms;
-    if (grid_x * groups > n_items) grid_x = (n_items + groups - 1) / groups;
-    kernel<<<grid_x, kLossThreads * groups, smem, st>>>(fp);
+    int grid_x = lc->sms;
+    if (grid_x * ch.groups > info.n_items) grid_x = (info.n_items + ch.groups - 1) / ch.groups;
+    kernel<<<grid_x, kLossThreads * ch.groups, ch.smem, as_stream(stream)>>>(fp);
+    DH_LAUNCH_CHECK();
+    return DH_OK;
+}
+
+size_t dh_guidance_loss_batch_workspace_bytes(int n_edits, int n_layers, int max_channels) {
+    if (n_edits < 1 || n_edits > kMaxBatchEdits) return 0;
+    return (size_t)n_edits * dh_guidance_loss_workspace_bytes(n_layers, max_channels);
+}
+
+int dh_guidance_loss_batch(const dh_loss_batch_edit* edits_host, int n_edits, int grid, int fg_kind, int bg_kind, void* ws,
+                           size_t ws_bytes, void* stream) {
+    DH_REQUIRE(edits_host && ws && n_edits >= 1);
+    if (n_edits > kMaxBatchEdits) return DH_ERR_UNSUPPORTED;
+    FusedBatchParams bp;
+    memset(&bp, 0, sizeof(bp));
+    EditLaunchInfo info[kMaxBatchEdits];
+    // edit e owns bytes [e * stride, (e + 1) * stride) of the workspace
+    const size_t stride = ws_bytes / (size_t)n_edits / 16 * 16;
+    int n_items = 0, ell_words = 0, tab_words = 0, scratch_floats = 0;
+    bool any_small = false, tab_ok = true, binary = true;
+    for (int e = 0; e < n_edits; ++e) {
+        const dh_loss_batch_edit& E = edits_host[e];
+        const int rc = prepare_edit(E.layers, E.n_layers, grid, E.plan, &E.desc, E.n_fg, E.n_bg_orig, E.n_bg_trans, E.n_bg_common, fg_kind,
+                                    bg_kind, E.loss_out, static_cast<char*>(ws) + e * stride, stride, true, bp.edit[e], info[e]);
+        if (rc != DH_OK) return rc;
+        // a descriptor that gives no sliced-ELL size for a plan with pairs: dh_guidance_loss then reads the slice count from the
+        // plan and keeps the plan in global memory, but a batch may place the other edits' plans in shared memory, sized by
+        // their descriptors - this edit's copy would not fit there
+        if (fg_kind && E.n_fg > 0 && info[e].ell_words == 0) return DH_ERR_INVALID_ARGUMENT;
+        n_items += info[e].n_items;
+        ell_words = std::max(ell_words, info[e].ell_words);
+        tab_words = std::max(tab_words, info[e].tab_words);
+        scratch_floats = std::max(scratch_floats, bp.edit[e].scratch_floats);
+        any_small |= bp.edit[e].n_small_items > 0;
+        tab_ok &= info[e].tab_ok;
+        binary &= info[e].binary;
+    }
+    LaunchCache* lc = nullptr;
+    int rc = launch_cache(&lc);
+    if (rc != DH_OK) return rc;
+    if (n_edits > lc->sms) return DH_ERR_UNSUPPORTED;      // (the one check that needs the device; no GPU has fewer than 16 SMs)
+    LaunchChoice ch;
+    if ((rc = choose_launch(*lc, grid, any_small, n_items, ell_words, tab_words, tab_ok, scratch_floats, binary, ch)) != DH_OK) return rc;
+    // CTAs in proportion to the work items, at least one per edit, at most sms in all; no group of an edit sits idle
+    int n_ctas = 0;
+    for (int e = 0; e < n_edits; ++e) {
+        FusedParams& fp = bp.edit[e];
+        fp.ell_floats = ch.mem >= 1 ? ell_words : 0;
+        fp.tab_floats = ch.mem == 2 ? tab_words : 0;
+        fp.scratch_floats = scratch_floats;
+        int share = 1 + (int)((long long)(lc->sms - n_edits) * info[e].n_items / n_items);
+        const int cap = (info[e].n_items + ch.groups - 1) / ch.groups;
+        if (share > cap) share = cap;
+        bp.cta_begin[e] = n_ctas;
+        n_ctas += share;
+    }
+    bp.cta_begin[n_edits] = n_ctas;
+    bp.n_edits = n_edits;
+    static void (*const kernels[10])(const FusedBatchParams) = DH_LOSS_VARIANTS(loss_fused_batch_kernel);
+    void (*kernel)(const FusedBatchParams) = kernels[ch.vi];
+    if (ch.smem > lc->smem_attr_set[10 + ch.vi]) {
+        DH_CUDA_CHECK(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)ch.smem));
+        lc->smem_attr_set[10 + ch.vi] = ch.smem;
+    }
+    kernel<<<n_ctas, kLossThreads * ch.groups, ch.smem, as_stream(stream)>>>(bp);
     DH_LAUNCH_CHECK();
     return DH_OK;
 }

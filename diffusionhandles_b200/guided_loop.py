@@ -16,7 +16,7 @@ import torch
 
 from . import _native as N
 from .guided_stable_diffuser import make_guidance_weight_schedule
-from .losses import guidance_loss, guidance_loss_and_grad
+from .losses import guidance_loss, guidance_loss_and_grad, guidance_loss_and_grad_batch
 
 
 class DDIMSchedule:
@@ -161,12 +161,51 @@ def guided_denoise(latents: torch.Tensor, timesteps: Sequence, unet: Callable, s
 
     guided_stable_diffuser.py:415-434: loss = sum_l fgw[l] * L_fg,l + bgw[l] * L_bg,l; latents -= 0.1 * dloss/dlatents.
     """
+    return _denoise(False, latents, timesteps, unet, scheduler_step, activations_orig, processed_correspondences, fg_weight,
+                    bg_weight, num_optsteps, guidance_max_step, guidance_schedule_type, bg_loss_type, fg_patch_size, bg_patch_size,
+                    step_size, scale_model_input, cfg_noise, skip_zero_weight_layers, on_step, ddim, cfg_pair, guidance_scale)
+
+
+def guided_denoise_batch(latents: torch.Tensor, timesteps: Sequence, unet: Callable, scheduler_step: Optional[Callable],
+                         activations_orig, processed_correspondences: Sequence,
+                         fg_weight: float = 1.5, bg_weight: float = 1.25, num_optsteps: int = 3, guidance_max_step: int = 38,
+                         guidance_schedule_type: str = "constant", bg_loss_type: str = "global_avg", fg_patch_size: int = 1,
+                         bg_patch_size: int = 1, step_size: float = 0.1, scale_model_input: Optional[Callable] = None,
+                         cfg_noise: Optional[Callable] = None, skip_zero_weight_layers: bool = False,
+                         on_step: Optional[Callable] = None, ddim: Optional[DDIMSchedule] = None, cfg_pair: Optional[Callable] = None,
+                         guidance_scale: float = 7.5) -> torch.Tensor:
+    """``guided_denoise`` for B edits at once: latents (B,4,h,w), ``processed_correspondences`` holds B dicts, and the callables
+    see all B edits (``unet`` returns activations (B,C,h,w)).  ``activations_orig`` is one identity (three (T,C,h,w) stacks)
+    shared by every edit, or a list of B identities.  Per guided iteration: one U-Net forward at batch B, one batched loss
+    launch (``guidance_loss_and_grad_batch``), one backward and one ``latent_step``; per timestep one ``cfg_ddim_step`` (all
+    edits share the timestep, so one set of coefficients serves them).
+
+    The backward runs on the sum of the per-edit losses.  Its gradient w.r.t. edit e's latents is edit e's own gradient as long
+    as the U-Net mixes no samples of the batch, which Stable Diffusion's U-Net (GroupNorm, per-sample attention) does not; a
+    model with batch statistics (BatchNorm in training mode) would break that.  'local_avg' with different foreground and
+    background patch sizes (the autograd path of ``guided_denoise``) is not implemented here."""
+    if bg_loss_type == 'local_avg' and bg_patch_size != fg_patch_size:
+        raise NotImplementedError("guided_denoise_batch: 'local_avg' with different fg / bg patch sizes is not implemented")
+    if latents.dim() != 4 or latents.shape[0] != len(processed_correspondences):
+        raise ValueError(f"latents must be (B,4,h,w) with B = {len(processed_correspondences)} edits, got {tuple(latents.shape)}")
+    return _denoise(True, latents, timesteps, unet, scheduler_step, activations_orig, list(processed_correspondences), fg_weight,
+                    bg_weight, num_optsteps, guidance_max_step, guidance_schedule_type, bg_loss_type, fg_patch_size, bg_patch_size,
+                    step_size, scale_model_input, cfg_noise, skip_zero_weight_layers, on_step, ddim, cfg_pair, guidance_scale)
+
+
+def _denoise(batch, latents, timesteps, unet, scheduler_step, activations_orig, processed_correspondences, fg_weight, bg_weight,
+             num_optsteps, guidance_max_step, guidance_schedule_type, bg_loss_type, fg_patch_size, bg_patch_size, step_size,
+             scale_model_input, cfg_noise, skip_zero_weight_layers, on_step, ddim, cfg_pair, guidance_scale):
+    """The loop of ``guided_denoise`` (batch=False: one edit) and ``guided_denoise_batch`` (batch=True: B edits)."""
     schedule = make_guidance_weight_schedule(fg_weight, bg_weight, guidance_max_step, guidance_schedule_type)
     fused_update = ddim is not None and cfg_pair is not None
     if not fused_update and scheduler_step is None:
         raise ValueError("either scheduler_step or (ddim, cfg_pair) is required")
     if fused_update:           # the timestep values index the coefficient table on the host: one read-back for the whole loop
         t_host = [int(v) for v in (timesteps.tolist() if isinstance(timesteps, (torch.Tensor, np.ndarray)) else timesteps)]
+    # batch mode: one identity shared by every edit, or one identity per edit (its per-step slices are stacked to (B,C,h,w))
+    per_edit_orig = batch and not isinstance(activations_orig[0], torch.Tensor)
+    ident = activations_orig[0] if per_edit_orig else activations_orig
     for t_idx, t in enumerate(timesteps):
         iteration = 0
         while iteration < num_optsteps and t_idx < guidance_max_step:
@@ -175,9 +214,12 @@ def guided_denoise(latents: torch.Tensor, timesteps: Sequence, unet: Callable, s
                 model_in = scale_model_input(lat, t) if scale_model_input is not None else lat
                 _, activations = unet(model_in, t)
                 fgw, bgw = schedule(t_idx, iteration)
-                acts = [a[0] for a in activations]
-                origs = [a[t_idx] for a in activations_orig]
-                activations_size = (activations_orig[2][t_idx].shape[-2], activations_orig[2][t_idx].shape[-1])
+                acts = list(activations) if batch else [a[0] for a in activations]
+                if per_edit_orig:
+                    origs = [torch.stack([ao[l][t_idx] for ao in activations_orig]) for l in range(len(acts))]
+                else:
+                    origs = [a[t_idx] for a in activations_orig]
+                activations_size = (ident[2][t_idx].shape[-2], ident[2][t_idx].shape[-1])
                 if skip_zero_weight_layers:       # a zero-weight layer contributes exactly 0 (the reference still evaluates it)
                     keep = [i for i in range(len(acts)) if fgw[i] != 0.0 or bgw[i] != 0.0]
                     acts, origs = [acts[i] for i in keep], [origs[i] for i in keep]
@@ -186,8 +228,9 @@ def guided_denoise(latents: torch.Tensor, timesteps: Sequence, unet: Callable, s
                 if acts and (bg_loss_type != 'local_avg' or bg_patch_size == fg_patch_size):
                     # value and d(loss)/d(activations) from one fused launch; the U-Net's backward then carries them to the latents
                     # (the chain rule of autograd.grad(loss, latents), guided_stable_diffuser.py:430-434)
-                    _, _, act_grads = guidance_loss_and_grad(acts, origs, processed_correspondences, fgw, bgw, bg_loss_type=bg_loss_type,
-                                                             activations_size=activations_size, patch_size=fg_patch_size)
+                    loss_and_grad = guidance_loss_and_grad_batch if batch else guidance_loss_and_grad
+                    _, _, act_grads = loss_and_grad(acts, origs, processed_correspondences, fgw, bgw, bg_loss_type=bg_loss_type,
+                                                    activations_size=activations_size, patch_size=fg_patch_size)
                     grad = torch.autograd.grad(acts, [lat], grad_outputs=act_grads)[0]
                 elif acts:
                     loss, _ = guidance_loss(acts, origs, processed_correspondences, fgw, bgw, bg_loss_type=bg_loss_type,

@@ -120,6 +120,17 @@ def _as_f32(t: torch.Tensor, dev) -> torch.Tensor:
     return t.detach().to(device=dev, dtype=torch.float32).contiguous()
 
 
+def _needs_general(shapes, grid: int, patch: int, bg_kind: int) -> bool:
+    """Whether layers of these (C,h,w) shapes go to the general patch kernel (dh_guidance_loss_patch) instead of K4."""
+    # maps smaller than grid/8 (e.g. 4x4) exceed the tap window of the specialised patch-1 kernels: the general kernel takes them
+    # 'local_avg' on a layer smaller than the grid needs the whole up-sampled map: the general kernel takes it (no shipped config does)
+    # the patch-1 kernels move whole 16-byte groups of a plane: maps whose area is not a multiple of 4 (e.g. 9x9, 63x63) go to the
+    # general kernel too
+    return (patch != 1 or any(2 * -(-grid // min(sh[1], sh[2])) > 16 for sh in shapes)
+            or any((sh[1] * sh[2]) % 4 for sh in shapes)
+            or (bg_kind == _BG_LOCAL and any((sh[1], sh[2]) != (grid, grid) for sh in shapes)))
+
+
 def _launch(curs: Sequence[torch.Tensor], origs: Sequence[torch.Tensor], want_grad: Sequence[bool],
             fgw: Sequence[float], bgw: Sequence[float], plan: LossPlan, fg_kind: int,
             bg_kind: int, patch: int = 1) -> Tuple[torch.Tensor, List[Optional[torch.Tensor]]]:
@@ -129,13 +140,7 @@ def _launch(curs: Sequence[torch.Tensor], origs: Sequence[torch.Tensor], want_gr
         raise N.NativeLibraryError("guidance losses run on CUDA only; there is no CPU fallback")
     L = len(curs)
     shapes = tuple(tuple(c.shape) for c in curs)
-    # maps smaller than grid/8 (e.g. 4x4) exceed the tap window of the specialised patch-1 kernels: the general kernel takes them
-    # 'local_avg' on a layer smaller than the grid needs the whole up-sampled map: the general kernel takes it (no shipped config does)
-    # the patch-1 kernels move whole 16-byte groups of a plane: maps whose area is not a multiple of 4 (e.g. 9x9, 63x63) go to the
-    # general kernel too
-    general = (patch != 1 or any(2 * -(-plan.grid // min(sh[1], sh[2])) > 16 for sh in shapes)
-               or any((sh[1] * sh[2]) % 4 for sh in shapes)
-               or (bg_kind == _BG_LOCAL and any((sh[1], sh[2]) != (plan.grid, plan.grid) for sh in shapes)))
+    general = _needs_general(shapes, plan.grid, patch, bg_kind)
     key = (shapes, fg_kind, bg_kind, patch, general)
     runner = plan._runners.get(key)
     if runner is None:
@@ -280,6 +285,107 @@ def guidance_loss_and_grad(activations: Sequence[torch.Tensor], activations_orig
     out, grads = _launch(activations, activations_orig, [True] * L, fg_weights, bg_weights, plan, _FG,
                          _BG_GLOBAL if bg_loss_type == 'global_avg' else _BG_LOCAL, _patch_of(patch_size))
     return out[0], out[1:], grads
+
+
+MAX_BATCH_EDITS = 16        # edits per dh_guidance_loss_batch launch; larger batches run in chunks of this size
+
+
+def _batch_runner(plans: Sequence[LossPlan], shapes, bg_kind: int):
+    """The ctypes edit and layer arrays, the workspace and the resize tables of one chunk of edits, created once per (plans,
+    shapes) and cached on the first plan (the entry keeps the plans alive, so their ids stay unique)."""
+    key = ("batch", tuple(id(p) for p in plans), shapes, bg_kind)
+    runner = plans[0]._runners.get(key)
+    if runner is None:
+        lib = N.load()
+        n, L = len(plans), len(shapes)
+        edits = (N.dh_loss_batch_edit * n)()
+        layer_arrays, tabs = [], []
+        for e, plan in enumerate(plans):
+            layers = (N.dh_loss_layer * L)()
+            for i, sh in enumerate(shapes):
+                if sh[1] > plan.grid or sh[2] > plan.grid:
+                    raise NotImplementedError(f"activation maps larger than the loss grid ({sh[1]}x{sh[2]} > {plan.grid}) are not implemented")
+                layers[i].channels, layers[i].h, layers[i].w = sh
+                t = plan.resize_tables(sh[1], sh[2], _FG, bg_kind) if (sh[1], sh[2]) != (plan.grid, plan.grid) else None
+                tabs.append(t)
+                layers[i].resize_tables = N.ptr(t) if t is not None else None
+            layer_arrays.append(layers)
+            edits[e].layers = C.cast(layers, C.POINTER(N.dh_loss_layer))
+            edits[e].n_layers = L
+            edits[e].plan = plan.buf.data_ptr()
+            edits[e].desc = plan.desc
+            edits[e].n_fg, edits[e].n_bg_orig, edits[e].n_bg_trans, edits[e].n_bg_common = plan.n
+        ws_bytes = int(lib.dh_guidance_loss_batch_workspace_bytes(n, L, max(sh[0] for sh in shapes)))
+        # zeroed once: the launch re-arms every edit's queue counters
+        runner = (tuple(plans), edits, layer_arrays, torch.zeros(ws_bytes, dtype=torch.uint8, device=plans[0].buf.device), ws_bytes, tabs)
+        plans[0]._runners[key] = runner
+    return runner
+
+
+def guidance_loss_and_grad_batch(activations: Sequence[torch.Tensor], activations_orig: Sequence[torch.Tensor],
+                                 processed_correspondences: Sequence, fg_weights: Sequence[float], bg_weights: Sequence[float],
+                                 bg_loss_type: str = 'global_avg', activations_size=(64, 64), patch_size: int = 1):
+    """``guidance_loss_and_grad`` for B edits at once: ONE K4 launch per 16 edits (dh_guidance_loss_batch).
+
+    ``activations[l]`` is (B,C_l,h_l,w_l), what a U-Net run at batch B returns; ``activations_orig[l]`` is (C_l,h_l,w_l), shared
+    by every edit (variants of one image), or (B,C_l,h_l,w_l); ``processed_correspondences`` holds B dicts.  The weights are
+    the same for every edit.  Returns (totals (B,), parts (B,2L), [grad_l (B,C_l,h_l,w_l)]): row / slice e is bit-identical to
+    what ``guidance_loss_and_grad`` returns for edit e alone.  Inputs that the single-edit call sends to the general patch kernel
+    (patch_size > 1, map areas that are not a multiple of 4, 'local_avg' on resized layers) run one such launch per edit; a batch
+    of one edit runs the single-edit launch."""
+    if bg_loss_type not in ('global_avg', 'local_avg'):
+        raise ValueError(f'Unknown background loss type: {bg_loss_type}')
+    grid = _grid_of(activations_size)
+    patch = _patch_of(patch_size)
+    bg_kind = _BG_GLOBAL if bg_loss_type == 'global_avg' else _BG_LOCAL
+    pcs = list(processed_correspondences)
+    B, L = len(pcs), len(activations)
+    if B < 1 or L < 1 or len(activations_orig) != L:
+        raise ValueError("guidance_loss_and_grad_batch needs at least one edit and one layer, and one recorded activation per layer")
+    for a, o in zip(activations, activations_orig):
+        if a.dim() != 4 or a.shape[0] != B:
+            raise ValueError(f"activations must be (B,C,h,w) with B = {B} edits, got {tuple(a.shape)}")
+        if tuple(o.shape) not in (tuple(a.shape[1:]), tuple(a.shape)):
+            raise ValueError(f"recorded activations must be (C,h,w) or (B,C,h,w) of the activations' shape, got {tuple(o.shape)}")
+    dev = activations[0].device
+    if dev.type != "cuda":
+        raise N.NativeLibraryError("guidance losses run on CUDA only; there is no CPU fallback")
+    plans = [_plan_for(pc, grid, dev) for pc in pcs]
+    shapes = tuple(tuple(a.shape[1:]) for a in activations)
+    if B == 1:      # one edit: the single-edit launch (its parameter block is 16x smaller; same bits)
+        o, g = _launch([a[0] for a in activations], [o if o.dim() == 3 else o[0] for o in activations_orig], [True] * L,
+                       fg_weights, bg_weights, plans[0], _FG, bg_kind, patch)
+        return o[None, 0], o[None, 1:], [x[None] for x in g]
+    out = torch.empty(B, 1 + 2 * L, dtype=torch.float32, device=dev)
+    if _needs_general(shapes, grid, patch, bg_kind):
+        grads = [torch.empty((B,) + sh, dtype=torch.float32, device=dev) for sh in shapes]
+        for e in range(B):
+            o, g = _launch([a[e] for a in activations], [o if o.dim() == 3 else o[e] for o in activations_orig], [True] * L,
+                           fg_weights, bg_weights, plans[e], _FG, bg_kind, patch)
+            out[e] = o
+            for l in range(L):
+                grads[l][e] = g[l]
+        return out[:, 0], out[:, 1:], grads
+    lib = N.load()
+    curs = [_as_f32(a, dev) for a in activations]
+    origs = [_as_f32(o, dev) for o in activations_orig]
+    grads = [torch.empty_like(c) for c in curs]
+    plane = [4 * sh[0] * sh[1] * sh[2] for sh in shapes]        # bytes of one edit's slice of layer l
+    cur_p, grad_p = [c.data_ptr() for c in curs], [g.data_ptr() for g in grads]
+    org_p = [(o.data_ptr(), 0 if o.dim() == 3 else plane[l]) for l, o in enumerate(origs)]
+    st = N.stream_handle(dev)
+    for b0 in range(0, B, MAX_BATCH_EDITS):
+        chunk = plans[b0:b0 + MAX_BATCH_EDITS]
+        _, edits, layer_arrays, ws, ws_bytes, _ = _batch_runner(chunk, shapes, bg_kind)
+        for j, layers in enumerate(layer_arrays):
+            e = b0 + j
+            for l in range(L):
+                layers[l].cur, layers[l].grad = cur_p[l] + e * plane[l], grad_p[l] + e * plane[l]
+                layers[l].orig = org_p[l][0] + e * org_p[l][1]
+                layers[l].fg_weight, layers[l].bg_weight = float(fg_weights[l]), float(bg_weights[l])
+            edits[j].loss_out = out.data_ptr() + 4 * e * (1 + 2 * L)
+        N.check(lib.dh_guidance_loss_batch(edits, len(chunk), grid, _FG, bg_kind, ws.data_ptr(), ws_bytes, st), "dh_guidance_loss_batch")
+    return out[:, 0], out[:, 1:], grads
 
 
 def compute_foreground_loss(activations, activations_orig, processed_correspondences, patch_size, activations_size):

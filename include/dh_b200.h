@@ -282,6 +282,29 @@ int dh_guidance_loss(const dh_loss_layer* layers_host, int n_layers, int grid, c
                      int n_fg, int n_bg_orig, int n_bg_trans, int n_bg_common, int fg_kind, int bg_kind,
                      float* loss_out /* device float[1 + 2*n_layers]: total, then fg_l, bg_l */,
                      void* ws, size_t ws_bytes, void* stream);
+/* Several edits in ONE launch: the dh_guidance_loss arguments of one edit (the plan descriptor by value). */
+typedef struct dh_loss_batch_edit {
+    const dh_loss_layer* layers;     /* HOST array of n_layers layer descriptors */
+    int32_t n_layers;
+    const void* plan;
+    dh_loss_plan_desc desc;
+    int32_t n_fg, n_bg_orig, n_bg_trans, n_bg_common;
+    float* loss_out;                 /* device float[1 + 2*n_layers] of this edit */
+} dh_loss_batch_edit;
+/* Workspace of a batch: n_edits times dh_guidance_loss_workspace_bytes (0 outside 1 <= n_edits <= 16). */
+size_t dh_guidance_loss_batch_workspace_bytes(int n_edits, int n_layers, int max_channels);
+/* dh_guidance_loss for each of the n_edits edits of the HOST array edits_host, in one launch.  grid, fg_kind and bg_kind are
+ * the same for every edit; every edit's results are bit-identical to a dh_guidance_loss call on that edit alone.  Each edit is
+ * validated as dh_guidance_loss validates one and is rejected with the same code; edit e owns bytes [e s, (e+1) s) of `ws`,
+ * s = ws_bytes / n_edits rounded down to 16, which must be large enough for that edit.  DH_ERR_INVALID_ARGUMENT for
+ * n_edits < 1 or NULL arrays, DH_ERR_UNSUPPORTED for n_edits above 16 or above the SM count (callers split larger batches).
+ * An edit with foreground pairs (fg_kind 1, n_fg > 0) whose descriptor gives no sliced-ELL size (ell_slices or ell_groups 0) is
+ * DH_ERR_INVALID_ARGUMENT: fill the descriptor with dh_loss_plan_info.  Every check runs before any CUDA call, except the
+ * comparison with the SM count, which follows the device query (it cannot fail on a GPU with 16 or more SMs).
+ * `ws` is zeroed once; the launch re-arms it (one evaluation at a time per workspace).
+ * No allocation, no synchronisation. */
+int dh_guidance_loss_batch(const dh_loss_batch_edit* edits_host, int n_edits, int grid, int fg_kind, int bg_kind,
+                           void* ws, size_t ws_bytes, void* stream);
 /* The same losses with patch_size > 1 (losses.py:62-77: both maps are replaced by their local averages over the indexed
  * cells, AvgPool2d(patch, stride 1, padding patch//2) of w*f divided by that of w plus 1e-10, before the L1 difference;
  * 'global_avg' ignores the patch).  Same plan, layer descriptors (resize_tables unused) and loss_out layout as
