@@ -127,6 +127,11 @@ _SIGNATURES = {
                                     c_float, c_float, c_int, c_int, c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_size_t,
                                     c_void_p]),
     "dh_interpolate_face_attributes": (c_int, [c_void_p, c_int, c_void_p, c_void_p, c_void_p, c_int, c_int, c_void_p, c_void_p]),
+    "dh_edit_mesh_batch_workspace_bytes": (c_size_t, [c_int, c_int, c_int, c_int, c_int]),
+    "dh_edit_mesh_batch": (c_int, [c_void_p, c_int, c_void_p, c_int, c_void_p, c_void_p, c_int, c_void_p, c_int, c_int,
+                                   C.POINTER(c_float), C.POINTER(c_float), C.POINTER(c_float), c_int, c_int, C.POINTER(c_float),
+                                   C.POINTER(c_float), c_float, c_float, c_float, c_int, c_int, c_int, c_void_p, c_void_p, c_void_p,
+                                   c_void_p, c_void_p, c_size_t, c_void_p]),
     "dh_poisson_workspace_bytes": (c_size_t, [c_int, c_int, c_int]),
     "dh_poisson_fill": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_void_p, c_int, C.c_double,
                                 c_void_p, c_void_p, c_size_t, c_void_p]),

@@ -67,6 +67,19 @@ __device__ inline float key_to_f(uint32_t k) {
     return __uint_as_float(b);
 }
 
+// transform_points (dh_geometry.cu) for B rigid transforms of one point set: the constants of one transform, prepared on the
+// host as dh_transform_points prepares them, and the launcher that applies B of them in one pass.  Transform b writes
+// out[3 N b .. 3 N (b + 1)), bit-identical to dh_transform_points with that transform.  `partial` holds 3 * kTpMaxPartials
+// doubles.
+constexpr int kTpMaxPartials = 256;
+struct TpEdit {
+    float ax, ay, az;    // unit rotation axis
+    float c, s;          // cos / sin of the angle
+    float tx, ty, tz;    // translation
+};
+TpEdit tp_edit(float angle_degrees, const float* axis3, const float* translation3);
+int tp_transform_batch(const float* pts, int N, int B, const TpEdit* edits_dev, double* partial, float* out, cudaStream_t st);
+
 __device__ inline int warp_id() { return threadIdx.x >> 5; }
 __device__ inline int lane_id() { return threadIdx.x & 31; }
 

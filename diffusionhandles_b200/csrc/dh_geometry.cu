@@ -681,25 +681,69 @@ __global__ void __launch_bounds__(256) tp_partial_sum_kernel(const float* __rest
     }
 }
 
-__global__ void __launch_bounds__(256) tp_apply_kernel(const float* __restrict__ pts, int N, const double* __restrict__ partial,
-                                                       int nblocks, float ax, float ay, float az, float c, float s,
-                                                       float tx, float ty, float tz, float* __restrict__ out) {
-    __shared__ float cen[3];
+// the centroid from the partial sums (every block repeats the short sum), then one point of one transform
+__device__ __forceinline__ void tp_centroid(const double* __restrict__ partial, int nblocks, int N, float* cen) {
     if (threadIdx.x < 3) {
         double t = 0;
         for (int b = 0; b < nblocks; ++b) t += partial[b * 3 + threadIdx.x];
         cen[threadIdx.x] = (float)(t / (double)N);
     }
     __syncthreads();
-    const int i = blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= N) return;
+}
+
+__device__ __forceinline__ void tp_apply_point(const float* __restrict__ pts, int i, const float* cen, const TpEdit& e,
+                                               float* __restrict__ out) {
+    const float ax = e.ax, ay = e.ay, az = e.az, c = e.c, s = e.s;
     const float qx = pts[3 * (size_t)i] - cen[0], qy = pts[3 * (size_t)i + 1] - cen[1], qz = pts[3 * (size_t)i + 2] - cen[2];
     const float crx = ay * qz - az * qy, cry = az * qx - ax * qz, crz = ax * qy - ay * qx;
     const float d = qx * ax + qy * ay + qz * az;
     const float omc = 1.0f - c;
-    out[3 * (size_t)i + 0] = (qx * c + crx * s + ax * d * omc) + cen[0] + tx;
-    out[3 * (size_t)i + 1] = (qy * c + cry * s + ay * d * omc) + cen[1] + ty;
-    out[3 * (size_t)i + 2] = (qz * c + crz * s + az * d * omc) + cen[2] + tz;
+    out[3 * (size_t)i + 0] = (qx * c + crx * s + ax * d * omc) + cen[0] + e.tx;
+    out[3 * (size_t)i + 1] = (qy * c + cry * s + ay * d * omc) + cen[1] + e.ty;
+    out[3 * (size_t)i + 2] = (qz * c + crz * s + az * d * omc) + cen[2] + e.tz;
+}
+
+__global__ void __launch_bounds__(256) tp_apply_kernel(const float* __restrict__ pts, int N, const double* __restrict__ partial,
+                                                       int nblocks, TpEdit e, float* __restrict__ out) {
+    __shared__ float cen[3];
+    tp_centroid(partial, nblocks, N, cen);
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= N) return;
+    tp_apply_point(pts, i, cen, e, out);
+}
+
+// B transforms of the same points: blockIdx.y = transform, output plane b = out + 3 N b
+__global__ void __launch_bounds__(256) tp_apply_batch_kernel(const float* __restrict__ pts, int N, const double* __restrict__ partial,
+                                                             int nblocks, const TpEdit* __restrict__ edits, float* __restrict__ out) {
+    __shared__ float cen[3];
+    tp_centroid(partial, nblocks, N, cen);
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= N) return;
+    const int b = blockIdx.y;
+    tp_apply_point(pts, i, cen, edits[b], out + 3 * (size_t)N * b);
+}
+
+static int tp_partial_blocks(int N) { return N >= 256 * kTpMaxPartials ? kTpMaxPartials : (N + 255) / 256; }
+
+TpEdit tp_edit(float angle_degrees, const float* axis3, const float* translation3) {
+    float a[3] = {axis3[0], axis3[1], axis3[2]};
+    const float nrm = sqrtf(a[0] * a[0] + a[1] * a[1] + a[2] * a[2]);
+    for (float& v : a) v /= nrm;
+    const float ang = angle_degrees * (float)(M_PI / 180.0);
+    TpEdit e;
+    e.ax = a[0]; e.ay = a[1]; e.az = a[2];
+    e.c = cosf(ang); e.s = sinf(ang);
+    e.tx = translation3[0]; e.ty = translation3[1]; e.tz = translation3[2];
+    return e;
+}
+
+int tp_transform_batch(const float* pts, int N, int B, const TpEdit* edits_dev, double* partial, float* out, cudaStream_t st) {
+    const int nblocks = tp_partial_blocks(N);
+    tp_partial_sum_kernel<<<nblocks, 256, 0, st>>>(pts, N, partial);
+    DH_LAUNCH_CHECK();
+    tp_apply_batch_kernel<<<dim3((N + 255) / 256, B), 256, 0, st>>>(pts, N, partial, nblocks, edits_dev, out);
+    DH_LAUNCH_CHECK();
+    return DH_OK;
 }
 
 }  // namespace dh
@@ -755,23 +799,18 @@ int dh_unproject(const float* depth, int B, int H, int W, const dh_camera* cam_h
 
 size_t dh_transform_points_workspace_bytes(int N) {
     (void)N;
-    return 256 * 3 * sizeof(double);
+    return kTpMaxPartials * 3 * sizeof(double);
 }
 
 int dh_transform_points(const float* points, int N, float angle_degrees, const float* axis_host3,
                         const float* translation_host3, float* out, void* ws, size_t ws_bytes, void* stream) {
     DH_REQUIRE(points && out && axis_host3 && translation_host3 && ws && N >= 1);
     if (ws_bytes < dh_transform_points_workspace_bytes(N)) return DH_ERR_WORKSPACE;
-    const int nblocks = N >= 256 * 256 ? 256 : (N + 255) / 256;
-    float a[3] = {axis_host3[0], axis_host3[1], axis_host3[2]};
-    const float nrm = sqrtf(a[0] * a[0] + a[1] * a[1] + a[2] * a[2]);
-    for (float& v : a) v /= nrm;
-    const float ang = angle_degrees * (float)(M_PI / 180.0);
+    const int nblocks = tp_partial_blocks(N);
     tp_partial_sum_kernel<<<nblocks, 256, 0, as_stream(stream)>>>(points, N, (double*)ws);
     DH_LAUNCH_CHECK();
-    tp_apply_kernel<<<(N + 255) / 256, 256, 0, as_stream(stream)>>>(points, N, (const double*)ws, nblocks, a[0], a[1], a[2],
-                                                                     cosf(ang), sinf(ang), translation_host3[0],
-                                                                     translation_host3[1], translation_host3[2], out);
+    tp_apply_kernel<<<(N + 255) / 256, 256, 0, as_stream(stream)>>>(points, N, (const double*)ws, nblocks,
+                                                                     tp_edit(angle_degrees, axis_host3, translation_host3), out);
     DH_LAUNCH_CHECK();
     return DH_OK;
 }

@@ -20,6 +20,8 @@
 #include <math.h>
 #include <string.h>
 
+#include <vector>
+
 namespace dh {
 
 constexpr float kRasterEps = 1e-8f;
@@ -139,11 +141,16 @@ __device__ __forceinline__ Tri load_tri(const float* __restrict__ ndc, const int
     return t;
 }
 
-__global__ void __launch_bounds__(128) raster_faces_kernel(const float* __restrict__ ndc, const int32_t* __restrict__ faces, int F,
-                                                           int H, int W, RasterSettings st, unsigned long long* keys) {
-    const int f = blockIdx.x * blockDim.x + threadIdx.x;
-    if (f >= F) return;
-    const Tri t = load_tri(ndc, faces, f);
+// component d of a (V,D) vertex attribute interpolated with the barycentrics of face (i0, i1, i2)
+__device__ __forceinline__ float interp_attr(const float* __restrict__ attr, int D, int d, int i0, int i1, int i2, float b0, float b1,
+                                             float b2) {
+    return __fadd_rn(__fadd_rn(__fmul_rn(attr[(size_t)i0 * D + d], b0), __fmul_rn(attr[(size_t)i1 * D + d], b1)),
+                     __fmul_rn(attr[(size_t)i2 * D + d], b2));
+}
+
+// one face: walk the pixels of its bounding box and offer (pz, key_face) to the z-buffer of every pixel it covers
+__device__ __forceinline__ void raster_face(const Tri& t, unsigned int key_face, int H, int W, const RasterSettings& st,
+                                            unsigned long long* keys) {
     const float zmax = fmaxf(t.z0, fmaxf(t.z1, t.z2));
     if (zmax < 0.0f) return;
     // candidate pixel range from the blur-grown bounding box (conservative; the exact test is repeated per pixel)
@@ -166,11 +173,18 @@ __global__ void __launch_bounds__(128) raster_faces_kernel(const float* __restri
             if (!pixel_in_face(t, px, py, st, pz, b0, b1, b2)) continue;
             // image row / column: both axes are reversed (+x left, +y up)
             const int row = H - 1 - yidx, col = W - 1 - xidx;
-            const unsigned long long key = ((unsigned long long)__float_as_uint(pz) << 32) | (unsigned int)f;
+            const unsigned long long key = ((unsigned long long)__float_as_uint(pz) << 32) | key_face;
             unsigned long long* k = keys + (size_t)row * W + col;
             if (key < *(volatile unsigned long long*)k) atomicMin(k, key);
         }
     }
+}
+
+__global__ void __launch_bounds__(128) raster_faces_kernel(const float* __restrict__ ndc, const int32_t* __restrict__ faces, int F,
+                                                           int H, int W, RasterSettings st, unsigned long long* keys) {
+    const int f = blockIdx.x * blockDim.x + threadIdx.x;
+    if (f >= F) return;
+    raster_face(load_tri(ndc, faces, f), (unsigned int)f, H, W, st, keys);
 }
 
 __global__ void __launch_bounds__(256) raster_resolve_kernel(const float* __restrict__ ndc, const int32_t* __restrict__ faces, int H,
@@ -209,9 +223,7 @@ __global__ void __launch_bounds__(256) raster_interpolate_kernel(const float* __
     }
     const int i0 = faces[3 * (size_t)f], i1 = faces[3 * (size_t)f + 1], i2 = faces[3 * (size_t)f + 2];
     const float b0 = bary[3 * (size_t)q], b1 = bary[3 * (size_t)q + 1], b2 = bary[3 * (size_t)q + 2];
-    for (int d = 0; d < D; ++d)
-        o[d] = __fadd_rn(__fadd_rn(__fmul_rn(attr[(size_t)i0 * D + d], b0), __fmul_rn(attr[(size_t)i1 * D + d], b1)),
-                         __fmul_rn(attr[(size_t)i2 * D + d], b2));
+    for (int d = 0; d < D; ++d) o[d] = interp_attr(attr, D, d, i0, i1, i2, b0, b1, b2);
     o[D] = 1.0f;
 }
 
@@ -220,6 +232,199 @@ static size_t raster_layout(int V, int P, size_t* o_ndc, size_t* o_keys) {
     *o_ndc = o;  o = align_up(o + sizeof(float) * 3 * (size_t)V, 256);
     *o_keys = o; o = align_up(o + sizeof(unsigned long long) * (size_t)P, 256);
     return o;
+}
+
+// ------------------------------------------------------------------------------------------------
+// Mesh mode for B rigid transforms of one scene's foreground (dh_edit_mesh_batch).
+//
+// A pixel's z-buffer entry is the minimum of (pz bits << 32 | face index) over the faces that cover it, and a minimum does not
+// depend on how the faces are split: the minimum over bg u fg is the minimum of the bg minimum and the fg minimum.  So the
+// background faces are rasterised ONCE, their keys are copied to every edit, and each edit's moved foreground faces go on top
+// with the index they have in the joined mesh (F_bg + f).  The result is bit-identical to rasterising [bg, fg] joined, and the
+// background faces still win exact ties.  Each (pixel, edit) winner is then resolved straight to what mesh mode reads off the
+// render - the world z and, for a foreground winner, the carried source pixel - without barycentric or attribute buffers.
+// ------------------------------------------------------------------------------------------------
+constexpr int kMeshTile = 1024;                 // pixels per compaction tile
+constexpr int kMeshTileThreads = kMeshTile / 4; // 4 consecutive pixels per thread (raster order = thread order)
+constexpr int kMaxGridY = 65535;
+
+struct MeshBatchScene {
+    const float* bg_ndc;      // (V_bg,3)
+    const float* bg_verts;    // (V_bg,3) world
+    const int32_t* bg_faces;  // (F_bg,3)
+    int F_bg;
+    const float* fg_ndc;      // (B,V_fg,3)
+    const float* fg_world;    // (B,V_fg,3) transformed world vertices
+    const float* fg_colors;   // (V_fg,3) source x/(W-1), y/(H-1), flag
+    const int32_t* fg_faces;  // (F_fg,3) fg-local vertex ids
+    int V_fg;
+};
+
+// keys of the background raster (edit 0) -> every other edit
+__global__ void __launch_bounds__(256) raster_keys_broadcast_kernel(unsigned long long* keys, int P, int B) {
+    const int q = blockIdx.x * blockDim.x + threadIdx.x;
+    if (q >= P) return;
+    const unsigned long long k = keys[q];
+    for (int b = 1; b < B; ++b) keys[(size_t)b * P + q] = k;
+}
+
+// the foreground faces of every edit (blockIdx.y = edit), keyed with their index in the joined mesh
+__global__ void __launch_bounds__(128) raster_faces_batch_kernel(const float* __restrict__ ndc, int V, const int32_t* __restrict__ faces,
+                                                                 int F, int key_base, int H, int W, RasterSettings st,
+                                                                 unsigned long long* keys) {
+    const int f = blockIdx.x * blockDim.x + threadIdx.x;
+    if (f >= F) return;
+    const int b = blockIdx.y;
+    raster_face(load_tri(ndc + 3 * (size_t)V * b, faces, f), (unsigned int)(key_base + f), H, W, st, keys + (size_t)b * H * W);
+}
+
+// Pixel q of edit b with z-buffer entry `key`: returns the world z of the winning surface (world_position[..., 2]: 0 when the pixel
+// is empty).  `emit` is set when a foreground face wins and its interpolated flag exceeds 0.5, with the source pixel it carries,
+// rounded half-to-even like torch.round.  A background face carries the colour (x, y, 0): its flag is exactly 0, it never emits.
+__device__ __forceinline__ float mesh_resolve(const MeshBatchScene& s, int b, int q, unsigned long long key, int H, int W,
+                                              const RasterSettings& st, bool& emit, float& src_x, float& src_y) {
+    emit = false;
+    if (key == 0xFFFFFFFFFFFFFFFFull) return 0.0f;
+    const int f = (int)(key & 0xFFFFFFFFull);
+    const bool fg = f >= s.F_bg;
+    const int lf = fg ? f - s.F_bg : f;
+    const float* ndc = fg ? s.fg_ndc + 3 * (size_t)s.V_fg * b : s.bg_ndc;
+    const float* verts = fg ? s.fg_world + 3 * (size_t)s.V_fg * b : s.bg_verts;
+    const int32_t* faces = fg ? s.fg_faces : s.bg_faces;
+    const int row = q / W, col = q - row * W;
+    const float px = pix_to_ndc(W - 1 - col, W, H), py = pix_to_ndc(H - 1 - row, H, W);
+    float pz, b0 = -1.0f, b1 = -1.0f, b2 = -1.0f;
+    pixel_in_face(load_tri(ndc, faces, lf), px, py, st, pz, b0, b1, b2);
+    const int i0 = faces[3 * (size_t)lf], i1 = faces[3 * (size_t)lf + 1], i2 = faces[3 * (size_t)lf + 2];
+    const float z = interp_attr(verts, 3, 2, i0, i1, i2, b0, b1, b2);
+    if (fg && interp_attr(s.fg_colors, 3, 2, i0, i1, i2, b0, b1, b2) > 0.5f) {
+        emit = true;
+        src_x = rintf(__fmul_rn(interp_attr(s.fg_colors, 3, 0, i0, i1, i2, b0, b1, b2), (float)(W - 1)));
+        src_y = rintf(__fmul_rn(interp_attr(s.fg_colors, 3, 1, i0, i1, i2, b0, b1, b2), (float)(H - 1)));
+    }
+    return z;
+}
+
+// pass 1 over (pixel, edit): target z (+ pix_to_face when asked for) and the number of correspondences per tile
+__global__ void __launch_bounds__(kMeshTileThreads) mesh_resolve_count_kernel(MeshBatchScene s, const unsigned long long* __restrict__ keys,
+                                                                               int H, int W, int ntiles, RasterSettings st,
+                                                                               float* __restrict__ target_z, int32_t* __restrict__ pix_to_face,
+                                                                               int32_t* __restrict__ tile_counts) {
+    __shared__ int warp_sums[32];
+    const int b = blockIdx.y, tile = blockIdx.x, P = H * W;
+    const size_t eo = (size_t)b * P;
+    const int q0 = tile * kMeshTile + threadIdx.x * 4;
+    int c = 0;
+#pragma unroll
+    for (int i = 0; i < 4; ++i) {
+        const int q = q0 + i;
+        if (q >= P) continue;
+        const unsigned long long key = keys[eo + q];
+        bool emit;
+        float sx, sy;
+        target_z[eo + q] = mesh_resolve(s, b, q, key, H, W, st, emit, sx, sy);
+        c += emit;
+        if (pix_to_face) pix_to_face[eo + q] = key == 0xFFFFFFFFFFFFFFFFull ? -1 : (int32_t)(key & 0xFFFFFFFFull);
+    }
+    c = __reduce_add_sync(0xFFFFFFFFu, c);
+    if (lane_id() == 0) warp_sums[warp_id()] = c;
+    __syncthreads();
+    if (warp_id() == 0) {
+        int t = lane_id() < (int)(blockDim.x >> 5) ? warp_sums[lane_id()] : 0;
+        t = __reduce_add_sync(0xFFFFFFFFu, t);
+        if (lane_id() == 0) tile_counts[b * ntiles + tile] = t;
+    }
+}
+
+// pass 2: the rows [x_src, y_src, x_dst, y_dst] of every edit in target raster order (tile offsets from the counts, then a block
+// scan); only foreground winners are resolved again.  The last tile of an edit publishes n_corr.
+__global__ void __launch_bounds__(kMeshTileThreads) mesh_emit_kernel(MeshBatchScene s, const unsigned long long* __restrict__ keys,
+                                                                      int H, int W, int ntiles, RasterSettings st,
+                                                                      const int32_t* __restrict__ tile_counts, int64_t* __restrict__ corr,
+                                                                      int32_t* __restrict__ n_corr) {
+    __shared__ int scan_smem[33];
+    __shared__ int base_smem;
+    const int b = blockIdx.y, tile = blockIdx.x, P = H * W;
+    if (tile_counts[b * ntiles + tile] == 0 && tile != ntiles - 1) return;     // nothing to emit (uniform over the block)
+    int part = 0;
+    for (int t = threadIdx.x; t < tile; t += blockDim.x) part += tile_counts[b * ntiles + t];
+    int tot;
+    block_exclusive_scan(part, scan_smem, tot);
+    if (threadIdx.x == 0) base_smem = tot;
+    __syncthreads();
+    const int base = base_smem;
+    const size_t eo = (size_t)b * P;
+    const int q0 = tile * kMeshTile + threadIdx.x * 4;
+    unsigned kmask = 0;
+    float sx[4], sy[4];          // rounded source coordinates, converted to int64 at the store
+#pragma unroll
+    for (int i = 0; i < 4; ++i) {
+        const int q = q0 + i;
+        sx[i] = sy[i] = 0.0f;
+        if (q >= P) continue;
+        const unsigned long long key = keys[eo + q];
+        if (key == 0xFFFFFFFFFFFFFFFFull || (int)(key & 0xFFFFFFFFull) < s.F_bg) continue;
+        bool emit;
+        mesh_resolve(s, b, q, key, H, W, st, emit, sx[i], sy[i]);
+        kmask |= (unsigned)emit << i;
+    }
+    int total;
+    int pos = base + block_exclusive_scan(__popc(kmask), scan_smem, total);
+#pragma unroll
+    for (int i = 0; i < 4; ++i) {
+        if (!((kmask >> i) & 1u)) continue;
+        const int q = q0 + i, row = q / W;
+        longlong4 v;
+        v.x = (long long)sx[i]; v.y = (long long)sy[i]; v.z = q - row * W; v.w = row;
+        *reinterpret_cast<longlong4*>(corr + (eo + pos) * 4) = v;
+        ++pos;
+    }
+    if (tile == ntiles - 1 && threadIdx.x == 0) n_corr[b] = base + total;
+}
+
+struct MeshBatchLayout {
+    size_t partial, edits, bg_ndc, fg_world, fg_ndc, keys, tile_counts, total;
+};
+
+static MeshBatchLayout mesh_batch_layout(int B, int V_bg, int V_fg, int H, int W) {
+    const size_t P = (size_t)H * W, ntiles = (P + kMeshTile - 1) / kMeshTile;
+    MeshBatchLayout L;
+    size_t o = 0;
+    L.partial = o;     o = align_up(o + sizeof(double) * 3 * kTpMaxPartials, 256);
+    L.edits = o;       o = align_up(o + sizeof(TpEdit) * (size_t)B, 256);
+    L.bg_ndc = o;      o = align_up(o + sizeof(float) * 3 * (size_t)V_bg, 256);
+    L.fg_world = o;    o = align_up(o + sizeof(float) * 3 * (size_t)V_fg * B, 256);
+    L.fg_ndc = o;      o = align_up(o + sizeof(float) * 3 * (size_t)V_fg * B, 256);
+    L.keys = o;        o = align_up(o + sizeof(unsigned long long) * P * B, 256);
+    L.tile_counts = o; o = align_up(o + sizeof(int32_t) * ntiles * B, 256);
+    L.total = o;
+    return L;
+}
+
+static RasterCamDev make_raster_cam(const float* R_host9, const float* T_host3, float sx, float sy) {
+    RasterCamDev cam;
+    memcpy(cam.R, R_host9, sizeof(cam.R));
+    memcpy(cam.T, T_host3, sizeof(cam.T));
+    cam.sx = sx; cam.sy = sy;
+    return cam;
+}
+
+static RasterSettings make_raster_settings(float blur_radius, int cull_backfaces, int perspective_correct, int clip_barycentric) {
+    RasterSettings st;
+    st.blur_radius = blur_radius; st.blur_sqrt = sqrtf(blur_radius);
+    st.cull_backfaces = cull_backfaces; st.perspective_correct = perspective_correct; st.clip_barycentric = clip_barycentric;
+    return st;
+}
+
+// size checks shared by the call and its workspace query
+static int mesh_batch_sizes(int B, int V_bg, int F_bg, int V_fg, int F_fg, int H, int W) {
+    if (B < 1 || V_bg < 1 || F_bg < 0 || V_fg < 0 || F_fg < 0 || H < 1 || W < 1) return DH_ERR_INVALID_ARGUMENT;
+    if (F_fg > 0 && V_fg == 0) return DH_ERR_INVALID_ARGUMENT;       // faces without vertices
+    if (B > kMaxGridY) return DH_ERR_UNSUPPORTED;                     // one grid row per edit
+    if ((long long)H * W > (1ll << 29)) return DH_ERR_UNSUPPORTED;
+    if ((long long)B * V_fg > 0x7FFFFFFFll) return DH_ERR_UNSUPPORTED; // the moved vertices are projected as one flat array
+    if ((long long)F_bg + F_fg > 0x7FFFFFFFll) return DH_ERR_UNSUPPORTED; // joined face indices are 31-bit in the keys
+    return DH_OK;
 }
 
 }  // namespace dh
@@ -244,13 +449,8 @@ int dh_rasterize_meshes(const float* verts, int V, const int32_t* faces, int F, 
     if (ws_bytes < raster_layout(V, H * W, &o_ndc, &o_keys)) return DH_ERR_WORKSPACE;
     float* ndc = reinterpret_cast<float*>(static_cast<char*>(ws) + o_ndc);
     unsigned long long* keys = reinterpret_cast<unsigned long long*>(static_cast<char*>(ws) + o_keys);
-    RasterCamDev cam;
-    memcpy(cam.R, R_host9, sizeof(cam.R));
-    memcpy(cam.T, T_host3, sizeof(cam.T));
-    cam.sx = sx; cam.sy = sy;
-    RasterSettings st;
-    st.blur_radius = blur_radius; st.blur_sqrt = sqrtf(blur_radius);
-    st.cull_backfaces = cull_backfaces; st.perspective_correct = perspective_correct; st.clip_barycentric = clip_barycentric;
+    const RasterCamDev cam = make_raster_cam(R_host9, T_host3, sx, sy);
+    const RasterSettings st = make_raster_settings(blur_radius, cull_backfaces, perspective_correct, clip_barycentric);
     cudaStream_t s = as_stream(stream);
     DH_CUDA_CHECK(cudaMemsetAsync(keys, 0xFF, sizeof(unsigned long long) * (size_t)H * W, s));
     raster_project_kernel<<<(V + 255) / 256, 256, 0, s>>>(verts, V, cam, ndc);
@@ -268,6 +468,80 @@ int dh_interpolate_face_attributes(const float* attr, int D, const int32_t* face
                                    int H, int W, float* out, void* stream) {
     DH_REQUIRE(attr && faces && pix_to_face && bary && out && D >= 1 && H >= 1 && W >= 1);
     raster_interpolate_kernel<<<(H * W + 255) / 256, 256, 0, as_stream(stream)>>>(attr, D, faces, pix_to_face, bary, H * W, out);
+    DH_LAUNCH_CHECK();
+    return DH_OK;
+}
+
+size_t dh_edit_mesh_batch_workspace_bytes(int B, int V_bg, int V_fg, int H, int W) {
+    if (mesh_batch_sizes(B, V_bg, 0, V_fg, 0, H, W) != DH_OK) return 0;
+    return mesh_batch_layout(B, V_bg, V_fg, H, W).total;
+}
+
+int dh_edit_mesh_batch(const float* bg_verts, int V_bg, const int32_t* bg_faces, int F_bg, const float* fg_verts, const float* fg_colors,
+                       int V_fg, const int32_t* fg_faces, int F_fg, int B, const float* angles_deg_host, const float* axes_host,
+                       const float* translations_host, int H, int W, const float* R_host9, const float* T_host3, float sx, float sy,
+                       float blur_radius, int cull_backfaces, int perspective_correct, int clip_barycentric, float* target_z,
+                       int64_t* corr, int32_t* n_corr, int32_t* pix_to_face, void* ws, size_t ws_bytes, void* stream) {
+    // every check runs before the first CUDA call
+    DH_REQUIRE(bg_verts && angles_deg_host && axes_host && translations_host && R_host9 && T_host3 && target_z && corr && n_corr && ws);
+    DH_REQUIRE(F_bg <= 0 || bg_faces);
+    DH_REQUIRE(V_fg <= 0 || (fg_verts && fg_colors));
+    DH_REQUIRE(F_fg <= 0 || fg_faces);
+    DH_REQUIRE(blur_radius >= 0.0f);
+    DH_REQUIRE((reinterpret_cast<uintptr_t>(corr) & 31) == 0);      // rows are stored as one 32-byte vector
+    const int sizes = mesh_batch_sizes(B, V_bg, F_bg, V_fg, F_fg, H, W);
+    if (sizes != DH_OK) return sizes;
+    const MeshBatchLayout L = mesh_batch_layout(B, V_bg, V_fg, H, W);
+    if (ws_bytes < L.total) return DH_ERR_WORKSPACE;
+    char* w = static_cast<char*>(ws);
+    double* partial = reinterpret_cast<double*>(w + L.partial);
+    TpEdit* edits = reinterpret_cast<TpEdit*>(w + L.edits);
+    float* bg_ndc = reinterpret_cast<float*>(w + L.bg_ndc);
+    float* fg_world = reinterpret_cast<float*>(w + L.fg_world);
+    float* fg_ndc = reinterpret_cast<float*>(w + L.fg_ndc);
+    unsigned long long* keys = reinterpret_cast<unsigned long long*>(w + L.keys);
+    int32_t* tile_counts = reinterpret_cast<int32_t*>(w + L.tile_counts);
+    const RasterCamDev cam = make_raster_cam(R_host9, T_host3, sx, sy);
+    const RasterSettings st = make_raster_settings(blur_radius, cull_backfaces, perspective_correct, clip_barycentric);
+    const int P = H * W, ntiles = (P + kMeshTile - 1) / kMeshTile;
+    cudaStream_t s = as_stream(stream);
+    std::vector<TpEdit> edits_host;
+    if (V_fg > 0) {
+        edits_host.resize(B);
+        for (int b = 0; b < B; ++b) edits_host[b] = tp_edit(angles_deg_host[b], axes_host + 3 * b, translations_host + 3 * b);
+        DH_CUDA_CHECK(cudaMemcpyAsync(edits, edits_host.data(), sizeof(TpEdit) * (size_t)B, cudaMemcpyHostToDevice, s));
+    }
+    // background: projected and rasterised once into edit 0's keys, then copied to the other edits
+    DH_CUDA_CHECK(cudaMemsetAsync(keys, 0xFF, sizeof(unsigned long long) * (size_t)P, s));
+    raster_project_kernel<<<(V_bg + 255) / 256, 256, 0, s>>>(bg_verts, V_bg, cam, bg_ndc);
+    DH_LAUNCH_CHECK();
+    if (F_bg > 0) {
+        raster_faces_kernel<<<(F_bg + 127) / 128, 128, 0, s>>>(bg_ndc, bg_faces, F_bg, H, W, st, keys);
+        DH_LAUNCH_CHECK();
+    }
+    if (B > 1) {
+        raster_keys_broadcast_kernel<<<(P + 255) / 256, 256, 0, s>>>(keys, P, B);
+        DH_LAUNCH_CHECK();
+    }
+    // foreground: B transforms of the same vertices, projected as one array, every edit's faces in one launch
+    if (V_fg > 0) {
+        const int rc = tp_transform_batch(fg_verts, V_fg, B, edits, partial, fg_world, s);
+        if (rc != DH_OK) return rc;
+        const int nv = B * V_fg;
+        raster_project_kernel<<<(nv + 255) / 256, 256, 0, s>>>(fg_world, nv, cam, fg_ndc);
+        DH_LAUNCH_CHECK();
+    }
+    if (F_fg > 0) {
+        raster_faces_batch_kernel<<<dim3((F_fg + 127) / 128, B), 128, 0, s>>>(fg_ndc, V_fg, fg_faces, F_fg, F_bg, H, W, st, keys);
+        DH_LAUNCH_CHECK();
+    }
+    MeshBatchScene sc;
+    sc.bg_ndc = bg_ndc; sc.bg_verts = bg_verts; sc.bg_faces = bg_faces; sc.F_bg = F_bg;
+    sc.fg_ndc = fg_ndc; sc.fg_world = fg_world; sc.fg_colors = fg_colors; sc.fg_faces = fg_faces; sc.V_fg = V_fg;
+    const dim3 tgrid(ntiles, B);
+    mesh_resolve_count_kernel<<<tgrid, kMeshTileThreads, 0, s>>>(sc, keys, H, W, ntiles, st, target_z, pix_to_face, tile_counts);
+    DH_LAUNCH_CHECK();
+    mesh_emit_kernel<<<tgrid, kMeshTileThreads, 0, s>>>(sc, keys, H, W, ntiles, st, tile_counts, corr, n_corr);
     DH_LAUNCH_CHECK();
     return DH_OK;
 }

@@ -303,6 +303,64 @@ def transform_depth_mesh(depth: torch.Tensor, bg_depth: torch.Tensor, fg_mask: t
     return normalize_depth(1.0 / target_depth, bounds=bounds), correspondences
 
 
+def transform_depth_mesh_batch(depth: torch.Tensor, bg_depth: torch.Tensor, fg_mask: torch.Tensor, intrinsics: torch.Tensor,
+                               rot_angles, rot_axes, translations, use_input_depth_normalization=False):
+    """``transform_depth_mesh`` for B transforms of one scene in one native call (``dh_edit_mesh_batch``).
+
+    Both meshes are built once; the background mesh is rasterised once and every edit's moved foreground faces are rasterised
+    over a copy of its z-buffer, which gives the z-buffer of the joined mesh bit for bit.  ``rot_angles`` / ``rot_axes`` /
+    ``translations`` hold one entry per edit (``None`` takes the defaults of the single call).  Returns ``(disparities
+    (B,1,H,W) fp32 on depth.device, [correspondences (n_b,4) int64 CPU] * B)``; entry b equals ``transform_depth_mesh`` with
+    transform b bit for bit."""
+    from .renderer import MeshRenderer, fov_scales
+    B = len(rot_angles)
+    if B < 1 or len(rot_axes) != B or len(translations) != B:
+        raise ValueError(f"rot_angles, rot_axes and translations must have one entry per edit (at least one), got {B}, "
+                         f"{len(rot_axes)}, {len(translations)}")
+    if not fg_mask.any():
+        disparity, corr = _empty_mask_result(depth, use_input_depth_normalization)
+        return disparity.expand(B, *disparity.shape[1:]).clone(), [corr.clone() for _ in range(B)]
+    _require_cuda(depth, "depth")
+    lib = N.load()
+    dev = depth.device
+    H, W = depth.shape[-2], depth.shape[-1]
+    f32 = torch.float32
+    background = depth_to_mesh(depth=bg_depth, intrinsics=intrinsics)
+    foreground = depth_to_mesh(depth=depth, intrinsics=intrinsics, mask=fg_mask[0, 0] > 0.5)
+    bg_verts = background.verts.to(f32).contiguous()
+    bg_faces = background.faces.to(torch.int32).contiguous()
+    fg_verts = foreground.verts.to(f32).contiguous()
+    fg_colors = foreground.vert_attributes["color"].to(f32).contiguous()
+    fg_faces = foreground.faces.to(torch.int32).contiguous()
+    V_bg, F_bg, V_fg, F_fg = bg_verts.shape[0], bg_faces.shape[0], fg_verts.shape[0], fg_faces.shape[0]
+    # the host values of the single call: the angle through an fp32 tensor, axis / translation as C floats
+    angles, axes, shifts = [], [], []
+    for a, ax, t in zip(rot_angles, rot_axes, translations):
+        angles.append(float(torch.tensor(0.0 if a is None else float(a), dtype=f32)))
+        axes += [float(v) for v in (torch.tensor([0.0, 1.0, 0.0]) if ax is None else ax).detach().cpu().reshape(-1)[:3]]
+        shifts += [float(v) for v in (torch.zeros(3) if t is None else t).detach().cpu().reshape(-1)[:3]]
+    # the camera of the single call: Camera(intrinsics) (identity extrinsics) through MeshRenderer, blur 1e-5, back faces culled
+    sx, sy = fov_scales(intrinsics[1, 1], H, W, MeshRenderer.z_near)
+    R = (C.c_float * 9)(1.0, 0.0, 0.0, 0.0, 1.0, 0.0, 0.0, 0.0, 1.0)
+    T = (C.c_float * 3)(0.0, 0.0, 0.0)
+    target_z = torch.empty((B, H, W), dtype=f32, device=dev)
+    corr = torch.empty((B, H * W, 4), dtype=torch.int64, device=dev)
+    n_corr = torch.empty(B, dtype=torch.int32, device=dev)
+    ws_bytes = int(lib.dh_edit_mesh_batch_workspace_bytes(B, V_bg, V_fg, H, W))
+    if ws_bytes == 0:
+        raise ValueError(f"dh_edit_mesh_batch: unsupported sizes (B={B}, {H}x{W}, {V_bg} + {V_fg} vertices)")
+    ws = torch.empty(ws_bytes, dtype=torch.uint8, device=dev)
+    N.check(lib.dh_edit_mesh_batch(N.ptr(bg_verts), V_bg, N.ptr(bg_faces), F_bg, N.ptr(fg_verts), N.ptr(fg_colors), V_fg,
+                                   N.ptr(fg_faces), F_fg, B, (C.c_float * B)(*angles), (C.c_float * (3 * B))(*axes),
+                                   (C.c_float * (3 * B))(*shifts), H, W, R, T, sx, sy, 1e-5, 1, 1, 1, N.ptr(target_z), N.ptr(corr),
+                                   N.ptr(n_corr), None, N.ptr(ws), ws_bytes, N.stream_handle(dev)), "dh_edit_mesh_batch")
+    counts = n_corr.tolist()                                                 # the one synchronisation
+    rows = corr[:, :max(counts)].cpu()
+    correspondences = [rows[b, :n].clone() for b, n in enumerate(counts)]
+    bounds = normalize_depth(1.0 / depth, return_bounds=True)[1] if use_input_depth_normalization else None
+    return normalize_depth(1.0 / target_z[:, None], bounds=bounds), correspondences
+
+
 def transform_depth(depth: torch.Tensor, bg_depth: torch.Tensor, fg_mask: torch.Tensor, intrinsics: torch.Tensor,
                     rot_angle: float = None, rot_axis: torch.Tensor = None, translation: torch.Tensor = None,
                     use_input_depth_normalization=False, depth_transform_mode: str = "pc"):

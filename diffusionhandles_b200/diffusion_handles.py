@@ -11,7 +11,7 @@ from types import SimpleNamespace
 
 import torch
 
-from .depth_transform import _require_cuda, normalize_depth, transform_depth
+from .depth_transform import _require_cuda, normalize_depth, transform_depth, transform_depth_mesh_batch
 from .engine import get_engine, make_rigid
 from .guided_stable_diffuser import GuidedStableDiffuser
 
@@ -108,13 +108,17 @@ class DiffusionHandles:
     def edit_geometry_batch(self, depth: torch.Tensor, fg_mask: torch.Tensor, bg_depth: torch.Tensor, rot_angles, rot_axes,
                             translations, use_input_depth_normalization=False):
         """B transforms of one scene: edited disparities (B,1,H,W) and a list of B correspondence lists, each equal bit for bit
-        to ``edit_geometry`` with that transform.  In 'pc' mode the B edits are ONE ``EditEngine`` batch; an empty mask and the
-        mesh mode run ``edit_geometry`` per transform."""
+        to ``edit_geometry`` with that transform.  In 'pc' mode the B edits are ONE ``EditEngine`` batch; in 'mesh' mode they are
+        ONE ``transform_depth_mesh_batch`` call (the background mesh rasterised once); an empty mask in 'pc' mode runs
+        ``edit_geometry`` per transform."""
         B = len(rot_angles)
         if len(rot_axes) != B or len(translations) != B:
             raise ValueError(f"rot_angles, rot_axes and translations must have one entry per edit, got {B}, {len(rot_axes)}, {len(translations)}")
         S = fg_mask.shape[-1]
         with torch.no_grad():
+            if self.conf.depth_transform_mode == "mesh" and B > 0:
+                return transform_depth_mesh_batch(depth, bg_depth, fg_mask, self.diffuser.get_depth_intrinsics(device=depth.device),
+                                                  rot_angles, rot_axes, translations, use_input_depth_normalization)
             if self.conf.depth_transform_mode != "pc" or not fg_mask.any() or fg_mask.shape[-2] != S or depth.shape[0] != 1:
                 outs = [self.edit_geometry(depth, fg_mask, bg_depth, a, ax, t, use_input_depth_normalization)
                         for a, ax, t in zip(rot_angles, rot_axes, translations)]
@@ -136,8 +140,8 @@ class DiffusionHandles:
                                    translations, fg_weight: float = None, bg_weight: float = None, use_input_depth_normalization=False):
         """``transform_foreground`` for B transforms of one scene: the geometry of all B edits in one batch
         (``edit_geometry_batch``), then the injected diffuser's ``guided_inference_batch`` with ``init_noise`` and the identity
-        ``activations`` shared by every edit.  Returns (edited images (B,...), edited disparities (B,1,H,W)).  Saving the
-        denoising steps is not supported in batch mode."""
+        ``activations`` shared by every edit; the geometry is batched in both depth transform modes ('pc' and 'mesh').  Returns
+        (edited images (B,...), edited disparities (B,1,H,W)).  Saving the denoising steps is not supported in batch mode."""
         guided = self._need(self.diffuser, "guided_inference_batch")
         if self.conf.guided_diffuser.save_denoising_steps:
             raise NotImplementedError("transform_foreground_batch does not save the denoising steps; use transform_foreground per edit")

@@ -371,6 +371,30 @@ int dh_rasterize_meshes(const float* verts, int V, const int32_t* faces, int F, 
 int dh_interpolate_face_attributes(const float* attr, int D, const int32_t* faces, const int32_t* pix_to_face,
                                    const float* bary, int H, int W, float* out, void* stream);
 
+/* ---- mesh mode for B transforms of one scene ------------------------------------------------------
+ * The geometry of B mesh-mode edits in one call: the foreground mesh (fg_verts (V_fg,3) world, fg_colors (V_fg,3) = source
+ * x/(W-1), y/(H-1), flag; fg_faces (F_fg,3) fg-local ids) is moved by transform b (angle in degrees, axes_host[3b..3b+2],
+ * translations_host[3b..3b+2]; bit-identical to dh_transform_points) and rendered over the background mesh (bg_verts (V_bg,3),
+ * bg_faces (F_bg,3), colour flag 0) exactly as dh_rasterize_meshes renders the joined mesh [bg, fg] (fg face f = F_bg + f):
+ * the background is rasterised once for all edits.  Outputs per edit b:
+ *   target_z (B,H,W)  world z of the visible surface (0 = empty pixel), as the interpolated world position;
+ *   corr (B,H*W,4) int64, 32-byte aligned: rows [x_src, y_src, x_dst, y_dst] in target raster order, one per pixel whose
+ *                     winning face carries an interpolated flag > 0.5, source = round-half-even(carried * (W-1, H-1));
+ *   n_corr[b]         device int32, rows of edit b;
+ *   pix_to_face       optional (B,H,W) int32, joined face index or -1.
+ * V_fg = 0 or F_fg = 0 is valid (no correspondences).  No allocation, no synchronisation; every check runs before any CUDA call:
+ * DH_ERR_INVALID_ARGUMENT for NULL required pointers, B < 1, V_bg < 1, negative counts, F_fg > 0 without vertices,
+ * blur_radius < 0; DH_ERR_UNSUPPORTED for B > 65535, H*W > 2^29, B*V_fg or F_bg + F_fg above 2^31 - 1.  The workspace query
+ * returns 0 for sizes the call rejects. */
+size_t dh_edit_mesh_batch_workspace_bytes(int B, int V_bg, int V_fg, int H, int W);
+int dh_edit_mesh_batch(const float* bg_verts, int V_bg, const int32_t* bg_faces, int F_bg,
+                       const float* fg_verts, const float* fg_colors, int V_fg, const int32_t* fg_faces, int F_fg,
+                       int B, const float* angles_deg_host, const float* axes_host, const float* translations_host,
+                       int H, int W, const float* R_host9, const float* T_host3, float sx, float sy, float blur_radius,
+                       int cull_backfaces, int perspective_correct, int clip_barycentric,
+                       float* target_z, int64_t* corr, int32_t* n_corr, int32_t* pix_to_face, void* ws, size_t ws_bytes,
+                       void* stream);
+
 #if defined(__GNUC__)
 #pragma GCC visibility pop
 #endif
