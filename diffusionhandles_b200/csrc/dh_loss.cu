@@ -1408,33 +1408,67 @@ static int choose_launch(const LaunchCache& lc, int grid, bool any_small, int n_
       K<64, false, 1, kMaxGroups>, K<64, true, 1, kMaxGroups>, K<64, false, 2, kMaxGroups>, K<64, true, 2, kMaxGroups>, \
       K<64, false, 1, 4>, K<64, true, 1, 4> }
 
+// Launches the edits bp.edit[0, n_edits) that prepare_edit filled (one grid, fg_kind and bg_kind).  One edit runs
+// loss_fused_kernel with bp.edit[0] alone, the 16x smaller parameter block; several run loss_fused_batch_kernel with all of bp.
+static int launch_edits(FusedBatchParams& bp, const EditLaunchInfo* info, int n_edits, int grid, void* stream) {
+    int n_items = 0, ell_words = 0, tab_words = 0, scratch_floats = 0;
+    bool any_small = false, tab_ok = true, binary = true;
+    for (int e = 0; e < n_edits; ++e) {
+        n_items += info[e].n_items;
+        ell_words = std::max(ell_words, info[e].ell_words);
+        tab_words = std::max(tab_words, info[e].tab_words);
+        scratch_floats = std::max(scratch_floats, bp.edit[e].scratch_floats);
+        any_small |= bp.edit[e].n_small_items > 0;
+        tab_ok &= info[e].tab_ok;
+        binary &= info[e].binary;
+    }
+    LaunchCache* lc = nullptr;
+    int rc = launch_cache(&lc);
+    if (rc != DH_OK) return rc;
+    if (n_edits > lc->sms) return DH_ERR_UNSUPPORTED;      // (the one check that needs the device; no GPU has fewer than 16 SMs)
+    LaunchChoice ch;
+    if ((rc = choose_launch(*lc, grid, any_small, n_items, ell_words, tab_words, tab_ok, scratch_floats, binary, ch)) != DH_OK) return rc;
+    // CTAs in proportion to the work items, at least one per edit, at most sms in all; no group of an edit sits idle.  For one
+    // edit this is min(sms, ceil(n_items / groups)) CTAs: the whole GPU, fewer when it would leave groups without an item.
+    int n_ctas = 0;
+    for (int e = 0; e < n_edits; ++e) {
+        FusedParams& fp = bp.edit[e];
+        fp.ell_floats = ch.mem >= 1 ? ell_words : 0;
+        fp.tab_floats = ch.mem == 2 ? tab_words : 0;
+        fp.scratch_floats = scratch_floats;
+        int share = 1 + (int)((long long)(lc->sms - n_edits) * info[e].n_items / n_items);
+        const int cap = (info[e].n_items + ch.groups - 1) / ch.groups;
+        if (share > cap) share = cap;
+        bp.cta_begin[e] = n_ctas;
+        n_ctas += share;
+    }
+    bp.cta_begin[n_edits] = n_ctas;
+    bp.n_edits = n_edits;
+    static const struct {
+        void (*one[10])(const FusedParams);
+        void (*many[10])(const FusedBatchParams);
+    } kernels = {DH_LOSS_VARIANTS(loss_fused_kernel), DH_LOSS_VARIANTS(loss_fused_batch_kernel)};
+    const bool batch = n_edits > 1;
+    size_t& attr_set = lc->smem_attr_set[10 * batch + ch.vi];
+    if (ch.smem > attr_set) {
+        const void* kernel = batch ? (const void*)kernels.many[ch.vi] : (const void*)kernels.one[ch.vi];
+        DH_CUDA_CHECK(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)ch.smem));
+        attr_set = ch.smem;
+    }
+    if (batch) kernels.many[ch.vi]<<<n_ctas, kLossThreads * ch.groups, ch.smem, as_stream(stream)>>>(bp);
+    else kernels.one[ch.vi]<<<n_ctas, kLossThreads * ch.groups, ch.smem, as_stream(stream)>>>(bp.edit[0]);
+    DH_LAUNCH_CHECK();
+    return DH_OK;
+}
+
 int dh_guidance_loss(const dh_loss_layer* layers_host, int n_layers, int grid, const void* plan, const dh_loss_plan_desc* desc,
                      int n_fg, int n_bg_orig, int n_bg_trans, int n_bg_common, int fg_kind, int bg_kind, float* loss_out,
                      void* ws, size_t ws_bytes, void* stream) {
-    FusedParams fp;
+    FusedBatchParams bp;        // (only edit[0] is filled and read)
     EditLaunchInfo info;
-    int rc = prepare_edit(layers_host, n_layers, grid, plan, desc, n_fg, n_bg_orig, n_bg_trans, n_bg_common, fg_kind, bg_kind, loss_out,
-                          ws, ws_bytes, false, fp, info);
-    if (rc != DH_OK) return rc;
-    LaunchCache* lc = nullptr;
-    if ((rc = launch_cache(&lc)) != DH_OK) return rc;
-    LaunchChoice ch;
-    rc = choose_launch(*lc, grid, fp.n_small_items > 0, info.n_items, info.ell_words, info.tab_words, info.tab_ok, fp.scratch_floats,
-                       info.binary, ch);
-    if (rc != DH_OK) return rc;
-    if (ch.mem >= 1) fp.ell_floats = info.ell_words;
-    if (ch.mem == 2) fp.tab_floats = info.tab_words;
-    static void (*const kernels[10])(const FusedParams) = DH_LOSS_VARIANTS(loss_fused_kernel);
-    void (*kernel)(const FusedParams) = kernels[ch.vi];
-    if (ch.smem > lc->smem_attr_set[ch.vi]) {
-        DH_CUDA_CHECK(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)ch.smem));
-        lc->smem_attr_set[ch.vi] = ch.smem;
-    }
-    int grid_x = lc->sms;
-    if (grid_x * ch.groups > info.n_items) grid_x = (info.n_items + ch.groups - 1) / ch.groups;
-    kernel<<<grid_x, kLossThreads * ch.groups, ch.smem, as_stream(stream)>>>(fp);
-    DH_LAUNCH_CHECK();
-    return DH_OK;
+    const int rc = prepare_edit(layers_host, n_layers, grid, plan, desc, n_fg, n_bg_orig, n_bg_trans, n_bg_common, fg_kind, bg_kind,
+                                loss_out, ws, ws_bytes, false, bp.edit[0], info);
+    return rc != DH_OK ? rc : launch_edits(bp, &info, 1, grid, stream);
 }
 
 size_t dh_guidance_loss_batch_workspace_bytes(int n_edits, int n_layers, int max_channels) {
@@ -1451,8 +1485,6 @@ int dh_guidance_loss_batch(const dh_loss_batch_edit* edits_host, int n_edits, in
     EditLaunchInfo info[kMaxBatchEdits];
     // edit e owns bytes [e * stride, (e + 1) * stride) of the workspace
     const size_t stride = ws_bytes / (size_t)n_edits / 16 * 16;
-    int n_items = 0, ell_words = 0, tab_words = 0, scratch_floats = 0;
-    bool any_small = false, tab_ok = true, binary = true;
     for (int e = 0; e < n_edits; ++e) {
         const dh_loss_batch_edit& E = edits_host[e];
         const int rc = prepare_edit(E.layers, E.n_layers, grid, E.plan, &E.desc, E.n_fg, E.n_bg_orig, E.n_bg_trans, E.n_bg_common, fg_kind,
@@ -1462,44 +1494,8 @@ int dh_guidance_loss_batch(const dh_loss_batch_edit* edits_host, int n_edits, in
         // plan and keeps the plan in global memory, but a batch may place the other edits' plans in shared memory, sized by
         // their descriptors - this edit's copy would not fit there
         if (fg_kind && E.n_fg > 0 && info[e].ell_words == 0) return DH_ERR_INVALID_ARGUMENT;
-        n_items += info[e].n_items;
-        ell_words = std::max(ell_words, info[e].ell_words);
-        tab_words = std::max(tab_words, info[e].tab_words);
-        scratch_floats = std::max(scratch_floats, bp.edit[e].scratch_floats);
-        any_small |= bp.edit[e].n_small_items > 0;
-        tab_ok &= info[e].tab_ok;
-        binary &= info[e].binary;
     }
-    LaunchCache* lc = nullptr;
-    int rc = launch_cache(&lc);
-    if (rc != DH_OK) return rc;
-    if (n_edits > lc->sms) return DH_ERR_UNSUPPORTED;      // (the one check that needs the device; no GPU has fewer than 16 SMs)
-    LaunchChoice ch;
-    if ((rc = choose_launch(*lc, grid, any_small, n_items, ell_words, tab_words, tab_ok, scratch_floats, binary, ch)) != DH_OK) return rc;
-    // CTAs in proportion to the work items, at least one per edit, at most sms in all; no group of an edit sits idle
-    int n_ctas = 0;
-    for (int e = 0; e < n_edits; ++e) {
-        FusedParams& fp = bp.edit[e];
-        fp.ell_floats = ch.mem >= 1 ? ell_words : 0;
-        fp.tab_floats = ch.mem == 2 ? tab_words : 0;
-        fp.scratch_floats = scratch_floats;
-        int share = 1 + (int)((long long)(lc->sms - n_edits) * info[e].n_items / n_items);
-        const int cap = (info[e].n_items + ch.groups - 1) / ch.groups;
-        if (share > cap) share = cap;
-        bp.cta_begin[e] = n_ctas;
-        n_ctas += share;
-    }
-    bp.cta_begin[n_edits] = n_ctas;
-    bp.n_edits = n_edits;
-    static void (*const kernels[10])(const FusedBatchParams) = DH_LOSS_VARIANTS(loss_fused_batch_kernel);
-    void (*kernel)(const FusedBatchParams) = kernels[ch.vi];
-    if (ch.smem > lc->smem_attr_set[10 + ch.vi]) {
-        DH_CUDA_CHECK(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)ch.smem));
-        lc->smem_attr_set[10 + ch.vi] = ch.smem;
-    }
-    kernel<<<n_ctas, kLossThreads * ch.groups, ch.smem, as_stream(stream)>>>(bp);
-    DH_LAUNCH_CHECK();
-    return DH_OK;
+    return launch_edits(bp, info, n_edits, grid, stream);
 }
 
 int dh_scale_inplace(float* data, size_t n, const float* scale, void* stream) {

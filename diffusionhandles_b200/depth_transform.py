@@ -233,6 +233,20 @@ def _empty_mask_result(depth, use_input_depth_normalization):
     return normalize_depth(disparity, bounds=bounds), torch.empty((0, 4), dtype=torch.int64)
 
 
+def _edit_count(rot_angles, rot_axes, translations) -> int:
+    B = len(rot_angles)
+    if B < 1 or len(rot_axes) != B or len(translations) != B:
+        raise ValueError(f"rot_angles, rot_axes and translations must have one entry per edit (at least one), got {B}, "
+                         f"{len(rot_axes)}, {len(translations)}")
+    return B
+
+
+def _empty_mask_batch(depth, use_input_depth_normalization, B):
+    """``_empty_mask_result`` for each of B edits."""
+    disparity, corr = _empty_mask_result(depth, use_input_depth_normalization)
+    return disparity.repeat(B, 1, 1, 1), [corr.clone() for _ in range(B)]
+
+
 def transform_depth_pc(depth: torch.Tensor, bg_depth: torch.Tensor, fg_mask: torch.Tensor, intrinsics: torch.Tensor,
                        rot_angle: float = None, rot_axis: torch.Tensor = None, translation: torch.Tensor = None,
                        use_input_depth_normalization=False, return_device_result: bool = False):
@@ -242,8 +256,21 @@ def transform_depth_pc(depth: torch.Tensor, bg_depth: torch.Tensor, fg_mask: tor
     With ``return_device_result=True`` a third value, the device-side ``EditResult`` (winner indices, masks,
     device copy of the correspondences), is appended for the warp / loss kernels.
     """
+    disparity, corrs, res = transform_depth_pc_batch(depth, bg_depth, fg_mask, intrinsics, [rot_angle], [rot_axis], [translation],
+                                                     use_input_depth_normalization, return_device_result=True)
+    return (disparity, corrs[0], res) if return_device_result else (disparity, corrs[0])
+
+
+def transform_depth_pc_batch(depth: torch.Tensor, bg_depth: torch.Tensor, fg_mask: torch.Tensor, intrinsics: torch.Tensor,
+                             rot_angles, rot_axes, translations, use_input_depth_normalization=False,
+                             return_device_result: bool = False):
+    """``transform_depth_pc`` for B transforms of one scene as ONE ``EditEngine`` batch.  ``rot_angles`` / ``rot_axes`` /
+    ``translations`` hold one entry per edit (``None`` takes the defaults of the single call).  Returns ``(disparities
+    (B,1,S,S) fp32 on depth.device, [correspondences (n_b,4) int64 CPU] * B)``, plus the ``EditResult`` (None for an empty
+    mask) with ``return_device_result=True``."""
+    B = _edit_count(rot_angles, rot_axes, translations)
     if not fg_mask.any():
-        res = _empty_mask_result(depth, use_input_depth_normalization)
+        res = _empty_mask_batch(depth, use_input_depth_normalization, B)
         return (*res, None) if return_device_result else res
     S = fg_mask.shape[-1]
     if fg_mask.shape[-2] != S:
@@ -252,20 +279,16 @@ def transform_depth_pc(depth: torch.Tensor, bg_depth: torch.Tensor, fg_mask: tor
         raise ValueError(f"one image per call (batch size 1), got a batch of {depth.shape[0]}")
     _require_cuda(depth, "depth")
     # defaults of the reference: no rotation about +y, no translation (depth_transform.py:219-224)
-    rot_angle = 0.0 if rot_angle is None else rot_angle
-    rot_axis = torch.tensor([0.0, 1.0, 0.0]) if rot_axis is None else rot_axis
-    translation = torch.zeros(3) if translation is None else translation
-    dev = depth.device
-    eng = get_engine(dev, 1, S, S)
-    f32 = torch.float32
-    d = depth.reshape(1, S, S).to(f32).contiguous()
-    b = bg_depth.reshape(1, S, S).to(device=dev, dtype=f32).contiguous()
-    m = fg_mask.reshape(1, S, S).to(device=dev, dtype=f32).contiguous()
-    res = eng.run(d, b, m, intrinsics, [make_rigid(rot_angle, rot_axis, translation)],
-                  use_input_depth_normalization=use_input_depth_normalization, poisson=True)
-    corr = res.correspondences(0).cpu()
-    disparity = res.disparity[0][None, None].clone()
-    return (disparity, corr, res) if return_device_result else (disparity, corr)
+    rigids = [make_rigid(0.0 if a is None else a, torch.tensor([0.0, 1.0, 0.0]) if ax is None else ax,
+                         torch.zeros(3) if t is None else t) for a, ax, t in zip(rot_angles, rot_axes, translations)]
+    dev, f32 = depth.device, torch.float32
+    d = depth.reshape(1, S, S).to(f32).expand(B, S, S).contiguous()
+    b = bg_depth.reshape(1, S, S).to(device=dev, dtype=f32).expand(B, S, S).contiguous()
+    m = fg_mask.reshape(1, S, S).to(device=dev, dtype=f32).expand(B, S, S).contiguous()
+    res = get_engine(dev, B, S, S).run(d, b, m, intrinsics, rigids, use_input_depth_normalization=use_input_depth_normalization,
+                                       poisson=True)
+    out = res.disparity[:, None].clone(), [res.correspondences(e).cpu() for e in range(B)]
+    return (*out, res) if return_device_result else out
 
 
 def transform_depth_mesh(depth: torch.Tensor, bg_depth: torch.Tensor, fg_mask: torch.Tensor, intrinsics: torch.Tensor,
@@ -274,33 +297,11 @@ def transform_depth_mesh(depth: torch.Tensor, bg_depth: torch.Tensor, fg_mask: t
     """depth_transform.py:91-195 - opt-in mesh mode: triangulate both depth maps, move the foreground mesh, rasterise the
     scene (hard z-buffer, back faces culled, blur 1e-5) and read depth and source coordinates off the render layers.
     Correspondences are enumerated over TARGET pixels in raster order; no mask cleaning and no hole fill (as in the
-    reference).  The rasteriser follows pytorch3d's published semantics; bit parity with pytorch3d is unpinned."""
-    from .pytorch3d_renderer import PyTorch3DRenderer, PyTorch3DRendererArgs
-    from .renderer import Camera
-    if not fg_mask.any():
-        return _empty_mask_result(depth, use_input_depth_normalization)
-    _require_cuda(depth, "depth")
-    dev = depth.device
-    H, W = depth.shape[-2], depth.shape[-1]
-    angle = torch.tensor(0.0 if rot_angle is None else float(rot_angle), dtype=torch.float32)
-    axis = torch.tensor([0.0, 1.0, 0.0], device=dev) if rot_axis is None else rot_axis
-    shift = torch.zeros(3, device=dev) if translation is None else translation
-    background = depth_to_mesh(depth=bg_depth, intrinsics=intrinsics)
-    foreground = depth_to_mesh(depth=depth, intrinsics=intrinsics, mask=fg_mask[0, 0] > 0.5)
-    foreground.verts = transform_points(points=foreground.verts, rot_angle=angle, rot_axis=axis, translation=shift)
-    renderer = PyTorch3DRenderer(output_names=['world_position', 'flat_vertex_color'],
-                                 args=PyTorch3DRendererArgs(device=dev, output_res=(H, W), cull_backfaces=True, blur_radius=1e-5))
-    renderer.update_scene(scene_elements={'meshes': [background, foreground], 'cameras': [Camera(intrinsics=intrinsics)]})
-    layers = renderer.render()
-    target_depth = layers['world_position'][None, ..., 2]                   # (1,1,H,W): world z of the visible surface
-    carried = layers['flat_vertex_color'][0]                                # (H,W,4): source x/(W-1), y/(H-1), fg flag, alpha
-    # one correspondence per target pixel that shows the foreground mesh, in target raster order; the destination is the
-    # pixel itself, the source the carried normalised coordinate scaled back to pixels and rounded half-to-even
-    ty, tx = torch.nonzero(carried[..., 2] > 0.5, as_tuple=True)
-    source = torch.round(carried[ty, tx, :2] * carried.new_tensor([W - 1, H - 1])).to(torch.int64)
-    correspondences = torch.stack([source[:, 0], source[:, 1], tx, ty], dim=-1).to(device='cpu')
-    bounds = normalize_depth(1.0 / depth, return_bounds=True)[1] if use_input_depth_normalization else None
-    return normalize_depth(1.0 / target_depth, bounds=bounds), correspondences
+    reference).  The rasteriser follows pytorch3d's published semantics; bit parity with pytorch3d is unpinned.  Runs as
+    ``transform_depth_mesh_batch`` with one transform."""
+    disparity, corrs = transform_depth_mesh_batch(depth, bg_depth, fg_mask, intrinsics, [rot_angle], [rot_axis], [translation],
+                                                  use_input_depth_normalization)
+    return disparity, corrs[0]
 
 
 def transform_depth_mesh_batch(depth: torch.Tensor, bg_depth: torch.Tensor, fg_mask: torch.Tensor, intrinsics: torch.Tensor,
@@ -310,16 +311,12 @@ def transform_depth_mesh_batch(depth: torch.Tensor, bg_depth: torch.Tensor, fg_m
     Both meshes are built once; the background mesh is rasterised once and every edit's moved foreground faces are rasterised
     over a copy of its z-buffer, which gives the z-buffer of the joined mesh bit for bit.  ``rot_angles`` / ``rot_axes`` /
     ``translations`` hold one entry per edit (``None`` takes the defaults of the single call).  Returns ``(disparities
-    (B,1,H,W) fp32 on depth.device, [correspondences (n_b,4) int64 CPU] * B)``; entry b equals ``transform_depth_mesh`` with
-    transform b bit for bit."""
+    (B,1,H,W) fp32 on depth.device, [correspondences (n_b,4) int64 CPU] * B)``; entry b equals bit for bit what the
+    renderer reads off the joined mesh [background, foreground moved by transform b]."""
     from .renderer import MeshRenderer, fov_scales
-    B = len(rot_angles)
-    if B < 1 or len(rot_axes) != B or len(translations) != B:
-        raise ValueError(f"rot_angles, rot_axes and translations must have one entry per edit (at least one), got {B}, "
-                         f"{len(rot_axes)}, {len(translations)}")
+    B = _edit_count(rot_angles, rot_axes, translations)
     if not fg_mask.any():
-        disparity, corr = _empty_mask_result(depth, use_input_depth_normalization)
-        return disparity.expand(B, *disparity.shape[1:]).clone(), [corr.clone() for _ in range(B)]
+        return _empty_mask_batch(depth, use_input_depth_normalization, B)
     _require_cuda(depth, "depth")
     lib = N.load()
     dev = depth.device

@@ -11,8 +11,7 @@ from types import SimpleNamespace
 
 import torch
 
-from .depth_transform import _require_cuda, normalize_depth, transform_depth, transform_depth_mesh_batch
-from .engine import get_engine, make_rigid
+from .depth_transform import normalize_depth, transform_depth, transform_depth_mesh_batch, transform_depth_pc_batch
 from .guided_stable_diffuser import GuidedStableDiffuser
 
 DEFAULT_CONF = SimpleNamespace(   # diffhandles/config/default.yaml
@@ -108,32 +107,15 @@ class DiffusionHandles:
     def edit_geometry_batch(self, depth: torch.Tensor, fg_mask: torch.Tensor, bg_depth: torch.Tensor, rot_angles, rot_axes,
                             translations, use_input_depth_normalization=False):
         """B transforms of one scene: edited disparities (B,1,H,W) and a list of B correspondence lists, each equal bit for bit
-        to ``edit_geometry`` with that transform.  In 'pc' mode the B edits are ONE ``EditEngine`` batch; in 'mesh' mode they are
-        ONE ``transform_depth_mesh_batch`` call (the background mesh rasterised once); an empty mask in 'pc' mode runs
-        ``edit_geometry`` per transform."""
-        B = len(rot_angles)
-        if len(rot_axes) != B or len(translations) != B:
-            raise ValueError(f"rot_angles, rot_axes and translations must have one entry per edit, got {B}, {len(rot_axes)}, {len(translations)}")
-        S = fg_mask.shape[-1]
+        to ``edit_geometry`` with that transform.  In 'pc' mode the B edits are ONE ``EditEngine`` batch
+        (``transform_depth_pc_batch``); in 'mesh' mode they are ONE ``transform_depth_mesh_batch`` call (the background mesh
+        rasterised once)."""
+        batch = {"pc": transform_depth_pc_batch, "mesh": transform_depth_mesh_batch}.get(self.conf.depth_transform_mode)
+        if batch is None:
+            raise ValueError(f"Unknown depth transform mode '{self.conf.depth_transform_mode}'.")
         with torch.no_grad():
-            if self.conf.depth_transform_mode == "mesh" and B > 0:
-                return transform_depth_mesh_batch(depth, bg_depth, fg_mask, self.diffuser.get_depth_intrinsics(device=depth.device),
-                                                  rot_angles, rot_axes, translations, use_input_depth_normalization)
-            if self.conf.depth_transform_mode != "pc" or not fg_mask.any() or fg_mask.shape[-2] != S or depth.shape[0] != 1:
-                outs = [self.edit_geometry(depth, fg_mask, bg_depth, a, ax, t, use_input_depth_normalization)
-                        for a, ax, t in zip(rot_angles, rot_axes, translations)]
-                return torch.cat([d for d, _ in outs]), [c for _, c in outs]
-            _require_cuda(depth, "depth")
-            dev, f32 = depth.device, torch.float32
-            # the defaults of transform_depth_pc: no rotation about +y, no translation
-            rigids = [make_rigid(0.0 if a is None else a, torch.tensor([0.0, 1.0, 0.0]) if ax is None else ax,
-                                 torch.zeros(3) if t is None else t) for a, ax, t in zip(rot_angles, rot_axes, translations)]
-            d = depth.reshape(1, S, S).to(f32).expand(B, S, S).contiguous()
-            b = bg_depth.reshape(1, S, S).to(device=dev, dtype=f32).expand(B, S, S).contiguous()
-            m = fg_mask.reshape(1, S, S).to(device=dev, dtype=f32).expand(B, S, S).contiguous()
-            res = get_engine(dev, B, S, S).run(d, b, m, self.diffuser.get_depth_intrinsics(device=dev), rigids,
-                                               use_input_depth_normalization=use_input_depth_normalization, poisson=True)
-            return res.disparity[:, None].clone(), [res.correspondences(e).cpu() for e in range(B)]
+            return batch(depth, bg_depth, fg_mask, self.diffuser.get_depth_intrinsics(device=depth.device), rot_angles, rot_axes,
+                         translations, use_input_depth_normalization)
 
     def transform_foreground_batch(self, depth: torch.Tensor, prompt: str, fg_mask: torch.Tensor, bg_depth: torch.Tensor,
                                    null_text_emb: torch.Tensor, init_noise: torch.Tensor, activations: list, rot_angles, rot_axes,

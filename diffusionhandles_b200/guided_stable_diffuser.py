@@ -206,11 +206,38 @@ class GuidedStableDiffuser:
         the latents driven by sum_l fgw[l] L_fg,l + bgw[l] L_bg,l (ONE fused K4 launch per evaluation, :415-434), then the
         classifier-free-guidance forward (scale 7.5, :452-470) and the scheduler step; finally the VAE decode.  Needs the
         injected diffusion models; without them this raises NotImplementedError (they are outside this build)."""
-        from .guided_loop import guided_denoise
+        return self._guided_inference(False, latents, depth, uncond_embeddings, prompt, activations_orig, correspondences, fg_weight,
+                                      bg_weight, save_denoising_steps)
+
+    def guided_inference_batch(self, latents: torch.Tensor, depth: torch.Tensor, uncond_embeddings: torch.Tensor, prompt: str,
+                               activations_orig, correspondences, fg_weight: float = None, bg_weight: float = None):
+        """``guided_inference`` for B edits at once (``guided_denoise_batch``): the U-Net runs at batch B, each guided step
+        evaluates the losses of all edits in one K4 launch.  ``depth`` is (B,1,H,W), ``correspondences`` a list of B (N,4)
+        lists; ``latents`` (1,4,h,w) is shared by every edit, or (B,4,h,w); ``activations_orig`` is one identity shared by every
+        edit, or a list of B identities.  Returns the B decoded images.  The saved denoising steps of ``save_denoising_steps``
+        are not supported here."""
+        return self._guided_inference(True, latents, depth, uncond_embeddings, prompt, activations_orig, correspondences, fg_weight,
+                                      bg_weight, False)
+
+    def _guided_inference(self, batch, latents, depth, uncond_embeddings, prompt, activations_orig, correspondences, fg_weight,
+                          bg_weight, save_denoising_steps):
+        """The body of ``guided_inference`` (batch=False: one edit, ``guided_denoise``) and ``guided_inference_batch``
+        (batch=True: B edits, ``guided_denoise_batch``)."""
+        from .guided_loop import guided_denoise, guided_denoise_batch
+        name = "guided_inference_batch" if batch else "guided_inference"
         missing = [n for n in ("unet", "scheduler") if getattr(self, n) is None]
         if missing:
-            raise NotImplementedError(f"guided_inference needs the stock diffusion models ({', '.join(missing)}); pass them to "
+            raise NotImplementedError(f"{name} needs the stock diffusion models ({', '.join(missing)}); pass them to "
                                       "GuidedStableDiffuser(conf, unet=..., scheduler=..., vae=..., tokenizer=..., text_encoder=...)")
+        corrs = correspondences if batch else [correspondences]
+        B = len(corrs)
+        if batch:
+            if self._conf("save_denoising_steps", False):
+                raise NotImplementedError("guided_inference_batch does not save the denoising steps; use guided_inference per edit")
+            if depth.shape[0] != B:
+                raise ValueError(f"depth must be (B,1,H,W) with B = {B} edits, got {tuple(depth.shape)}")
+            if latents.shape[0] not in (1, B):
+                raise ValueError(f"latents must be (1,4,h,w) or ({B},4,h,w), got {tuple(latents.shape)}")
         fg_weight = self._conf("fg_weight", 1.5) if fg_weight is None else fg_weight
         bg_weight = self._conf("bg_weight", 1.25) if bg_weight is None else bg_weight
         use_depth = self._conf("use_depth", True)
@@ -219,11 +246,14 @@ class GuidedStableDiffuser:
             n_steps = self._conf("num_timesteps", 50)
             self.scheduler.set_timesteps(n_steps, device=self.device)
             timesteps, _ = self.get_timesteps(n_steps, 1.0)
-            pc = self.process_correspondences(correspondences, img_res=depth.shape[-1], bg_erosion=self._conf("bg_erosion", 0))
+            pcs = [self.process_correspondences(c, img_res=depth.shape[-1], bg_erosion=self._conf("bg_erosion", 0)) for c in corrs]
             if use_depth:
                 depth = self.init_depth(depth)
             cond = self._encode_prompt(prompt)
             extra = self.prepare_extra_step_kwargs(generator, 0.0)
+            if batch:
+                cond = cond.expand(B, *cond.shape[1:])
+                latents = latents.expand(B, *latents.shape[1:]).contiguous()
 
         def unet_fn(model_in, t):
             if use_depth:
@@ -245,15 +275,15 @@ class GuidedStableDiffuser:
         steps = {'opt': [], 'post-opt': []} if save_denoising_steps else None
 
         def on_step(kind, lat):
-            if steps is not None:
-                if kind == 'opt':
-                    steps['opt'].append([self.decode_latent_image(lat.detach()).cpu()])
-                else:
-                    steps['opt'][-1].append(self.decode_latent_image(lat.detach()).cpu())
+            if kind == 'opt':
+                steps['opt'].append([self.decode_latent_image(lat.detach()).cpu()])
+            else:
+                steps['opt'][-1].append(self.decode_latent_image(lat.detach()).cpu())
 
-        latents = guided_denoise(
+        denoise = guided_denoise_batch if batch else guided_denoise
+        latents = denoise(
             latents, timesteps, unet_fn, lambda noise, t, lat: self.scheduler.step(noise, t, lat, **extra, return_dict=False)[0],
-            activations_orig, pc, fg_weight=fg_weight, bg_weight=bg_weight, num_optsteps=self._conf("num_optsteps", 3),
+            activations_orig, pcs if batch else pcs[0], fg_weight=fg_weight, bg_weight=bg_weight, num_optsteps=self._conf("num_optsteps", 3),
             guidance_max_step=self._conf("guidance_max_step", 38), guidance_schedule_type=self._conf("guidance_schedule_type", "constant"),
             bg_loss_type=self._conf("bg_loss_type", "global_avg"), fg_patch_size=self._conf("fg_patch_size", 1),
             bg_patch_size=self._conf("bg_patch_size", 1), scale_model_input=self.scheduler.scale_model_input, cfg_noise=cfg_noise,
@@ -264,65 +294,6 @@ class GuidedStableDiffuser:
         with torch.no_grad():
             image = self.decode_latent_image(latents)
         return (image, steps) if save_denoising_steps else image
-
-    def guided_inference_batch(self, latents: torch.Tensor, depth: torch.Tensor, uncond_embeddings: torch.Tensor, prompt: str,
-                               activations_orig, correspondences, fg_weight: float = None, bg_weight: float = None):
-        """``guided_inference`` for B edits at once (``guided_denoise_batch``): the U-Net runs at batch B, each guided step
-        evaluates the losses of all edits in one K4 launch.  ``depth`` is (B,1,H,W), ``correspondences`` a list of B (N,4)
-        lists; ``latents`` (1,4,h,w) is shared by every edit, or (B,4,h,w); ``activations_orig`` is one identity shared by every
-        edit, or a list of B identities.  Returns the B decoded images.  The saved denoising steps of ``save_denoising_steps``
-        are not supported here."""
-        from .guided_loop import guided_denoise_batch
-        missing = [n for n in ("unet", "scheduler") if getattr(self, n) is None]
-        if missing:
-            raise NotImplementedError(f"guided_inference_batch needs the stock diffusion models ({', '.join(missing)}); pass them to "
-                                      "GuidedStableDiffuser(conf, unet=..., scheduler=..., vae=..., tokenizer=..., text_encoder=...)")
-        if self._conf("save_denoising_steps", False):
-            raise NotImplementedError("guided_inference_batch does not save the denoising steps; use guided_inference per edit")
-        B = len(correspondences)
-        if depth.shape[0] != B:
-            raise ValueError(f"depth must be (B,1,H,W) with B = {B} edits, got {tuple(depth.shape)}")
-        if latents.shape[0] not in (1, B):
-            raise ValueError(f"latents must be (1,4,h,w) or ({B},4,h,w), got {tuple(latents.shape)}")
-        fg_weight = self._conf("fg_weight", 1.5) if fg_weight is None else fg_weight
-        bg_weight = self._conf("bg_weight", 1.25) if bg_weight is None else bg_weight
-        use_depth = self._conf("use_depth", True)
-        with torch.no_grad():
-            generator = torch.manual_seed(self._conf("seed", 2773))
-            n_steps = self._conf("num_timesteps", 50)
-            self.scheduler.set_timesteps(n_steps, device=self.device)
-            timesteps, _ = self.get_timesteps(n_steps, 1.0)
-            pcs = [self.process_correspondences(c, img_res=depth.shape[-1], bg_erosion=self._conf("bg_erosion", 0)) for c in correspondences]
-            if use_depth:
-                depth = self.init_depth(depth)
-            cond = self._encode_prompt(prompt)
-            cond = cond.expand(B, *cond.shape[1:])
-            extra = self.prepare_extra_step_kwargs(generator, 0.0)
-            latents = latents.expand(B, *latents.shape[1:]).contiguous()
-
-        def unet_fn(model_in, t):
-            if use_depth:
-                model_in = torch.cat([model_in, depth], dim=1)
-            out = self.unet(model_in, t, encoder_hidden_states=cond, cross_attention_kwargs=None, return_dict=False)
-            return out[0], [out[4], out[5], out[6]]
-
-        def cfg_pair(lat, t, t_idx):
-            return self._cfg_forward(lat, t, uncond_embeddings[t_idx], cond, depth if use_depth else None)
-
-        def cfg_noise(lat, t, t_idx):
-            n_uncond, n_text = cfg_pair(lat, t, t_idx)
-            return n_uncond + 7.5 * (n_text - n_uncond)
-
-        ddim = self._fused_ddim()
-        latents = guided_denoise_batch(
-            latents, timesteps, unet_fn, lambda noise, t, lat: self.scheduler.step(noise, t, lat, **extra, return_dict=False)[0],
-            activations_orig, pcs, fg_weight=fg_weight, bg_weight=bg_weight, num_optsteps=self._conf("num_optsteps", 3),
-            guidance_max_step=self._conf("guidance_max_step", 38), guidance_schedule_type=self._conf("guidance_schedule_type", "constant"),
-            bg_loss_type=self._conf("bg_loss_type", "global_avg"), fg_patch_size=self._conf("fg_patch_size", 1),
-            bg_patch_size=self._conf("bg_patch_size", 1), scale_model_input=self.scheduler.scale_model_input, cfg_noise=cfg_noise,
-            ddim=ddim, cfg_pair=cfg_pair if ddim is not None else None, skip_zero_weight_layers=True)
-        with torch.no_grad():
-            return self.decode_latent_image(latents)
 
     def _fused_ddim(self):
         """DDIMSchedule of the injected scheduler when the fused update reproduces its step(), else None."""

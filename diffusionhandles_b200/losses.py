@@ -131,6 +131,21 @@ def _needs_general(shapes, grid: int, patch: int, bg_kind: int) -> bool:
             or (bg_kind == _BG_LOCAL and any((sh[1], sh[2]) != (grid, grid) for sh in shapes)))
 
 
+def _layers(plan: LossPlan, shapes, fg_kind: int, bg_kind: int, general: bool):
+    """The ctypes ``dh_loss_layer`` array of one plan for layers of these (C,h,w) shapes, with the resize tables of the layers
+    smaller than the loss grid (the general patch kernel takes none).  Returns (layers, tables); the caller keeps both alive."""
+    layers = (N.dh_loss_layer * len(shapes))()
+    tabs = []
+    for i, sh in enumerate(shapes):
+        if sh[1] > plan.grid or sh[2] > plan.grid:
+            raise NotImplementedError(f"activation maps larger than the loss grid ({sh[1]}x{sh[2]} > {plan.grid}) are not implemented")
+        layers[i].channels, layers[i].h, layers[i].w = sh
+        t = plan.resize_tables(sh[1], sh[2], fg_kind, bg_kind) if not general and (sh[1], sh[2]) != (plan.grid, plan.grid) else None
+        tabs.append(t)
+        layers[i].resize_tables = N.ptr(t) if t is not None else None
+    return layers, tabs
+
+
 def _launch(curs: Sequence[torch.Tensor], origs: Sequence[torch.Tensor], want_grad: Sequence[bool],
             fgw: Sequence[float], bgw: Sequence[float], plan: LossPlan, fg_kind: int,
             bg_kind: int, patch: int = 1) -> Tuple[torch.Tensor, List[Optional[torch.Tensor]]]:
@@ -148,17 +163,7 @@ def _launch(curs: Sequence[torch.Tensor], origs: Sequence[torch.Tensor], want_gr
         for c, o in zip(curs, origs):
             if c.dim() != 3 or tuple(c.shape) != tuple(o.shape):
                 raise ValueError("activations must be (C,h,w) with matching recorded activations")
-        layers = (N.dh_loss_layer * L)()
-        tabs = []
-        for i, sh in enumerate(shapes):
-            layers[i].channels, layers[i].h, layers[i].w = sh
-            if sh[1] > plan.grid or sh[2] > plan.grid:
-                raise NotImplementedError(f"activation maps larger than the loss grid ({sh[1]}x{sh[2]} > {plan.grid}) are not implemented")
-            t = None
-            if not general and (sh[1], sh[2]) != (plan.grid, plan.grid):
-                t = plan.resize_tables(sh[1], sh[2], fg_kind, bg_kind)
-            tabs.append(t)
-            layers[i].resize_tables = N.ptr(t) if t is not None else None
+        layers, tabs = _layers(plan, shapes, fg_kind, bg_kind, general)
         ws_fn = lib.dh_guidance_loss_patch_workspace_bytes if general else lib.dh_guidance_loss_workspace_bytes
         ws_bytes = int(ws_fn(L, max(sh[0] for sh in shapes)))
         runner = (layers, torch.zeros(ws_bytes, dtype=torch.uint8, device=dev), ws_bytes, tabs)   # zero once: the kernel re-arms its queue counters
@@ -301,15 +306,9 @@ def _batch_runner(plans: Sequence[LossPlan], shapes, bg_kind: int):
         edits = (N.dh_loss_batch_edit * n)()
         layer_arrays, tabs = [], []
         for e, plan in enumerate(plans):
-            layers = (N.dh_loss_layer * L)()
-            for i, sh in enumerate(shapes):
-                if sh[1] > plan.grid or sh[2] > plan.grid:
-                    raise NotImplementedError(f"activation maps larger than the loss grid ({sh[1]}x{sh[2]} > {plan.grid}) are not implemented")
-                layers[i].channels, layers[i].h, layers[i].w = sh
-                t = plan.resize_tables(sh[1], sh[2], _FG, bg_kind) if (sh[1], sh[2]) != (plan.grid, plan.grid) else None
-                tabs.append(t)
-                layers[i].resize_tables = N.ptr(t) if t is not None else None
+            layers, t = _layers(plan, shapes, _FG, bg_kind, False)
             layer_arrays.append(layers)
+            tabs += t
             edits[e].layers = C.cast(layers, C.POINTER(N.dh_loss_layer))
             edits[e].n_layers = L
             edits[e].plan = plan.buf.data_ptr()
@@ -331,8 +330,8 @@ def guidance_loss_and_grad_batch(activations: Sequence[torch.Tensor], activation
     by every edit (variants of one image), or (B,C_l,h_l,w_l); ``processed_correspondences`` holds B dicts.  The weights are
     the same for every edit.  Returns (totals (B,), parts (B,2L), [grad_l (B,C_l,h_l,w_l)]): row / slice e is bit-identical to
     what ``guidance_loss_and_grad`` returns for edit e alone.  Inputs that the single-edit call sends to the general patch kernel
-    (patch_size > 1, map areas that are not a multiple of 4, 'local_avg' on resized layers) run one such launch per edit; a batch
-    of one edit runs the single-edit launch."""
+    (patch_size > 1, map areas that are not a multiple of 4, 'local_avg' on resized layers) run one such launch per edit.  A chunk
+    of one edit runs the single-edit kernel (dh_guidance_loss_batch picks it)."""
     if bg_loss_type not in ('global_avg', 'local_avg'):
         raise ValueError(f'Unknown background loss type: {bg_loss_type}')
     grid = _grid_of(activations_size)
@@ -352,10 +351,6 @@ def guidance_loss_and_grad_batch(activations: Sequence[torch.Tensor], activation
         raise N.NativeLibraryError("guidance losses run on CUDA only; there is no CPU fallback")
     plans = [_plan_for(pc, grid, dev) for pc in pcs]
     shapes = tuple(tuple(a.shape[1:]) for a in activations)
-    if B == 1:      # one edit: the single-edit launch (its parameter block is 16x smaller; same bits)
-        o, g = _launch([a[0] for a in activations], [o if o.dim() == 3 else o[0] for o in activations_orig], [True] * L,
-                       fg_weights, bg_weights, plans[0], _FG, bg_kind, patch)
-        return o[None, 0], o[None, 1:], [x[None] for x in g]
     out = torch.empty(B, 1 + 2 * L, dtype=torch.float32, device=dev)
     if _needs_general(shapes, grid, patch, bg_kind):
         grads = [torch.empty((B,) + sh, dtype=torch.float32, device=dev) for sh in shapes]

@@ -1,6 +1,6 @@
 """GPU (-m gpu): mesh mode for B transforms of one scene (depth_transform.transform_depth_mesh_batch / dh_edit_mesh_batch).
 The background mesh is rasterised once and every edit's moved foreground goes on top of a copy of its z-buffer; every edit
-must equal the single-edit path (transform_depth_mesh: joined mesh, one dh_rasterize_meshes per edit) bit for bit -
+must equal the joined-mesh renderer (MeshRenderer on [bg, moved fg], one dh_rasterize_meshes per edit) bit for bit -
 disparities and correspondences, values and order - and the NumPy oracle on the joined mesh."""
 import ctypes as C
 from types import SimpleNamespace
@@ -62,8 +62,8 @@ def _batch_vs_singles(td, tb, tm, K, edits, unn=False):
     disp, corrs = dt.transform_depth_mesh_batch(td, tb, tm, K, list(angles), list(axes), list(shifts), use_input_depth_normalization=unn)
     H, W = td.shape[-2:]
     assert disp.shape == (len(edits), 1, H, W) and disp.device == td.device and len(corrs) == len(edits)
-    for b, (a, ax, t) in enumerate(edits):
-        d1, c1 = dt.transform_depth_mesh(td, tb, tm, K, a, ax, t, use_input_depth_normalization=unn)
+    for b, edit in enumerate(edits):
+        d1, c1 = _joined_mesh_edit(td, tb, tm, K, edit, unn)
         assert _bits_equal(disp[b:b + 1], d1), b
         assert corrs[b].device.type == "cpu" and corrs[b].dtype == torch.int64
         assert torch.equal(corrs[b], c1), (b, corrs[b].shape, c1.shape)
@@ -120,18 +120,41 @@ def _native_batch(dev, K, bg, fg, edits, H, W):
 
 
 def _joined_render(dev, K, bg, fg, edit, H, W):
-    """the single-edit path: transform_points, then the renderer on the joined mesh [bg, moved fg]"""
+    """transform_points, then the renderer on the joined mesh [bg, moved fg]; None in the edit takes transform_depth_mesh's
+    defaults"""
     from diffusionhandles_b200 import depth_transform as dt
     from diffusionhandles_b200.mesh import Mesh
     from diffusionhandles_b200.renderer import Camera, MeshRenderer, SplatRendererArgs
     a, ax, t = edit
-    moved = Mesh(dt.transform_points(fg.verts, torch.tensor(a, dtype=torch.float32), torch.tensor(ax), torch.tensor(t)), fg.faces)
+    angle = torch.tensor(0.0 if a is None else float(a), dtype=torch.float32)
+    axis = torch.tensor([0.0, 1.0, 0.0]) if ax is None else torch.as_tensor(ax)
+    shift = torch.zeros(3) if t is None else torch.as_tensor(t)
+    moved = Mesh(dt.transform_points(fg.verts, angle, axis, shift), fg.faces)
     moved.add_vert_attribute("color", fg.vert_attributes["color"])
     r = MeshRenderer(['world_position', 'flat_vertex_color'],
                      SplatRendererArgs(device=dev, output_res=(H, W), cull_backfaces=True, blur_radius=1e-5))
     r.update_scene({'meshes': [bg, moved], 'cameras': [Camera(intrinsics=K)]})
     layers = r.render()
     return moved, layers, r.fragments[0][0]
+
+
+def _joined_mesh_edit(td, tb, tm, K, edit, unn):
+    """One edit through the joined-mesh renderer: (disparity (1,1,H,W), correspondences (n,4) int64 CPU) read off the
+    'world_position' z and the carried 'flat_vertex_color' layers, one row per target pixel that shows the foreground, in target
+    raster order, sources rounded half-to-even; an empty mask gives the normalised input disparity."""
+    from diffusionhandles_b200 import depth_transform as dt
+    if not tm.any():
+        return dt._empty_mask_result(td, unn)
+    H, W = td.shape[-2:]
+    bg, fg = _meshes(td.device, K, td, tb, tm)
+    _, layers, _ = _joined_render(td.device, K, bg, fg, edit, H, W)
+    target_depth = layers['world_position'][None, ..., 2]
+    carried = layers['flat_vertex_color'][0]
+    ty, tx = torch.nonzero(carried[..., 2] > 0.5, as_tuple=True)
+    source = torch.round(carried[ty, tx, :2] * carried.new_tensor([W - 1, H - 1])).to(torch.int64)
+    correspondences = torch.stack([source[:, 0], source[:, 1], tx, ty], dim=-1).cpu()
+    bounds = dt.normalize_depth(1.0 / td, return_bounds=True)[1] if unn else None
+    return dt.normalize_depth(1.0 / target_depth, bounds=bounds), correspondences
 
 
 def test_tie_order_background_wins(dev, K):
