@@ -68,12 +68,6 @@ _SIGNATURES = {
     "dh_transform_points": (c_int, [c_void_p, c_int, c_float, C.POINTER(c_float), C.POINTER(c_float), c_void_p, c_void_p,
                                     c_size_t, c_void_p]),
     "dh_edit_workspace_bytes": (c_size_t, [c_int, c_int, c_int]),
-    "dh_unproject_transform_project": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, C.POINTER(dh_camera),
-                                               C.POINTER(dh_rigid), c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,
-                                               c_void_p, c_void_p, c_void_p, c_void_p, c_size_t, c_void_p]),
-    "dh_unproject_transform_project_splat": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, C.POINTER(dh_camera),
-                                                     C.POINTER(dh_rigid), c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,
-                                                     c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_size_t, c_void_p]),
     "dh_edit_splat": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, C.POINTER(dh_camera), C.POINTER(dh_rigid), c_void_p,
                               c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,
                               c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_size_t, c_void_p]),
@@ -83,7 +77,6 @@ _SIGNATURES = {
     "dh_project_points": (c_int, [c_void_p, c_int, c_int, c_int, C.POINTER(dh_camera), c_void_p, c_void_p, c_void_p,
                                   c_void_p, c_void_p]),
     "dh_splat_zbuffer": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_int, c_void_p, c_void_p, c_void_p]),
-    "dh_splat_winner": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_int, c_void_p, c_void_p, c_void_p]),
     "dh_splat_resolve": (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_void_p, c_void_p, c_int, c_void_p,
                                  c_void_p, c_void_p, c_void_p, c_void_p, c_void_p]),
     "dh_splat_visible": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_int, c_int, c_void_p,
@@ -99,7 +92,6 @@ _SIGNATURES = {
                                    c_void_p, c_void_p, c_void_p, c_size_t, c_void_p]),
     "dh_process_correspondences": (c_int, [c_void_p, c_int, c_int, c_int, c_int, c_void_p, c_void_p, c_void_p, c_void_p,
                                            c_void_p, c_void_p, c_void_p]),
-    "dh_dense_source_map": (c_int, [c_void_p, c_void_p, c_int, c_void_p, c_int, c_int, c_int, c_void_p, c_void_p]),
     "dh_dense_source_maps": (c_int, [c_void_p, c_void_p, c_int, c_void_p, c_int, c_int, C.POINTER(c_int), c_int, c_void_p, c_void_p]),
     "dh_warp_gather_list": (c_int, [c_void_p, c_int, c_int, c_void_p, c_int, c_void_p, c_void_p]),
     "dh_warp_gather_dense": (c_int, [C.POINTER(dh_warp_level), c_int, c_int, c_void_p]),
@@ -118,7 +110,6 @@ _SIGNATURES = {
                                  c_int, c_int, c_void_p, c_void_p, c_size_t, c_void_p]),
     "dh_guidance_loss_batch_workspace_bytes": (c_size_t, [c_int, c_int, c_int]),
     "dh_guidance_loss_batch": (c_int, [C.POINTER(dh_loss_batch_edit), c_int, c_int, c_int, c_int, c_void_p, c_size_t, c_void_p]),
-    "dh_scale_inplace": (c_int, [c_void_p, c_size_t, c_void_p, c_void_p]),
     "dh_scale_inplace_many": (c_int, [C.POINTER(c_void_p), C.POINTER(c_size_t), c_int, c_void_p, c_void_p]),
     "dh_latent_step": (c_int, [c_void_p, c_void_p, c_float, c_void_p, c_size_t, c_void_p]),
     "dh_cfg_ddim_step": (c_int, [c_void_p, c_void_p, c_void_p, C.POINTER(dh_ddim_coeffs), c_void_p, c_void_p, c_size_t, c_void_p]),

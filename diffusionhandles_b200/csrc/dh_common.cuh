@@ -83,6 +83,27 @@ int tp_transform_batch(const float* pts, int N, int B, const TpEdit* edits_dev, 
 __device__ inline int warp_id() { return threadIdx.x >> 5; }
 __device__ inline int lane_id() { return threadIdx.x & 31; }
 
+// Pass 1 of the z-buffer splat for one point per lane (q < 0: no point), called by all 32 lanes: zb[q] = min(zb[q], key).
+// When every lane hits one pixel - clamped off-screen points pile onto border pixels - the warp reduces its keys (high halves,
+// then the low halves of the lanes that hold the minimal high half) and issues one atomic.  A plain load first shows whether
+// the key can win at all: the buffer only ever decreases, so a stale read is conservative.
+__device__ __forceinline__ void zbuf_atomic_min_warp(uint64_t* zb, int q, uint64_t key) {
+    const unsigned full = 0xFFFFFFFFu;
+    const int q0 = __shfl_sync(full, q, 0);
+    if (__all_sync(full, q == q0)) {
+        if (q0 < 0) return;
+        const uint32_t hi = (uint32_t)(key >> 32), lo = (uint32_t)key;
+        const uint32_t mhi = __reduce_min_sync(full, hi);
+        const uint32_t mlo = __reduce_min_sync(full, hi == mhi ? lo : 0xFFFFFFFFu);
+        if (lane_id() == 0) {
+            const uint64_t m = ((uint64_t)mhi << 32) | mlo;
+            if (m < *(volatile uint64_t*)(zb + q0)) atomicMin((unsigned long long*)(zb + q0), (unsigned long long)m);
+        }
+        return;
+    }
+    if (q >= 0 && key < *(volatile uint64_t*)(zb + q)) atomicMin((unsigned long long*)(zb + q), (unsigned long long)key);
+}
+
 // Exclusive scan of one int per thread over a CTA of up to 1024 threads; returns the exclusive prefix,
 // writes the CTA total to `total`.  `smem` needs 33 ints.
 __device__ inline int block_exclusive_scan(int v, int* smem, int& total) {

@@ -265,69 +265,6 @@ __global__ void __launch_bounds__(256) rigid_all_kernel(const float* __restrict_
 }
 
 // ------------------------------------------------------------------------------------------------
-// K1 main kernel: slot s < P -> background point s; slot s >= P -> foreground point j = s - P.
-// ------------------------------------------------------------------------------------------------
-// With kSplat the kernel also performs pass 1 of the z-buffer splat (dh_splat.cu): the 64-bit atomicMin on the
-// order-preserving z key, pre-reduced inside a warp when all of its lanes hit one pixel and skipped when a plain load already
-// shows the point cannot win.  The kernel is bound by its fp64 arithmetic, so the atomics ride along for free and the
-// separate pass - one more read of pix / zkey - disappears.
-template <bool kSplat>
-__global__ void __launch_bounds__(256) transform_project_kernel(
-    const float* __restrict__ bg_depth, int P, int H, int W, CamDev cam, const dh_rigid* __restrict__ rigid,
-    const float* __restrict__ xs, const float* __restrict__ ys,
-    const float* __restrict__ fgX, const float* __restrict__ fgY, const float* __restrict__ fgZ,
-    const int32_t* __restrict__ n_fg, const float* __restrict__ centroid,
-    int32_t* __restrict__ pix, uint64_t* __restrict__ zkey, double* __restrict__ points_out, uint64_t* zbuf) {
-    const int e = blockIdx.y;
-    const int slot = blockIdx.x * blockDim.x + threadIdx.x;
-    const size_t po = (size_t)e * 2 * P + slot;
-    bool live = slot < 2 * P;
-    double X = 0.0, Y = 0.0, Z = 0.0;
-    if (live && slot < P) {
-        const int row = slot / W, col = slot - row * W;
-        float x, y, z;
-        unproject(cam, bg_depth[(size_t)e * P + slot], xs[col], ys[row], x, y, z);
-        X = (double)x; Y = (double)y; Z = (double)z;
-    } else if (live) {
-        const int j = slot - P;
-        live = j < n_fg[e];
-        if (live) {
-            const size_t eo = (size_t)e * P + j;
-            rigid_point(fgX[eo], fgY[eo], fgZ[eo], centroid[e * 3 + 0], centroid[e * 3 + 1], centroid[e * 3 + 2], rigid[e], X, Y, Z);
-        }
-    }
-    int q = -1;
-    uint64_t key = kEmptyZ;
-    if (live) {
-        int u, v;
-        const bool ok = project(cam, X, Y, Z, H, W, u, v, key);
-        q = ok ? v * W + u : -1;
-        pix[po] = q;
-        zkey[po] = key;
-        if (points_out) {
-            double* o = points_out + po * 3;
-            o[0] = X; o[1] = Y; o[2] = Z;
-        }
-    }
-    if (!kSplat) return;
-    uint64_t* zb = zbuf + (size_t)e * P;
-    const unsigned full = 0xFFFFFFFFu;
-    const int q0 = __shfl_sync(full, q, 0);
-    if (__all_sync(full, q == q0)) {                 // clamped off-screen points pile onto border pixels: one atomic per warp
-        if (q0 < 0) return;
-        const uint32_t hi = (uint32_t)(key >> 32), lo = (uint32_t)key;
-        const uint32_t mhi = __reduce_min_sync(full, hi);
-        const uint32_t mlo = __reduce_min_sync(full, hi == mhi ? lo : 0xFFFFFFFFu);
-        if (lane_id() == 0) {
-            const uint64_t m = ((uint64_t)mhi << 32) | mlo;
-            if (m < *(volatile uint64_t*)(zb + q0)) atomicMin((unsigned long long*)(zb + q0), (unsigned long long)m);
-        }
-        return;
-    }
-    if (q >= 0 && key < *(volatile uint64_t*)(zb + q)) atomicMin((unsigned long long*)(zb + q), (unsigned long long)key);
-}
-
-// ------------------------------------------------------------------------------------------------
 // The edit fast path: K1 + K2 of a batch of edits in seven launches, no memsets, built on one fact:
 //
 //   a background point keeps its pixel.  With the library's pinhole camera (diagonal K, principal point 0, square image)
@@ -342,7 +279,8 @@ __global__ void __launch_bounds__(256) transform_project_kernel(
 // camera / image is not of the class above - are not trusted: those pixels are appended to a per-edit list of ODD points that
 // travel through the generic path together with the foreground points (index < P, so they keep their rank in ties).  NaN
 // depths never reach the z-buffer at all (depth_transform.py:697-712: a NaN never satisfies '<').  Results are bit-identical
-// to the all-points formulation (dh_unproject_transform_project + dh_splat_zbuffer + dh_splat_resolve) in every case.
+// in every case to dh_splat_zbuffer + dh_splat_resolve over the generic pixel / key of every point (the debug outputs below
+// record them for the background points too).
 // ------------------------------------------------------------------------------------------------
 struct EditWs {
     int32_t* tile_counts;
@@ -473,7 +411,6 @@ __global__ void __launch_bounds__(256) edit_points_splat_kernel(
     const int e = blockIdx.y;
     const int n = n_fg[e] + ws.odd_count[e];
     uint64_t* zb = zbuf + (size_t)e * P;
-    const unsigned full = 0xFFFFFFFFu;
     for (int base = blockIdx.x * blockDim.x; base < n; base += gridDim.x * blockDim.x) {      // (block-stride: n is only known here)
         const int slot = base + threadIdx.x;
         const EditPoint pt = edit_point(e, slot, P, W, cam, rigid, xs, ys, bg_depth, n_fg, centroid, ws);
@@ -492,20 +429,7 @@ __global__ void __launch_bounds__(256) edit_points_splat_kernel(
                 o[0] = pt.X; o[1] = pt.Y; o[2] = pt.Z;
             }
         }
-        const int q0 = __shfl_sync(full, q, 0);
-        if (__all_sync(full, q == q0)) {                 // clamped off-screen points pile onto border pixels: one atomic per warp
-            if (q0 >= 0) {
-                const uint32_t hi = (uint32_t)(key >> 32), lo = (uint32_t)key;
-                const uint32_t mhi = __reduce_min_sync(full, hi);
-                const uint32_t mlo = __reduce_min_sync(full, hi == mhi ? lo : 0xFFFFFFFFu);
-                if (lane_id() == 0) {
-                    const uint64_t m = ((uint64_t)mhi << 32) | mlo;
-                    if (m < *(volatile uint64_t*)(zb + q0)) atomicMin((unsigned long long*)(zb + q0), (unsigned long long)m);
-                }
-            }
-        } else if (q >= 0 && key < *(volatile uint64_t*)(zb + q)) {
-            atomicMin((unsigned long long*)(zb + q), (unsigned long long)key);
-        }
+        zbuf_atomic_min_warp(zb, q, key);
     }
 }
 
@@ -843,63 +767,6 @@ size_t dh_edit_workspace_bytes(int B, int H, int W) {
     if (B < 1 || H < 1 || W < 1) return 0;
     size_t a, b, c, d, e;
     return edit_ws_layout(B, H * W, k1_ws_layout(B, H * W, &a, &b, &c, &d, &e)).total;
-}
-
-static int k1_launch(const float* depth, const float* bg_depth, const float* fg_mask, int B, int H, int W,
-                     const dh_camera* cam_host, const dh_rigid* rigid_host, const float* xs, const float* ys,
-                     int32_t* pix, uint64_t* zkey, int32_t* fg_index, int32_t* n_fg, float* centroid,
-                     double* points_out, void* ws, size_t ws_bytes, uint64_t* zbuf, void* stream) {
-    DH_REQUIRE(depth && bg_depth && fg_mask && cam_host && rigid_host && xs && ys && pix && zkey && fg_index && n_fg && centroid && ws);
-    DH_REQUIRE(B >= 1 && H >= 2 && W >= 2);
-    DH_REQUIRE((long long)H * W <= (1ll << 29));
-    const int P = H * W;
-    size_t oc, orr, ox, oy, oz;
-    if (ws_bytes < k1_ws_layout(B, P, &oc, &orr, &ox, &oy, &oz)) return DH_ERR_WORKSPACE;
-    char* w = static_cast<char*>(ws);
-    int32_t* tile_counts = reinterpret_cast<int32_t*>(w + oc);
-    dh_rigid* rigid_dev = reinterpret_cast<dh_rigid*>(w + orr);
-    float* fgX = reinterpret_cast<float*>(w + ox);
-    float* fgY = reinterpret_cast<float*>(w + oy);
-    float* fgZ = reinterpret_cast<float*>(w + oz);
-    cudaStream_t st = as_stream(stream);
-    const CamDev cam = make_cam(cam_host);
-    const int ntiles = (P + kTile - 1) / kTile;
-    DH_CUDA_CHECK(cudaMemcpyAsync(rigid_dev, rigid_host, sizeof(dh_rigid) * (size_t)B, cudaMemcpyHostToDevice, st));
-    dim3 tgrid(ntiles, B);
-    fg_count_kernel<<<tgrid, kTileThreads, 0, st>>>(fg_mask, P, ntiles, tile_counts);
-    DH_LAUNCH_CHECK();
-    fg_compact_kernel<<<tgrid, kTileThreads, 0, st>>>(depth, fg_mask, P, W, ntiles, cam, xs, ys, tile_counts, fg_index, fgX, fgY, fgZ, n_fg,
-                                                      nullptr);
-    DH_LAUNCH_CHECK();
-    fg_centroid_kernel<<<B, 96, 0, st>>>(fgX, fgY, fgZ, n_fg, P, centroid);
-    DH_LAUNCH_CHECK();
-    dim3 grid((2 * P + 255) / 256, B);
-    if (zbuf)
-        transform_project_kernel<true><<<grid, 256, 0, st>>>(bg_depth, P, H, W, cam, rigid_dev, xs, ys, fgX, fgY, fgZ, n_fg, centroid,
-                                                             pix, zkey, points_out, zbuf);
-    else
-        transform_project_kernel<false><<<grid, 256, 0, st>>>(bg_depth, P, H, W, cam, rigid_dev, xs, ys, fgX, fgY, fgZ, n_fg, centroid,
-                                                              pix, zkey, points_out, nullptr);
-    DH_LAUNCH_CHECK();
-    return DH_OK;
-}
-
-int dh_unproject_transform_project(const float* depth, const float* bg_depth, const float* fg_mask, int B, int H, int W,
-                                   const dh_camera* cam_host, const dh_rigid* rigid_host, const float* xs, const float* ys,
-                                   int32_t* pix, uint64_t* zkey, int32_t* fg_index, int32_t* n_fg, float* centroid,
-                                   double* points_out, void* ws, size_t ws_bytes, void* stream) {
-    return k1_launch(depth, bg_depth, fg_mask, B, H, W, cam_host, rigid_host, xs, ys, pix, zkey, fg_index, n_fg, centroid, points_out,
-                     ws, ws_bytes, nullptr, stream);
-}
-
-int dh_unproject_transform_project_splat(const float* depth, const float* bg_depth, const float* fg_mask, int B, int H, int W,
-                                         const dh_camera* cam_host, const dh_rigid* rigid_host, const float* xs, const float* ys,
-                                         int32_t* pix, uint64_t* zkey, int32_t* fg_index, int32_t* n_fg, float* centroid,
-                                         double* points_out, uint64_t* zbuf, void* ws, size_t ws_bytes, void* stream) {
-    DH_REQUIRE(zbuf && B >= 1 && H >= 1 && W >= 1);
-    DH_CUDA_CHECK(cudaMemsetAsync(zbuf, 0xFF, sizeof(uint64_t) * (size_t)B * H * W, as_stream(stream)));
-    return k1_launch(depth, bg_depth, fg_mask, B, H, W, cam_host, rigid_host, xs, ys, pix, zkey, fg_index, n_fg, centroid, points_out,
-                     ws, ws_bytes, zbuf, stream);
 }
 
 int dh_edit_splat(const float* depth, const float* bg_depth, const float* fg_mask, int B, int H, int W, const dh_camera* cam_host,

@@ -1079,19 +1079,6 @@ __global__ void __launch_bounds__(kLossThreads * kGroups, 1) loss_fused_batch_ke
     loss_fused_body<kG, kBinary, kMem, kGroups, true>(bp.edit[e], cta);
 }
 
-__global__ void __launch_bounds__(256) scale_inplace_kernel(float* __restrict__ data, size_t n, const float* __restrict__ scale) {
-    const float s = *scale;
-    if (s == 1.0f) return;      // the common autograd.grad(loss, ...) case: nothing to do
-    const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
-    const size_t n4 = n / 4;
-    if (i < n4) {
-        float4 v = reinterpret_cast<float4*>(data)[i];
-        v.x *= s; v.y *= s; v.z *= s; v.w *= s;
-        reinterpret_cast<float4*>(data)[i] = v;
-    }
-    if (i < (n & 3)) data[n4 * 4 + i] *= s;
-}
-
 struct ScaleMany {
     float* data[kMaxLossLayers];
     unsigned long long n[kMaxLossLayers];
@@ -1496,16 +1483,6 @@ int dh_guidance_loss_batch(const dh_loss_batch_edit* edits_host, int n_edits, in
         if (fg_kind && E.n_fg > 0 && info[e].ell_words == 0) return DH_ERR_INVALID_ARGUMENT;
     }
     return launch_edits(bp, info, n_edits, grid, stream);
-}
-
-int dh_scale_inplace(float* data, size_t n, const float* scale, void* stream) {
-    DH_REQUIRE(data && scale);
-    if (n == 0) return DH_OK;
-    if (reinterpret_cast<uintptr_t>(data) & 15) return DH_ERR_INVALID_ARGUMENT;
-    const size_t threads = n / 4 > 3 ? n / 4 : 4;
-    scale_inplace_kernel<<<(unsigned)((threads + 255) / 256), 256, 0, as_stream(stream)>>>(data, n, scale);
-    DH_LAUNCH_CHECK();
-    return DH_OK;
 }
 
 int dh_scale_inplace_many(float* const* data_host, const size_t* n_host, int count, const float* scale, void* stream) {

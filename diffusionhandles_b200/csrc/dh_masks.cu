@@ -243,55 +243,8 @@ __global__ void __launch_bounds__(1024) process_corr_kernel(const int64_t* __res
 }
 
 // ------------------------------------------------------------------------------------------------
-// dense per-level source maps
+// dense per-level source maps: all levels of a stack in one pass
 // ------------------------------------------------------------------------------------------------
-__global__ void __launch_bounds__(256) dense_map_scatter_kernel(const int64_t* __restrict__ corr, const int32_t* __restrict__ n_corr,
-                                                                int corr_stride_rows, int img_res, int side, int32_t* src_map) {
-    const int e = blockIdx.y;
-    const int n = blockIdx.x * blockDim.x + threadIdx.x;
-    if (n >= n_corr[e]) return;
-    const int r = img_res / side;
-    const longlong4 v = *reinterpret_cast<const longlong4*>(corr + ((size_t)e * corr_stride_rows + n) * 4);
-    if ((unsigned long long)v.x >= (unsigned long long)img_res || (unsigned long long)v.y >= (unsigned long long)img_res ||
-        (unsigned long long)v.z >= (unsigned long long)img_res || (unsigned long long)v.w >= (unsigned long long)img_res)
-        return;                                   // rows outside the image are ignored
-    const int d = (int)(v.w / r) * side + (int)(v.z / r);
-    atomicMin(src_map + (size_t)e * side * side + d, n);
-}
-
-// one warp per destination cell
-__global__ void __launch_bounds__(256) dense_map_finalize_kernel(const int64_t* __restrict__ corr, int corr_stride_rows,
-                                                                 const int32_t* __restrict__ winner_src, int img_res, int side,
-                                                                 int32_t* src_map) {
-    const int e = blockIdx.y;
-    const int cell = blockIdx.x * (blockDim.x >> 5) + warp_id();
-    if (cell >= side * side) return;
-    const int r = img_res / side;
-    int32_t* m = src_map + (size_t)e * side * side + cell;
-    const int first = *m;
-    int res = -1;
-    if (first < 0x7F000000) {
-        const longlong4 v = *reinterpret_cast<const longlong4*>(corr + ((size_t)e * corr_stride_rows + first) * 4);
-        res = (int)(v.y / r) * side + (int)(v.x / r);
-    } else if (winner_src) {
-        const int cy = cell / side, cx = cell - cy * side;
-        const int32_t* ws = winner_src + (size_t)e * img_res * img_res;
-        const int n = r * r;
-        for (int k0 = 0; k0 < n && res < 0; k0 += 32) {
-            const int k = k0 + lane_id();
-            int s = -1;
-            if (k < n) s = ws[(cy * r + k / r) * img_res + cx * r + k % r];
-            const unsigned b = __ballot_sync(0xFFFFFFFFu, s >= 0);
-            if (b) {
-                s = __shfl_sync(0xFFFFFFFFu, s, __ffs(b) - 1);
-                res = ((s / img_res) / r) * side + (s % img_res) / r;
-            }
-        }
-    }
-    if (lane_id() == 0) *m = res;
-}
-
-// ---- all levels of a stack in one pass --------------------------------------------------------------
 constexpr int kMaxMapLevels = 8;
 struct MapLevels {
     int n_levels, img_res;
@@ -452,21 +405,6 @@ int dh_process_correspondences(const int64_t* corr, int n_corr, int img_res, int
         DH_CUDA_CHECK(cudaFuncSetAttribute(process_corr_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     process_corr_kernel<<<1, 1024, smem, as_stream(stream)>>>(corr, n_corr, img_res, grid, bg_erosion, fg_src, fg_dst, bg,
                                                               bg_orig, bg_trans, counts);
-    DH_LAUNCH_CHECK();
-    return DH_OK;
-}
-
-int dh_dense_source_map(const int64_t* corr, const int32_t* n_corr, int corr_stride_rows, const int32_t* winner_src, int B,
-                        int img_res, int side, int32_t* src_map, void* stream) {
-    DH_REQUIRE(corr && n_corr && src_map && B >= 1 && side >= 1 && img_res >= side && img_res % side == 0);
-    DH_REQUIRE(corr_stride_rows >= 1);
-    cudaStream_t st = as_stream(stream);
-    DH_CUDA_CHECK(cudaMemsetAsync(src_map, 0x7F, sizeof(int32_t) * (size_t)B * side * side, st));
-    dim3 g1((corr_stride_rows + 255) / 256, B);
-    dense_map_scatter_kernel<<<g1, 256, 0, st>>>(corr, n_corr, corr_stride_rows, img_res, side, src_map);
-    DH_LAUNCH_CHECK();
-    dim3 g2((side * side + 7) / 8, B);
-    dense_map_finalize_kernel<<<g2, 256, 0, st>>>(corr, corr_stride_rows, winner_src, img_res, side, src_map);
     DH_LAUNCH_CHECK();
     return DH_OK;
 }

@@ -32,22 +32,7 @@ __global__ void __launch_bounds__(256) splat_z_kernel(const int32_t* __restrict_
         q = pix[(size_t)e * stride + i];
         key = zkey[(size_t)e * stride + i];
     }
-    uint64_t* zb = zbuf + (size_t)e * P;
-    // warp-uniform pixel -> one atomic per warp
-    const unsigned full = 0xFFFFFFFFu;
-    const int q0 = __shfl_sync(full, q, 0);
-    if (__all_sync(full, q == q0)) {
-        if (q0 < 0) return;
-        uint32_t hi = (uint32_t)(key >> 32), lo = (uint32_t)key;
-        const uint32_t mhi = __reduce_min_sync(full, hi);
-        const uint32_t mlo = __reduce_min_sync(full, hi == mhi ? lo : 0xFFFFFFFFu);
-        if (lane_id() == 0) {
-            const uint64_t m = ((uint64_t)mhi << 32) | mlo;
-            if (m < *(volatile uint64_t*)(zb + q0)) atomicMin((unsigned long long*)(zb + q0), (unsigned long long)m);
-        }
-        return;
-    }
-    if (q >= 0 && key < *(volatile uint64_t*)(zb + q)) atomicMin((unsigned long long*)(zb + q), (unsigned long long)key);
+    zbuf_atomic_min_warp(zbuf + (size_t)e * P, q, key);
 }
 
 __global__ void __launch_bounds__(256) splat_winner_kernel(const int32_t* __restrict__ pix, const uint64_t* __restrict__ zkey,
@@ -227,17 +212,6 @@ int dh_splat_zbuffer(const int32_t* pix, const uint64_t* zkey, const int32_t* n_
     splat_z_kernel<<<grid, 256, 0, st>>>(pix, zkey, n_points, n_fixed, stride_points, P, zbuf);
     DH_LAUNCH_CHECK();
     splat_winner_kernel<<<grid, 256, 0, st>>>(pix, zkey, n_points, n_fixed, stride_points, P, zbuf, winner);
-    DH_LAUNCH_CHECK();
-    return DH_OK;
-}
-
-int dh_splat_winner(const int32_t* pix, const uint64_t* zkey, const int32_t* n_points, int n_fixed, int n_max,
-                    int stride_points, int B, int P, const uint64_t* zbuf, uint32_t* winner, void* stream) {
-    DH_REQUIRE(pix && zkey && zbuf && winner && B >= 1 && P >= 1 && n_max >= 0 && stride_points >= n_max);
-    cudaStream_t st = as_stream(stream);
-    DH_CUDA_CHECK(cudaMemsetAsync(winner, 0xFF, sizeof(uint32_t) * (size_t)B * P, st));
-    if (n_max == 0) return DH_OK;
-    splat_winner_kernel<<<dim3((n_max + 255) / 256, B), 256, 0, st>>>(pix, zkey, n_points, n_fixed, stride_points, P, zbuf, winner);
     DH_LAUNCH_CHECK();
     return DH_OK;
 }

@@ -7,7 +7,6 @@ edits costs one host synchronisation (reading the per-edit correspondence counts
 from __future__ import annotations
 
 import ctypes as C
-import os
 from dataclasses import dataclass
 from typing import Dict, List, Optional, Sequence, Tuple
 
@@ -155,7 +154,6 @@ class EditEngine:
         # the transforms are uploaded from this (pageable, engine-owned) array: it outlives the call, so a CUDA graph that captured
         # the launch chain re-reads the transforms stored here at every replay
         self._rigids = (N.dh_rigid * B)()
-        self.fast_splat = os.environ.get("DH_ALL_POINTS_SPLAT", "0") != "1"
         self.xs, self.ys = pixel_grid(H, W, dev)
         S = max(H, W)
         # depth_transform.py:311-313: MORPH_ELLIPSE elements of size img_res//250 (open) and img_res//50 (close)
@@ -180,24 +178,12 @@ class EditEngine:
             rg[i] = r
         f32 = torch.float32
         # K1 + K2 (unproject, transform, project, exact (z, index) splat, depth map / target mask / winner sources / min-max)
-        if self.fast_splat:
-            N.check(lib.dh_edit_splat(
-                N.ptr(depth, f32, "depth"), N.ptr(bg_depth, f32, "bg_depth"), N.ptr(fg_mask, f32, "fg_mask"), B, H, W,
-                C.byref(cam), rg, N.ptr(self.xs), N.ptr(self.ys), N.ptr(self.pix), N.ptr(self.zkey), N.ptr(self.fg_index),
-                N.ptr(self.n_fg), N.ptr(self.centroid), N.ptr(self.points) if self.points is not None else None,
-                N.ptr(self.zbuf), N.ptr(self.winner), N.ptr(self.depth_map), N.ptr(self.target_mask), N.ptr(self.target_bits),
-                N.ptr(self.winner_src), N.ptr(self.inv_minmax), N.ptr(self.ws), self.ws_bytes, st), "dh_edit_splat")
-        else:       # the all-points formulation (every background point through the generic path): kept for cross-checks
-            N.check(lib.dh_unproject_transform_project_splat(
-                N.ptr(depth, f32, "depth"), N.ptr(bg_depth, f32, "bg_depth"), N.ptr(fg_mask, f32, "fg_mask"), B, H, W,
-                C.byref(cam), rg, N.ptr(self.xs), N.ptr(self.ys), N.ptr(self.pix), N.ptr(self.zkey), N.ptr(self.fg_index),
-                N.ptr(self.n_fg), N.ptr(self.centroid), N.ptr(self.points) if self.points is not None else None,
-                N.ptr(self.zbuf), N.ptr(self.ws), self.ws_bytes, st), "dh_unproject_transform_project_splat")
-            N.check(lib.dh_splat_winner(N.ptr(self.pix), N.ptr(self.zkey), N.ptr(self.n_fg), P, 2 * P, 2 * P, B, P,
-                                        N.ptr(self.zbuf), N.ptr(self.winner), st), "dh_splat_winner")
-            N.check(lib.dh_splat_resolve(N.ptr(self.zbuf), N.ptr(self.winner), B, H, W, P, None, N.ptr(self.fg_index), 2 * P,
-                                         N.ptr(self.depth_map), N.ptr(self.target_mask), N.ptr(self.target_bits),
-                                         N.ptr(self.winner_src), N.ptr(self.inv_minmax), st), "dh_splat_resolve")
+        N.check(lib.dh_edit_splat(
+            N.ptr(depth, f32, "depth"), N.ptr(bg_depth, f32, "bg_depth"), N.ptr(fg_mask, f32, "fg_mask"), B, H, W,
+            C.byref(cam), rg, N.ptr(self.xs), N.ptr(self.ys), N.ptr(self.pix), N.ptr(self.zkey), N.ptr(self.fg_index),
+            N.ptr(self.n_fg), N.ptr(self.centroid), N.ptr(self.points) if self.points is not None else None,
+            N.ptr(self.zbuf), N.ptr(self.winner), N.ptr(self.depth_map), N.ptr(self.target_mask), N.ptr(self.target_bits),
+            N.ptr(self.winner_src), N.ptr(self.inv_minmax), N.ptr(self.ws), self.ws_bytes, st), "dh_edit_splat")
         N.check(lib.dh_mask_clean(N.ptr(self.target_bits), N.ptr(self.cleaned_bits), N.ptr(self.tmp_bits), B, H, W,
                                   self.close_rows, self.close_k, self.open_rows, self.open_k, st), "dh_mask_clean")
         N.check(lib.dh_correspondences(N.ptr(self.pix), N.ptr(self.winner), N.ptr(self.fg_index), N.ptr(self.n_fg),

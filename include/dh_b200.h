@@ -93,22 +93,6 @@ int dh_transform_points(const float* points, int N, float angle_degrees, const f
 /* ---- per-edit scratch for the fused pc path (rows 2-6) ------------------------------------------- */
 size_t dh_edit_workspace_bytes(int B, int H, int W);
 
-/* ---- K1, rows 2-4: fused unproject -> rigid transform -> project ----------------------------------
- * depth_transform.py:226-274 (+ :461-533, :666-687).  For every edit e:
- *   points 0..P-1   = unprojected bg_depth pixels (raster order),
- *   points P..P+n-1 = unprojected depth pixels under fg_mask (non-zero = foreground), rotated about
- *                     their fp32 sequential centroid and translated (fp64), raster order of the source.
- * Outputs (all per edit, capacity 2*P points): pix int32 (v*W+u, -1 = z is NaN), zkey uint64
- * (order-preserving bits of the fp64 z), fg_index int32[P] (source pixel of fg point j), n_fg int32,
- * centroid float[3]; optional points_out double[2P][3] for parity checks (may be NULL).
- * rigid_host: B structs on the host (copied by value into the launch). */
-int dh_unproject_transform_project(const float* depth, const float* bg_depth, const float* fg_mask,
-                                   int B, int H, int W, const dh_camera* cam_host, const dh_rigid* rigid_host,
-                                   const float* xs, const float* ys,
-                                   int32_t* pix, uint64_t* zkey, int32_t* fg_index, int32_t* n_fg,
-                                   float* centroid, double* points_out,
-                                   void* ws, size_t ws_bytes, void* stream);
-
 /* ---- row 3: transform_point_cloud, depth_transform.py:461-533 -----------------------------------------
  * points (N,3) fp32, mask (N) fp32 (non-zero = selected): Rodrigues rotation about the fp32 sequential centroid of
  * the selected points + translation, applied to ALL N points -> out (N,3) fp64; centroid float[3]; n_masked int32. */
@@ -120,18 +104,16 @@ int dh_transform_point_cloud(const float* points, const float* mask, int N, cons
 int dh_project_points(const double* points, int N, int H, int W, const dh_camera* cam_host,
                       int32_t* pix, uint64_t* zkey, int32_t* u, int32_t* v, void* stream);
 
-/* K1 fused with pass 1 of the z-buffer splat: as above, and zbuf[e][q] = min over the edit's points that land on pixel q of
- * the order-preserving z key (zbuf is initialised here).  Follow it with dh_splat_winner (pass 2).  The kernel is bound by
- * its fp64 arithmetic, so the atomics cost nothing extra and one read of pix / zkey is saved. */
-int dh_unproject_transform_project_splat(const float* depth, const float* bg_depth, const float* fg_mask,
-                                         int B, int H, int W, const dh_camera* cam_host, const dh_rigid* rigid_host,
-                                         const float* xs, const float* ys,
-                                         int32_t* pix, uint64_t* zkey, int32_t* fg_index, int32_t* n_fg,
-                                         float* centroid, double* points_out, uint64_t* zbuf,
-                                         void* ws, size_t ws_bytes, void* stream);
-
 /* ---- K1 + K2 of a batch of edits in one call (what transform_depth_pc runs, depth_transform.py:226-306) ----------
- * Same results as dh_unproject_transform_project_splat + dh_splat_winner + dh_splat_resolve, bit for bit, in seven
+ * The points of edit e, in the reference's order:
+ *   points 0..P-1   = unprojected bg_depth pixels (raster order),
+ *   points P..P+n-1 = unprojected depth pixels under fg_mask (non-zero = foreground), rotated about
+ *                     their fp32 sequential centroid and translated (fp64), raster order of the source.
+ * Per-point outputs sit at the point's index (capacity 2*P per edit): pix int32 (v*W+u, -1 = z is NaN), zkey uint64
+ * (order-preserving bits of the fp64 z); optional points_out double[2P][3] (debug, may be NULL).  Per edit: fg_index int32[P]
+ * (source pixel of fg point j), n_fg int32, centroid float[3], and the splat outputs of dh_splat_resolve with fg_start = P.
+ * rigid_host: B structs on the host.
+ * Same results as dh_splat_zbuffer + dh_splat_resolve over the generic pixel / key of every point, bit for bit, in seven
  * launches and without memsets: with the library's pinhole camera a background point provably keeps its pixel, so the
  * z-buffer is initialised with the background keys (float4 loads, 128-bit stores), the fp64 transform / projection runs for
  * the foreground points only, and a background pixel resolves itself.  Background depths that are zero, infinite or of absurd
@@ -152,12 +134,6 @@ int dh_edit_splat(const float* depth, const float* bg_depth, const float* fg_mas
 int dh_splat_zbuffer(const int32_t* pix, const uint64_t* zkey, const int32_t* n_points, int n_fixed,
                      int n_max, int stride_points, int B, int P,
                      uint64_t* zbuf, uint32_t* winner, void* stream);
-
-/* Pass 2 alone (winner index among the points whose key equals zbuf), for a zbuf produced by
- * dh_unproject_transform_project_splat.  Same arguments as dh_splat_zbuffer. */
-int dh_splat_winner(const int32_t* pix, const uint64_t* zkey, const int32_t* n_points, int n_fixed,
-                    int n_max, int stride_points, int B, int P,
-                    const uint64_t* zbuf, uint32_t* winner, void* stream);
 
 /* ---- K2 epilogue, rows 5-6: depth_transform.py:714-747, :283-306 ----------------------------------
  * depth_map fp32 (+inf = empty), target_mask uint8 {0,1} = winner is a foreground point,
@@ -208,15 +184,13 @@ int dh_process_correspondences(const int64_t* corr, int n_corr, int img_res, int
                                int32_t* fg_src, int32_t* fg_dst, int32_t* bg, int32_t* bg_orig, int32_t* bg_trans,
                                int32_t* counts, void* stream);
 
-/* ---- row 9: dense per-level source map -------------------------------------------------------------
+/* ---- row 9: dense per-level source maps ------------------------------------------------------------
  * src_map[q] = source cell of the lowest-n correspondence whose destination cell is q; cells without
  * one fall back (if winner_src != NULL) to the first target pixel of the cell (raster order) that has
- * a splat winner; else -1.  side = cells per image side at this level. */
-int dh_dense_source_map(const int64_t* corr, const int32_t* n_corr, int corr_stride_rows, const int32_t* winner_src,
-                        int B, int img_res, int side, int32_t* src_map, void* stream);
-/* All levels of a stack in one pass (the correspondences are read once): sides_host[l] = cells per side of level l
+ * a splat winner; else -1.
+ * All levels of a stack in one pass (the correspondences are read once): sides_host[l] = cells per side of level l
  * (HOST array); maps = one buffer of B * sum(side_l^2) ints, level-major (level l starts at B * sum_{k<l} side_k^2,
- * inside it edit-major like src_map above). */
+ * inside it edit-major: B maps of side_l^2 cells). */
 int dh_dense_source_maps(const int64_t* corr, const int32_t* n_corr, int corr_stride_rows, const int32_t* winner_src,
                          int B, int img_res, const int* sides_host, int n_levels, int32_t* maps, void* stream);
 
@@ -313,9 +287,8 @@ size_t dh_guidance_loss_patch_workspace_bytes(int n_layers, int max_channels);
 int dh_guidance_loss_patch(const dh_loss_layer* layers_host, int n_layers, int grid, int patch_size, const void* plan,
                            int n_fg, int n_bg_orig, int n_bg_trans, int n_bg_common, int fg_kind, int bg_kind,
                            float* loss_out, void* ws, size_t ws_bytes, void* stream);
-/* grads *= *scale (device scalar); exits early on the device when *scale == 1. */
-int dh_scale_inplace(float* data, size_t n, const float* scale, void* stream);
-/* The same for up to 8 tensors in one launch (HOST arrays of device pointers and element counts). */
+/* grads *= *scale (device scalar) for up to 8 tensors in one launch (HOST arrays of device pointers and element counts); exits
+ * early on the device when *scale == 1. */
 int dh_scale_inplace_many(float* const* data_host, const size_t* n_host, int count, const float* scale, void* stream);
 
 /* ---- 8(f) rank 1: Poisson hole fill of the edited disparity, depth_transform.py:346-363, :535-587 ----

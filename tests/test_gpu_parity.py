@@ -1090,15 +1090,21 @@ def test_device_sweep_graph_replay_matches_plain_launches(dev, K):
 
 
 @pytest.mark.parametrize("H,W", [(128, 128), (96, 160)])
-def test_edit_fast_splat_equals_all_points_formulation(dev, K, H, W):
-    """dh_edit_splat (background pixels resolve themselves, generic path for foreground + odd points) against the all-points
-    formulation (dh_unproject_transform_project_splat + dh_splat_winner + dh_splat_resolve), bit for bit: regular scenes, background
-    depths that are zero / infinite / NaN / subnormal / negative / huge, exact z ties between background and foreground, a
-    non-square image (no pixel-keeping guarantee: every background point takes the generic path), with and without the debug outputs."""
+def test_edit_fast_splat_equals_generic_splat_of_every_point(dev, K, H, W):
+    """dh_edit_splat (background pixels resolve themselves, generic path for foreground + odd points) against the generic splat
+    of every point (dh_splat_zbuffer + dh_splat_resolve over the pixel / key the debug outputs record for all P + n_fg points), bit
+    for bit: regular scenes, background depths that are zero / infinite / NaN / subnormal / negative / huge, exact z ties between
+    background and foreground, a non-square image (no pixel-keeping guarantee: every background point takes the generic path).
+    The debug outputs change no result, and the points they record are the oracle's, their pixels / keys dh_project_points'.
+    (The oracle has no defined answer for some of these depths - an inf depth projects to a NaN pixel coordinate - so it does
+    not replace the generic splat here.)"""
+    import ctypes
+    from diffusionhandles_b200 import _native as Nn
     from diffusionhandles_b200.engine import EditEngine, make_rigid
     rng = np.random.default_rng(5)
     B = 4
     S = max(H, W)
+    P = H * W
     scenes = [O.synthetic_scene(S, 60 + i, quantize=0.1 if i == 1 else None) for i in range(B)]
     depth = np.stack([s[0][:H, :W] for s in scenes]).copy()
     bg = np.stack([s[1][:H, :W] for s in scenes]).copy()
@@ -1110,37 +1116,67 @@ def test_edit_fast_splat_equals_all_points_formulation(dev, K, H, W):
         jdx = rng.choice(H * W, 40, replace=False)      # (finite odd foreground depths: a NaN / inf would poison the centroid)
         depth[e].reshape(-1)[jdx] = np.array([0.0, -0.0, 1e-42, -2.5, 1e-33], np.float32)[rng.integers(0, 5, 40)]
     bg[3, :8] = 0.0                                # whole rows of zeros: thousands of points on one pixel
-    rig = [make_rigid(20.0 * i - 30.0, [0.0, 1.0, 0.0], [0.1 * i, 0.0, 0.05 * i]) for i in range(B)]
+    angles = [20.0 * i - 30.0 for i in range(B)]
+    trans = [(0.1 * i, 0.0, 0.05 * i) for i in range(B)]
+    rig = [make_rigid(a, [0.0, 1.0, 0.0], t) for a, t in zip(angles, trans)]
     td, tb, tm = (torch.from_numpy(a).to(dev) for a in (depth, bg, mask))
     Kc = K.cpu()
+
+    def bits(t):                                   # (NaN-safe: float tensors are compared by their bit patterns)
+        return t.view(torch.int32) if t.dtype == torch.float32 else t
+
     out = {}
-    for fast, keep in ((False, True), (True, True), (True, False)):
+    for keep in (False, True):
         eng = EditEngine(dev, B, H, W, keep_points=keep)
-        eng.fast_splat = fast
         res = eng.run(td, tb, tm, Kc, rig, poisson=False)
-        out[(fast, keep)] = {k: getattr(res, k).clone() for k in ("winner", "winner_src", "depth_map", "target_mask", "target_bits",
-                                                                 "cleaned_bits", "disparity_raw", "n_corr", "n_fg", "centroid")}
-        out[(fast, keep)]["corr"] = [res.correspondences(e).clone() for e in range(B)]
-        if keep:
-            n = [H * W + int(v) for v in res.n_fg_host]
-            out[(fast, keep)]["pix"] = [res.pix[e, :n[e]].clone() for e in range(B)]
-            out[(fast, keep)]["zkey"] = [res.zkey[e, :n[e]].clone() for e in range(B)]
-            out[(fast, keep)]["points"] = [res.points[e, :n[e]].clone() for e in range(B)]
-    ref = out[(False, True)]
-    assert int(ref["n_corr"].sum()) > 0
-    for key in ((True, True), (True, False)):
-        got = out[key]
-        for k in ("winner", "winner_src", "target_mask", "target_bits", "cleaned_bits", "n_corr", "n_fg"):
-            assert torch.equal(got[k], ref[k]), (key, k)
-        for k in ("depth_map", "disparity_raw", "centroid"):       # (NaN-safe: compare bit patterns)
-            assert torch.equal(got[k].view(torch.int32), ref[k].view(torch.int32)), (key, k)
-        for a, b in zip(got["corr"], ref["corr"]):
-            assert torch.equal(a, b)
-    for k in ("pix", "zkey"):
-        for a, b in zip(out[(True, True)][k], ref[k]):
-            assert torch.equal(a, b), k
-    for a, b in zip(out[(True, True)]["points"], ref["points"]):
-        assert torch.equal(a.view(torch.int64), b.view(torch.int64))
+        out[keep] = {k: getattr(res, k).clone() for k in ("winner", "winner_src", "depth_map", "target_mask", "target_bits",
+                                                         "cleaned_bits", "disparity_raw", "n_corr", "n_fg", "centroid")}
+        out[keep]["inv_minmax"] = eng.inv_minmax.clone()
+        out[keep]["corr"] = [res.correspondences(e).clone() for e in range(B)]
+    fast = out[True]                               # `res` is the run with the debug outputs
+    assert int(fast["n_corr"].sum()) > 0
+    for k, v in out[False].items():
+        if k == "corr":
+            for a, b in zip(v, fast[k]):
+                assert torch.equal(a, b)
+        else:
+            assert torch.equal(bits(v), bits(fast[k])), k
+
+    # the generic splat of all P + n_fg points, from the pixels / keys the debug run recorded
+    lib, st = Nn.load(), Nn.stream_handle(dev)
+    zbuf = torch.empty((B, P), dtype=torch.int64, device=dev)
+    ref = {"winner": torch.empty((B, P), dtype=torch.int32, device=dev), "winner_src": torch.empty((B, P), dtype=torch.int32, device=dev),
+           "depth_map": torch.empty((B, H, W), dtype=torch.float32, device=dev),
+           "target_mask": torch.empty((B, H, W), dtype=torch.uint8, device=dev),
+           "target_bits": torch.empty_like(res.target_bits), "inv_minmax": torch.empty((B, 2), dtype=torch.float32, device=dev)}
+    Nn.check(lib.dh_splat_zbuffer(Nn.ptr(res.pix), Nn.ptr(res.zkey), Nn.ptr(res.n_fg), P, 2 * P, 2 * P, B, P, Nn.ptr(zbuf),
+                                  Nn.ptr(ref["winner"]), st), "dh_splat_zbuffer")
+    Nn.check(lib.dh_splat_resolve(Nn.ptr(zbuf), Nn.ptr(ref["winner"]), B, H, W, P, None, Nn.ptr(res.fg_index), 2 * P,
+                                  Nn.ptr(ref["depth_map"]), Nn.ptr(ref["target_mask"]), Nn.ptr(ref["target_bits"]),
+                                  Nn.ptr(ref["winner_src"]), Nn.ptr(ref["inv_minmax"]), st), "dh_splat_resolve")
+    for k, v in ref.items():
+        assert torch.equal(bits(fast[k]), bits(v)), k
+
+    # the recorded points against the oracle (background: every pixel unprojected; foreground: the masked points moved), and
+    # the recorded pixels / keys against dh_project_points of those points
+    cam = Nn.make_camera(Kc)
+    for e in range(B):
+        F = np.flatnonzero(mask[e].reshape(-1))
+        n = P + len(F)
+        assert int(res.n_fg_host[e]) == len(F)
+        with np.errstate(all="ignore"):
+            fg_pts, _ = O.rigid_transform_fg(O.depth_to_world_coords(depth[e], K_NP).reshape(-1, 3)[F], (0.0, 1.0, 0.0), angles[e],
+                                             f32_translation(trans[e]))
+            want = np.vstack([O.depth_to_world_coords(bg[e], K_NP).reshape(-1, 3).astype(np.float64), fg_pts])
+        got = res.points[e, :n].cpu().numpy()
+        nan = np.isnan(want)
+        assert np.array_equal(np.isnan(got), nan)                  # (NaN sign bits differ between NumPy and the GPU)
+        assert np.array_equal(got[~nan].view(np.int64), want[~nan].view(np.int64))
+        pix = torch.empty(n, dtype=torch.int32, device=dev)
+        zkey = torch.empty(n, dtype=torch.int64, device=dev)
+        Nn.check(lib.dh_project_points(Nn.ptr(res.points[e, :n]), n, H, W, ctypes.byref(cam), Nn.ptr(pix), Nn.ptr(zkey), None, None,
+                                       st), "dh_project_points")
+        assert torch.equal(res.pix[e, :n], pix) and torch.equal(res.zkey[e, :n], zkey)
 
 
 def test_poisson_large_hole_and_non_convergence_flag(dev):
