@@ -123,6 +123,13 @@ _SIGNATURES = {
                                    C.POINTER(c_float), C.POINTER(c_float), C.POINTER(c_float), c_int, c_int, C.POINTER(c_float),
                                    C.POINTER(c_float), c_float, c_float, c_float, c_int, c_int, c_int, c_void_p, c_void_p, c_void_p,
                                    c_void_p, c_void_p, c_size_t, c_void_p]),
+    "dh_edit_mesh_scenes_workspace_bytes": (c_size_t, [c_int, C.POINTER(C.c_int32), C.POINTER(C.c_int32), C.POINTER(C.c_int32),
+                                                       C.POINTER(C.c_int32), c_int, C.POINTER(C.c_int32), c_int, c_int]),
+    "dh_edit_mesh_scenes": (c_int, [c_int, c_void_p, c_void_p, C.POINTER(C.c_int32), C.POINTER(C.c_int32), c_void_p, c_void_p, c_void_p,
+                                    C.POINTER(C.c_int32), C.POINTER(C.c_int32), c_int, C.POINTER(C.c_int32), C.POINTER(c_float),
+                                    C.POINTER(c_float), C.POINTER(c_float), c_int, c_int, C.POINTER(c_float), C.POINTER(c_float), c_float,
+                                    c_float, c_float, c_int, c_int, c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_size_t,
+                                    c_void_p]),
     "dh_poisson_workspace_bytes": (c_size_t, [c_int, c_int, c_int]),
     "dh_poisson_fill": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_void_p, c_int, C.c_double,
                                 c_void_p, c_void_p, c_size_t, c_void_p]),

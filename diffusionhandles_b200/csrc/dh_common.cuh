@@ -80,6 +80,25 @@ struct TpEdit {
 TpEdit tp_edit(float angle_degrees, const float* axis3, const float* translation3);
 int tp_transform_batch(const float* pts, int N, int B, const TpEdit* edits_dev, double* partial, float* out, cudaStream_t st);
 
+// One scene of a scene table (device copy; offsets into concatenated per-scene arrays) and one edit of a scene batch.
+// tp_transform_scenes moves the V_fg foreground points of edit b's scene (pts + 3 fg_v0) by its transform into
+// out + 3 out0 with the centroid of that scene alone, bit-identical to dh_transform_points on that scene: each scene sums its
+// partials with its own block count and stride (tp_partial_blocks of its V_fg) into partial + 3 tp_partial0.
+struct SceneDesc {
+    int bg_v0, V_bg, bg_f0, F_bg;    // background vertices / faces (faces scene-local)
+    int fg_v0, V_fg, fg_f0, F_fg;    // foreground vertices (and colours) / faces (faces scene-local)
+    int tp_blocks, tp_partial0;      // centroid partial sums of the foreground
+    int plane;                       // the edit whose key plane receives the background raster (-1: no edit uses the scene)
+};
+struct SceneEdit {
+    TpEdit t;
+    int scene;
+    int out0;                        // first moved vertex of this edit in the flat (sum over edits of V_fg) arrays
+};
+int tp_partial_blocks(int N);
+int tp_transform_scenes(const float* pts, const SceneDesc* scenes_dev, int n_scenes, int max_blocks, const SceneEdit* edits_dev, int B,
+                        int max_n, double* partial, float* out, cudaStream_t st);
+
 __device__ inline int warp_id() { return threadIdx.x >> 5; }
 __device__ inline int lane_id() { return threadIdx.x & 31; }
 

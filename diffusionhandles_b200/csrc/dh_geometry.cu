@@ -585,10 +585,11 @@ __global__ void __launch_bounds__(256) project_points_kernel(const double* __res
 // transform_points (torch fp32 variant, depth_transform.py:439-459): centroid = mean over ALL points.
 // Pairwise (deterministic) fp32 reduction; parity with torch is tolerance based.
 // ------------------------------------------------------------------------------------------------
-__global__ void __launch_bounds__(256) tp_partial_sum_kernel(const float* __restrict__ pts, int N, double* __restrict__ partial) {
+// block `blk` of `nblocks` (256 threads each, grid stride nblocks * 256) -> partial[3 blk .. 3 blk + 2]
+__device__ __forceinline__ void tp_partial_sum(const float* __restrict__ pts, int N, int blk, int nblocks, double* __restrict__ partial) {
     __shared__ double sm[3][8];
     double s[3] = {0, 0, 0};
-    for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < N; i += gridDim.x * blockDim.x) {
+    for (int i = blk * blockDim.x + threadIdx.x; i < N; i += nblocks * blockDim.x) {
         s[0] += pts[3 * (size_t)i]; s[1] += pts[3 * (size_t)i + 1]; s[2] += pts[3 * (size_t)i + 2];
     }
 #pragma unroll
@@ -601,8 +602,20 @@ __global__ void __launch_bounds__(256) tp_partial_sum_kernel(const float* __rest
     if (threadIdx.x < 3) {
         double t = 0;
         for (int w = 0; w < 8; ++w) t += sm[threadIdx.x][w];
-        partial[blockIdx.x * 3 + threadIdx.x] = t;
+        partial[blk * 3 + threadIdx.x] = t;
     }
+}
+
+__global__ void __launch_bounds__(256) tp_partial_sum_kernel(const float* __restrict__ pts, int N, double* __restrict__ partial) {
+    tp_partial_sum(pts, N, blockIdx.x, gridDim.x, partial);
+}
+
+// the partial sums of every scene's foreground (blockIdx.y = scene), each with its own block count
+__global__ void __launch_bounds__(256) tp_partial_sum_scenes_kernel(const float* __restrict__ pts, const SceneDesc* __restrict__ scenes,
+                                                                    double* __restrict__ partial) {
+    const SceneDesc sc = scenes[blockIdx.y];
+    if ((int)blockIdx.x >= sc.tp_blocks) return;
+    tp_partial_sum(pts + 3 * (size_t)sc.fg_v0, sc.V_fg, blockIdx.x, sc.tp_blocks, partial + 3 * (size_t)sc.tp_partial0);
 }
 
 // the centroid from the partial sums (every block repeats the short sum), then one point of one transform
@@ -647,7 +660,40 @@ __global__ void __launch_bounds__(256) tp_apply_batch_kernel(const float* __rest
     tp_apply_point(pts, i, cen, edits[b], out + 3 * (size_t)N * b);
 }
 
-static int tp_partial_blocks(int N) { return N >= 256 * kTpMaxPartials ? kTpMaxPartials : (N + 255) / 256; }
+// edit b of a scene batch (blockIdx.y = edit): its scene's foreground moved with that scene's centroid
+__global__ void __launch_bounds__(256) tp_apply_scenes_kernel(const float* __restrict__ pts, const SceneDesc* __restrict__ scenes,
+                                                              const double* __restrict__ partial, const SceneEdit* __restrict__ edits,
+                                                              float* __restrict__ out) {
+    __shared__ float cen[3];
+    const SceneEdit e = edits[blockIdx.y];
+    const SceneDesc sc = scenes[e.scene];
+    if ((int)(blockIdx.x * blockDim.x) >= sc.V_fg) return;          // uniform over the block, before the barrier
+    tp_centroid(partial + 3 * (size_t)sc.tp_partial0, sc.tp_blocks, sc.V_fg, cen);
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= sc.V_fg) return;
+    tp_apply_point(pts + 3 * (size_t)sc.fg_v0, i, cen, e.t, out + 3 * (size_t)e.out0);
+}
+
+int tp_partial_blocks(int N) { return N >= 256 * kTpMaxPartials ? kTpMaxPartials : (N + 255) / 256; }
+
+int tp_transform_batch(const float* pts, int N, int B, const TpEdit* edits_dev, double* partial, float* out, cudaStream_t st) {
+    const int nblocks = tp_partial_blocks(N);
+    tp_partial_sum_kernel<<<nblocks, 256, 0, st>>>(pts, N, partial);
+    DH_LAUNCH_CHECK();
+    tp_apply_batch_kernel<<<dim3((N + 255) / 256, B), 256, 0, st>>>(pts, N, partial, nblocks, edits_dev, out);
+    DH_LAUNCH_CHECK();
+    return DH_OK;
+}
+
+int tp_transform_scenes(const float* pts, const SceneDesc* scenes_dev, int n_scenes, int max_blocks, const SceneEdit* edits_dev, int B,
+                        int max_n, double* partial, float* out, cudaStream_t st) {
+    if (max_n < 1) return DH_OK;
+    tp_partial_sum_scenes_kernel<<<dim3(max_blocks, n_scenes), 256, 0, st>>>(pts, scenes_dev, partial);
+    DH_LAUNCH_CHECK();
+    tp_apply_scenes_kernel<<<dim3((max_n + 255) / 256, B), 256, 0, st>>>(pts, scenes_dev, partial, edits_dev, out);
+    DH_LAUNCH_CHECK();
+    return DH_OK;
+}
 
 TpEdit tp_edit(float angle_degrees, const float* axis3, const float* translation3) {
     float a[3] = {axis3[0], axis3[1], axis3[2]};
@@ -659,15 +705,6 @@ TpEdit tp_edit(float angle_degrees, const float* axis3, const float* translation
     e.c = cosf(ang); e.s = sinf(ang);
     e.tx = translation3[0]; e.ty = translation3[1]; e.tz = translation3[2];
     return e;
-}
-
-int tp_transform_batch(const float* pts, int N, int B, const TpEdit* edits_dev, double* partial, float* out, cudaStream_t st) {
-    const int nblocks = tp_partial_blocks(N);
-    tp_partial_sum_kernel<<<nblocks, 256, 0, st>>>(pts, N, partial);
-    DH_LAUNCH_CHECK();
-    tp_apply_batch_kernel<<<dim3((N + 255) / 256, B), 256, 0, st>>>(pts, N, partial, nblocks, edits_dev, out);
-    DH_LAUNCH_CHECK();
-    return DH_OK;
 }
 
 }  // namespace dh

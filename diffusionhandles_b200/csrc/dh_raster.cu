@@ -234,6 +234,7 @@ static size_t raster_layout(int V, int P, size_t* o_ndc, size_t* o_keys) {
     return o;
 }
 
+
 // ------------------------------------------------------------------------------------------------
 // Mesh mode for B rigid transforms of one scene's foreground (dh_edit_mesh_batch).
 //
@@ -427,6 +428,377 @@ static int mesh_batch_sizes(int B, int V_bg, int F_bg, int V_fg, int F_fg, int H
     return DH_OK;
 }
 
+// ------------------------------------------------------------------------------------------------
+// Mesh mode for B rigid transforms over a table of scenes (dh_edit_mesh_scenes): the one-scene scheme above per scene.  Each
+// scene's background faces are rasterised ONCE, into the key plane of the first edit of that scene, their keys are copied to the
+// scene's other edits, and each edit's moved foreground faces go on top with the index they have in the joined mesh of its scene
+// (F_bg + f).  Edit b is bit-identical to dh_edit_mesh_batch on its scene.
+//
+// dh_edit_mesh_batch keeps its own kernels: run through this path its device time was about 1 % longer at B = 1..16 (DESIGN.md 5),
+// from the per-block descriptor reads of the foreground raster, the moved-vertex transform and the emit pass.
+//
+// Per-scene and per-edit offsets live in two small device tables (SceneDesc, SceneEdit; one upload).  Grids whose x extent
+// depends on a scene (face blocks, centroid blocks, moved vertices) are sized by the largest one and the blocks past a smaller
+// scene's end exit at once: no search over per-edit face ranges is needed, and an idle block costs a block launch.
+// ------------------------------------------------------------------------------------------------
+constexpr unsigned long long kNoKey = 0xFFFFFFFFFFFFFFFFull;
+
+// the concatenated arrays of a scene batch and its device tables
+struct MeshScenes {
+    const float* bg_ndc;      // (sum V_bg,3)
+    const float* bg_verts;    // (sum V_bg,3) world
+    const int32_t* bg_faces;  // (sum F_bg,3) scene-local
+    const float* fg_ndc;      // (sum over edits of V_fg,3)
+    const float* fg_world;    // (sum over edits of V_fg,3) transformed world vertices
+    const float* fg_colors;   // (sum V_fg,3) source x/(W-1), y/(H-1), flag
+    const int32_t* fg_faces;  // (sum F_fg,3) scene-local
+    const SceneDesc* scenes;
+    const SceneEdit* edits;
+};
+
+// the arrays of edit b's scene, as mesh_resolve reads them
+struct MeshEditScene {
+    const float* bg_ndc;
+    const float* bg_verts;
+    const int32_t* bg_faces;
+    int F_bg;
+    const float* fg_ndc;      // (V_fg,3) of this edit
+    const float* fg_world;    // (V_fg,3) of this edit
+    const float* fg_colors;
+    const int32_t* fg_faces;
+};
+
+__device__ __forceinline__ MeshEditScene mesh_edit_scene(const MeshScenes& m, int b) {
+    const SceneEdit& e = m.edits[b];
+    const int out0 = e.out0;
+    const SceneDesc& sc = m.scenes[e.scene];
+    MeshEditScene s;
+    s.bg_ndc = m.bg_ndc + 3 * (size_t)sc.bg_v0;
+    s.bg_verts = m.bg_verts + 3 * (size_t)sc.bg_v0;
+    s.bg_faces = m.bg_faces + 3 * (size_t)sc.bg_f0;
+    s.F_bg = sc.F_bg;
+    s.fg_ndc = m.fg_ndc + 3 * (size_t)out0;
+    s.fg_world = m.fg_world + 3 * (size_t)out0;
+    s.fg_colors = m.fg_colors + 3 * (size_t)sc.fg_v0;
+    s.fg_faces = m.fg_faces + 3 * (size_t)sc.fg_f0;
+    return s;
+}
+
+// the key plane (KS keys, KS even, 16-byte aligned) of every used scene's background raster <- empty
+__global__ void __launch_bounds__(256) raster_keys_clear_kernel(const SceneDesc* __restrict__ scenes, int KS, unsigned long long* keys) {
+    const int plane = scenes[blockIdx.y].plane;
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (plane < 0 || 2 * i >= KS) return;
+    reinterpret_cast<ulonglong2*>(keys + (size_t)plane * KS)[i] = make_ulonglong2(kNoKey, kNoKey);
+}
+
+// the background faces of every used scene (blockIdx.y = scene) into that scene's key plane
+__global__ void raster_faces_scenes_kernel(const float* __restrict__ ndc, const int32_t* __restrict__ faces,
+                                                                  const SceneDesc* __restrict__ scenes, int H, int W, int KS,
+                                                                  RasterSettings st, unsigned long long* keys) {
+    const SceneDesc* sc = scenes + blockIdx.y;
+    const int f = blockIdx.x * blockDim.x + threadIdx.x;
+    const int plane = sc->plane;
+    if (plane < 0 || f >= sc->F_bg) return;
+    const Tri t = load_tri(ndc + 3 * (size_t)sc->bg_v0, faces + 3 * (size_t)sc->bg_f0, f);
+    raster_face(t, (unsigned int)f, H, W, st, keys + (size_t)plane * KS);
+}
+
+// keys of edit b (blockIdx.y) <- the background raster of its scene, 16 bytes per thread; the edit holding the raster is skipped
+__global__ void __launch_bounds__(256) raster_keys_scenes_broadcast_kernel(const SceneDesc* __restrict__ scenes, const SceneEdit* __restrict__ edits,
+                                                                    int KS, unsigned long long* keys) {
+    const int b = blockIdx.y;
+    const int src = scenes[edits[b].scene].plane;
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (src == b || 2 * i >= KS) return;
+    reinterpret_cast<ulonglong2*>(keys + (size_t)b * KS)[i] = reinterpret_cast<const ulonglong2*>(keys + (size_t)src * KS)[i];
+}
+
+// the moved foreground faces of every edit (blockIdx.y = edit), keyed with their index in the joined mesh of its scene
+__global__ void raster_faces_edits_kernel(const float* __restrict__ ndc, const int32_t* __restrict__ faces,
+                                                                 const SceneDesc* __restrict__ scenes, const SceneEdit* __restrict__ edits,
+                                                                 int H, int W, int KS, RasterSettings st, unsigned long long* keys) {
+    const int b = blockIdx.y;
+    const SceneDesc* sc = scenes + edits[b].scene;
+    const int f = blockIdx.x * blockDim.x + threadIdx.x;
+    if (f >= sc->F_fg) return;
+    const Tri t = load_tri(ndc + 3 * (size_t)edits[b].out0, faces + 3 * (size_t)sc->fg_f0, f);
+    raster_face(t, (unsigned int)(sc->F_bg + f), H, W, st, keys + (size_t)b * KS);
+}
+
+// Pixel q with z-buffer entry `key` in an edit of scene s: returns the world z of the winning surface (world_position[..., 2]: 0
+// when the pixel is empty).  `emit` is set when a foreground face wins and its interpolated flag exceeds 0.5, with the source pixel
+// it carries, rounded half-to-even like torch.round.  A background face carries the colour (x, y, 0): its flag is exactly 0, it
+// never emits.
+__device__ __forceinline__ float mesh_scenes_resolve(const MeshEditScene& s, int q, unsigned long long key, int H, int W, const RasterSettings& st,
+                                              bool& emit, float& src_x, float& src_y) {
+    emit = false;
+    if (key == kNoKey) return 0.0f;
+    const int f = (int)(key & 0xFFFFFFFFull);
+    const bool fg = f >= s.F_bg;
+    const int lf = fg ? f - s.F_bg : f;
+    const float* ndc = fg ? s.fg_ndc : s.bg_ndc;
+    const float* verts = fg ? s.fg_world : s.bg_verts;
+    const int32_t* faces = fg ? s.fg_faces : s.bg_faces;
+    const int row = q / W, col = q - row * W;
+    const float px = pix_to_ndc(W - 1 - col, W, H), py = pix_to_ndc(H - 1 - row, H, W);
+    float pz, b0 = -1.0f, b1 = -1.0f, b2 = -1.0f;
+    pixel_in_face(load_tri(ndc, faces, lf), px, py, st, pz, b0, b1, b2);
+    const int i0 = faces[3 * (size_t)lf], i1 = faces[3 * (size_t)lf + 1], i2 = faces[3 * (size_t)lf + 2];
+    const float z = interp_attr(verts, 3, 2, i0, i1, i2, b0, b1, b2);
+    if (fg && interp_attr(s.fg_colors, 3, 2, i0, i1, i2, b0, b1, b2) > 0.5f) {
+        emit = true;
+        src_x = rintf(__fmul_rn(interp_attr(s.fg_colors, 3, 0, i0, i1, i2, b0, b1, b2), (float)(W - 1)));
+        src_y = rintf(__fmul_rn(interp_attr(s.fg_colors, 3, 1, i0, i1, i2, b0, b1, b2), (float)(H - 1)));
+    }
+    return z;
+}
+
+// pass 1 over (pixel, edit): target z (+ pix_to_face when asked for) and the number of correspondences per tile
+__global__ void __launch_bounds__(kMeshTileThreads) mesh_scenes_resolve_count_kernel(MeshScenes m, const unsigned long long* __restrict__ keys,
+                                                                               int H, int W, int KS, int ntiles, RasterSettings st,
+                                                                               float* __restrict__ target_z, int32_t* __restrict__ pix_to_face,
+                                                                               int32_t* __restrict__ tile_counts) {
+    __shared__ int warp_sums[32];
+    const int b = blockIdx.y, tile = blockIdx.x, P = H * W;
+    const MeshEditScene s = mesh_edit_scene(m, b);
+    const size_t eo = (size_t)b * P, ko = (size_t)b * KS;
+    const int q0 = tile * kMeshTile + threadIdx.x * 4;
+    int c = 0;
+#pragma unroll
+    for (int i = 0; i < 4; ++i) {
+        const int q = q0 + i;
+        if (q >= P) continue;
+        const unsigned long long key = keys[ko + q];
+        bool emit;
+        float sx, sy;
+        target_z[eo + q] = mesh_scenes_resolve(s, q, key, H, W, st, emit, sx, sy);
+        c += emit;
+        if (pix_to_face) pix_to_face[eo + q] = key == kNoKey ? -1 : (int32_t)(key & 0xFFFFFFFFull);
+    }
+    c = __reduce_add_sync(0xFFFFFFFFu, c);
+    if (lane_id() == 0) warp_sums[warp_id()] = c;
+    __syncthreads();
+    if (warp_id() == 0) {
+        int t = lane_id() < (int)(blockDim.x >> 5) ? warp_sums[lane_id()] : 0;
+        t = __reduce_add_sync(0xFFFFFFFFu, t);
+        if (lane_id() == 0) tile_counts[b * ntiles + tile] = t;
+    }
+}
+
+// pass 2: the rows [x_src, y_src, x_dst, y_dst] of every edit in target raster order (tile offsets from the counts, then a block
+// scan); only foreground winners are resolved again.  The last tile of an edit publishes n_corr.
+__global__ void __launch_bounds__(kMeshTileThreads) mesh_scenes_emit_kernel(MeshScenes m, const unsigned long long* __restrict__ keys,
+                                                                      int H, int W, int KS, int ntiles, RasterSettings st,
+                                                                      const int32_t* __restrict__ tile_counts, int64_t* __restrict__ corr,
+                                                                      int32_t* __restrict__ n_corr) {
+    __shared__ int scan_smem[33];
+    __shared__ int base_smem;
+    const int b = blockIdx.y, tile = blockIdx.x, P = H * W;
+    if (tile_counts[b * ntiles + tile] == 0 && tile != ntiles - 1) return;     // nothing to emit (uniform over the block)
+    const MeshEditScene s = mesh_edit_scene(m, b);
+    int part = 0;
+    for (int t = threadIdx.x; t < tile; t += blockDim.x) part += tile_counts[b * ntiles + t];
+    int tot;
+    block_exclusive_scan(part, scan_smem, tot);
+    if (threadIdx.x == 0) base_smem = tot;
+    __syncthreads();
+    const int base = base_smem;
+    const size_t eo = (size_t)b * P, ko = (size_t)b * KS;
+    const int q0 = tile * kMeshTile + threadIdx.x * 4;
+    unsigned kmask = 0;
+    float sx[4], sy[4];          // rounded source coordinates, converted to int64 at the store
+#pragma unroll
+    for (int i = 0; i < 4; ++i) {
+        const int q = q0 + i;
+        sx[i] = sy[i] = 0.0f;
+        if (q >= P) continue;
+        const unsigned long long key = keys[ko + q];
+        if (key == kNoKey || (int)(key & 0xFFFFFFFFull) < s.F_bg) continue;
+        bool emit;
+        mesh_scenes_resolve(s, q, key, H, W, st, emit, sx[i], sy[i]);
+        kmask |= (unsigned)emit << i;
+    }
+    int total;
+    int pos = base + block_exclusive_scan(__popc(kmask), scan_smem, total);
+#pragma unroll
+    for (int i = 0; i < 4; ++i) {
+        if (!((kmask >> i) & 1u)) continue;
+        const int q = q0 + i, row = q / W;
+        longlong4 v;
+        v.x = (long long)sx[i]; v.y = (long long)sy[i]; v.z = q - row * W; v.w = row;
+        *reinterpret_cast<longlong4*>(corr + (eo + pos) * 4) = v;
+        ++pos;
+    }
+    if (tile == ntiles - 1 && threadIdx.x == 0) n_corr[b] = base + total;
+}
+
+// Host view of a scene batch: the sizes every check and every launch needs, computed from the host count arrays.
+struct MeshScenesPlan {
+    long long V_bg, F_bg, V_fg, F_fg;   // totals over the scenes
+    long long moved;                    // sum over edits of V_fg of the edit's scene
+    int max_F_bg, max_F_fg, max_V_fg;   // over the scenes an edit uses (foreground: per edit)
+    int tp_partials, max_tp_blocks;     // centroid partial sums over the scenes, and the most of one scene
+    int KS, ntiles;                     // key plane stride (even), compaction tiles per edit
+};
+
+// every size check of dh_edit_mesh_scenes and its workspace query, before anything else
+static int mesh_scenes_plan(int n_scenes, const int32_t* V_bg, const int32_t* F_bg, const int32_t* V_fg, const int32_t* F_fg, int B,
+                            const int32_t* scene_index, int H, int W, MeshScenesPlan& p) {
+    if (!V_bg || !F_bg || !V_fg || !F_fg || !scene_index) return DH_ERR_INVALID_ARGUMENT;
+    if (n_scenes < 1 || B < 1 || H < 1 || W < 1) return DH_ERR_INVALID_ARGUMENT;
+    if (n_scenes > kMaxGridY || B > kMaxGridY) return DH_ERR_UNSUPPORTED;   // one grid row per scene / per edit
+    p = MeshScenesPlan{};
+    bool too_big = false;
+    for (int s = 0; s < n_scenes; ++s) {
+        if (V_bg[s] < 1 || F_bg[s] < 0 || V_fg[s] < 0 || F_fg[s] < 0) return DH_ERR_INVALID_ARGUMENT;
+        if (F_fg[s] > 0 && V_fg[s] == 0) return DH_ERR_INVALID_ARGUMENT;     // faces without vertices
+        p.V_bg += V_bg[s]; p.F_bg += F_bg[s]; p.V_fg += V_fg[s]; p.F_fg += F_fg[s];
+        too_big |= (long long)F_bg[s] + F_fg[s] > 0x7FFFFFFFll;               // joined face indices are 31-bit in the keys
+        p.tp_partials += tp_partial_blocks(V_fg[s]);
+    }
+    for (int b = 0; b < B; ++b) {
+        const int s = scene_index[b];
+        if (s < 0 || s >= n_scenes) return DH_ERR_INVALID_ARGUMENT;
+        p.moved += V_fg[s];
+        p.max_F_bg = max(p.max_F_bg, F_bg[s]);
+        p.max_F_fg = max(p.max_F_fg, F_fg[s]);
+        p.max_V_fg = max(p.max_V_fg, V_fg[s]);
+        p.max_tp_blocks = max(p.max_tp_blocks, tp_partial_blocks(V_fg[s]));
+    }
+    if ((long long)H * W > (1ll << 29)) return DH_ERR_UNSUPPORTED;
+    // vertex and face totals are indexed with 31-bit offsets; the moved vertices are projected as one flat array
+    if (too_big || p.V_bg > 0x7FFFFFFFll || p.F_bg > 0x7FFFFFFFll || p.V_fg > 0x7FFFFFFFll || p.F_fg > 0x7FFFFFFFll ||
+        p.moved > 0x7FFFFFFFll)
+        return DH_ERR_UNSUPPORTED;
+    const int P = H * W;
+    p.KS = (P + 1) & ~1;
+    p.ntiles = (P + kMeshTile - 1) / kMeshTile;
+    return DH_OK;
+}
+
+struct MeshScenesLayout {
+    size_t scenes, edits, partial, bg_ndc, fg_world, fg_ndc, keys, tile_counts, total;
+};
+
+static MeshScenesLayout mesh_scenes_layout(int n_scenes, int B, const MeshScenesPlan& p) {
+    MeshScenesLayout L;
+    size_t o = 0;
+    L.scenes = o;      o = align_up(o + sizeof(SceneDesc) * (size_t)n_scenes, 16);
+    L.edits = o;       o = align_up(o + sizeof(SceneEdit) * (size_t)B, 256);       // [scenes, edits]: one upload
+    L.partial = o;     o = align_up(o + sizeof(double) * 3 * (size_t)p.tp_partials, 256);
+    L.bg_ndc = o;      o = align_up(o + sizeof(float) * 3 * (size_t)p.V_bg, 256);
+    L.fg_world = o;    o = align_up(o + sizeof(float) * 3 * (size_t)p.moved, 256);
+    L.fg_ndc = o;      o = align_up(o + sizeof(float) * 3 * (size_t)p.moved, 256);
+    L.keys = o;        o = align_up(o + sizeof(unsigned long long) * (size_t)p.KS * B, 256);
+    L.tile_counts = o; o = align_up(o + sizeof(int32_t) * (size_t)p.ntiles * B, 256);
+    L.total = o;
+    return L;
+}
+
+static size_t mesh_scenes_workspace(int n_scenes, const int32_t* V_bg, const int32_t* F_bg, const int32_t* V_fg, const int32_t* F_fg,
+                                    int B, const int32_t* scene_index, int H, int W) {
+    MeshScenesPlan p;
+    if (mesh_scenes_plan(n_scenes, V_bg, F_bg, V_fg, F_fg, B, scene_index, H, W, p) != DH_OK) return 0;
+    return mesh_scenes_layout(n_scenes, B, p).total;
+}
+
+static int mesh_scenes(int n_scenes, const float* bg_verts, const int32_t* bg_faces, const int32_t* V_bg, const int32_t* F_bg,
+                       const float* fg_verts, const float* fg_colors, const int32_t* fg_faces, const int32_t* V_fg, const int32_t* F_fg,
+                       int B, const int32_t* scene_index, const float* angles_deg_host, const float* axes_host,
+                       const float* translations_host, int H, int W, const float* R_host9, const float* T_host3, float sx, float sy,
+                       float blur_radius, int cull_backfaces, int perspective_correct, int clip_barycentric, float* target_z,
+                       int64_t* corr, int32_t* n_corr, int32_t* pix_to_face, void* ws, size_t ws_bytes, void* stream) {
+    // every check runs before the first CUDA call
+    DH_REQUIRE(bg_verts && angles_deg_host && axes_host && translations_host && R_host9 && T_host3 && target_z && corr && n_corr && ws);
+    DH_REQUIRE(blur_radius >= 0.0f);
+    DH_REQUIRE((reinterpret_cast<uintptr_t>(corr) & 31) == 0);      // rows are stored as one 32-byte vector
+    MeshScenesPlan p;
+    const int sizes = mesh_scenes_plan(n_scenes, V_bg, F_bg, V_fg, F_fg, B, scene_index, H, W, p);
+    if (sizes != DH_OK) return sizes;
+    DH_REQUIRE(p.F_bg <= 0 || bg_faces);
+    DH_REQUIRE(p.V_fg <= 0 || (fg_verts && fg_colors));
+    DH_REQUIRE(p.F_fg <= 0 || fg_faces);
+    const MeshScenesLayout L = mesh_scenes_layout(n_scenes, B, p);
+    if (ws_bytes < L.total) return DH_ERR_WORKSPACE;
+    // the descriptor tables, uploaded as one block
+    std::vector<char> tables(L.partial);
+    SceneDesc* scenes_h = reinterpret_cast<SceneDesc*>(tables.data() + L.scenes);
+    SceneEdit* edits_h = reinterpret_cast<SceneEdit*>(tables.data() + L.edits);
+    int bg_v0 = 0, bg_f0 = 0, fg_v0 = 0, fg_f0 = 0, partial0 = 0;
+    for (int s = 0; s < n_scenes; ++s) {
+        SceneDesc& d = scenes_h[s];
+        d.bg_v0 = bg_v0; d.V_bg = V_bg[s]; d.bg_f0 = bg_f0; d.F_bg = F_bg[s];
+        d.fg_v0 = fg_v0; d.V_fg = V_fg[s]; d.fg_f0 = fg_f0; d.F_fg = F_fg[s];
+        d.tp_blocks = tp_partial_blocks(V_fg[s]); d.tp_partial0 = partial0;
+        d.plane = -1;
+        bg_v0 += V_bg[s]; bg_f0 += F_bg[s]; fg_v0 += V_fg[s]; fg_f0 += F_fg[s]; partial0 += d.tp_blocks;
+    }
+    int out0 = 0, planes = 0;
+    for (int b = 0; b < B; ++b) {
+        SceneEdit& e = edits_h[b];
+        e.scene = scene_index[b];
+        e.out0 = out0;
+        out0 += V_fg[e.scene];
+        if (V_fg[e.scene] > 0) e.t = tp_edit(angles_deg_host[b], axes_host + 3 * b, translations_host + 3 * b);
+        else e.t = TpEdit{};
+        if (scenes_h[e.scene].plane < 0) {
+            scenes_h[e.scene].plane = b;
+            ++planes;
+        }
+    }
+    char* w = static_cast<char*>(ws);
+    const SceneDesc* scenes = reinterpret_cast<const SceneDesc*>(w + L.scenes);
+    const SceneEdit* edits = reinterpret_cast<const SceneEdit*>(w + L.edits);
+    double* partial = reinterpret_cast<double*>(w + L.partial);
+    float* bg_ndc = reinterpret_cast<float*>(w + L.bg_ndc);
+    float* fg_world = reinterpret_cast<float*>(w + L.fg_world);
+    float* fg_ndc = reinterpret_cast<float*>(w + L.fg_ndc);
+    unsigned long long* keys = reinterpret_cast<unsigned long long*>(w + L.keys);
+    int32_t* tile_counts = reinterpret_cast<int32_t*>(w + L.tile_counts);
+    const RasterCamDev cam = make_raster_cam(R_host9, T_host3, sx, sy);
+    const RasterSettings st = make_raster_settings(blur_radius, cull_backfaces, perspective_correct, clip_barycentric);
+    const int KS = p.KS, ntiles = p.ntiles, pair_blocks = (KS / 2 + 255) / 256;
+    cudaStream_t s = as_stream(stream);
+    DH_CUDA_CHECK(cudaMemcpyAsync(w, tables.data(), tables.size(), cudaMemcpyHostToDevice, s));
+    // backgrounds: projected as one array, each used scene rasterised once into the plane of its first edit, copied to the others
+    raster_keys_clear_kernel<<<dim3(pair_blocks, n_scenes), 256, 0, s>>>(scenes, KS, keys);
+    DH_LAUNCH_CHECK();
+    const int nbg = (int)p.V_bg;
+    raster_project_kernel<<<(nbg + 255) / 256, 256, 0, s>>>(bg_verts, nbg, cam, bg_ndc);
+    DH_LAUNCH_CHECK();
+    if (p.max_F_bg > 0) {
+        raster_faces_scenes_kernel<<<dim3((p.max_F_bg + 127) / 128, n_scenes), 128, 0, s>>>(bg_ndc, bg_faces, scenes, H, W, KS, st, keys);
+        DH_LAUNCH_CHECK();
+    }
+    if (B > planes) {
+        raster_keys_scenes_broadcast_kernel<<<dim3(pair_blocks, B), 256, 0, s>>>(scenes, edits, KS, keys);
+        DH_LAUNCH_CHECK();
+    }
+    // foregrounds: every edit's transform of its scene's vertices, projected as one array, every edit's faces in one launch
+    if (p.moved > 0) {
+        const int rc = tp_transform_scenes(fg_verts, scenes, n_scenes, p.max_tp_blocks, edits, B, p.max_V_fg, partial, fg_world, s);
+        if (rc != DH_OK) return rc;
+        const int nv = (int)p.moved;
+        raster_project_kernel<<<(nv + 255) / 256, 256, 0, s>>>(fg_world, nv, cam, fg_ndc);
+        DH_LAUNCH_CHECK();
+    }
+    if (p.max_F_fg > 0) {
+        raster_faces_edits_kernel<<<dim3((p.max_F_fg + 127) / 128, B), 128, 0, s>>>(fg_ndc, fg_faces, scenes, edits, H, W, KS, st, keys);
+        DH_LAUNCH_CHECK();
+    }
+    MeshScenes m;
+    m.bg_ndc = bg_ndc; m.bg_verts = bg_verts; m.bg_faces = bg_faces;
+    m.fg_ndc = fg_ndc; m.fg_world = fg_world; m.fg_colors = fg_colors; m.fg_faces = fg_faces;
+    m.scenes = scenes; m.edits = edits;
+    const dim3 tgrid(ntiles, B);
+    mesh_scenes_resolve_count_kernel<<<tgrid, kMeshTileThreads, 0, s>>>(m, keys, H, W, KS, ntiles, st, target_z, pix_to_face, tile_counts);
+    DH_LAUNCH_CHECK();
+    mesh_scenes_emit_kernel<<<tgrid, kMeshTileThreads, 0, s>>>(m, keys, H, W, KS, ntiles, st, tile_counts, corr, n_corr);
+    DH_LAUNCH_CHECK();
+    return DH_OK;
+}
+
 }  // namespace dh
 
 using namespace dh;
@@ -470,6 +842,22 @@ int dh_interpolate_face_attributes(const float* attr, int D, const int32_t* face
     raster_interpolate_kernel<<<(H * W + 255) / 256, 256, 0, as_stream(stream)>>>(attr, D, faces, pix_to_face, bary, H * W, out);
     DH_LAUNCH_CHECK();
     return DH_OK;
+}
+
+size_t dh_edit_mesh_scenes_workspace_bytes(int n_scenes, const int32_t* V_bg_host, const int32_t* F_bg_host, const int32_t* V_fg_host, const int32_t* F_fg_host,
+                                           int B, const int32_t* scene_index_host, int H, int W) {
+    return mesh_scenes_workspace(n_scenes, V_bg_host, F_bg_host, V_fg_host, F_fg_host, B, scene_index_host, H, W);
+}
+
+int dh_edit_mesh_scenes(int n_scenes, const float* bg_verts, const int32_t* bg_faces, const int32_t* V_bg_host, const int32_t* F_bg_host,
+                        const float* fg_verts, const float* fg_colors, const int32_t* fg_faces, const int32_t* V_fg_host, const int32_t* F_fg_host,
+                        int B, const int32_t* scene_index_host, const float* angles_deg_host, const float* axes_host,
+                        const float* translations_host, int H, int W, const float* R_host9, const float* T_host3, float sx, float sy,
+                        float blur_radius, int cull_backfaces, int perspective_correct, int clip_barycentric, float* target_z,
+                        int64_t* corr, int32_t* n_corr, int32_t* pix_to_face, void* ws, size_t ws_bytes, void* stream) {
+    return mesh_scenes(n_scenes, bg_verts, bg_faces, V_bg_host, F_bg_host, fg_verts, fg_colors, fg_faces, V_fg_host, F_fg_host, B, scene_index_host,
+                       angles_deg_host, axes_host, translations_host, H, W, R_host9, T_host3, sx, sy, blur_radius, cull_backfaces,
+                       perspective_correct, clip_barycentric, target_z, corr, n_corr, pix_to_face, ws, ws_bytes, stream);
 }
 
 size_t dh_edit_mesh_batch_workspace_bytes(int B, int V_bg, int V_fg, int H, int W) {
@@ -545,5 +933,6 @@ int dh_edit_mesh_batch(const float* bg_verts, int V_bg, const int32_t* bg_faces,
     DH_LAUNCH_CHECK();
     return DH_OK;
 }
+
 
 }  // extern "C"

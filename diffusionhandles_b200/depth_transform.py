@@ -241,10 +241,136 @@ def _edit_count(rot_angles, rot_axes, translations) -> int:
     return B
 
 
-def _empty_mask_batch(depth, use_input_depth_normalization, B):
-    """``_empty_mask_result`` for each of B edits."""
-    disparity, corr = _empty_mask_result(depth, use_input_depth_normalization)
-    return disparity.repeat(B, 1, 1, 1), [corr.clone() for _ in range(B)]
+def _as_scene(t: torch.Tensor, H: int, W: int) -> torch.Tensor:
+    """One image of H x W elements as a (1,1,H,W) scene; anything else is left for the scene checks to reject."""
+    return t.reshape(1, 1, H, W) if t.numel() == H * W else t
+
+
+def _scene_planes(x, name: str) -> torch.Tensor:
+    """Scenes as one (S,1,H,W) tensor: a 4-D tensor is taken as it is, a sequence of (1,1,H,W) tensors is concatenated."""
+    if isinstance(x, torch.Tensor):
+        if x.dim() != 4 or x.shape[1] != 1 or x.shape[0] < 1:
+            raise ValueError(f"{name} must be (S,1,H,W) with at least one scene, got {tuple(x.shape)}")
+        return x
+    x = list(x)
+    if not x:
+        raise ValueError(f"{name} must hold at least one scene")
+    for t in x:
+        if t.shape[0] != 1:
+            raise ValueError(f"one image per scene (batch size 1), got a batch of {t.shape[0]} in {name}")
+    if len({tuple(t.shape) for t in x}) != 1 or x[0].dim() != 4:
+        raise ValueError(f"the scenes of {name} must all be (1,1,H,W) of one size, got {[tuple(t.shape) for t in x]}")
+    return x[0] if len(x) == 1 else torch.cat(x)
+
+
+def _scene_args(depths, bg_depths, fg_masks, scene_index, rot_angles, rot_axes, translations):
+    """Argument checks of the scene calls, before any device work: ``(depths, bg_depths, fg_masks, scene_index list, B)``."""
+    depths, bg_depths, fg_masks = (_scene_planes(x, n) for x, n in ((depths, "depths"), (bg_depths, "bg_depths"), (fg_masks, "fg_masks")))
+    S, H, W = depths.shape[0], depths.shape[-2], depths.shape[-1]
+    for name, t in (("bg_depths", bg_depths), ("fg_masks", fg_masks)):
+        if tuple(t.shape) != (S, 1, H, W):
+            raise ValueError(f"{name} must be {(S, 1, H, W)} like depths, got {tuple(t.shape)}")
+    B = _edit_count(rot_angles, rot_axes, translations)
+    index = [int(i) for i in (scene_index.tolist() if isinstance(scene_index, torch.Tensor) else scene_index)]
+    if len(index) != B:
+        raise ValueError(f"scene_index must have one entry per edit ({B}), got {len(index)}")
+    for i in index:
+        if not 0 <= i < S:
+            raise IndexError(f"scene_index {i} outside [0, {S})")
+    return depths, bg_depths, fg_masks, index, B
+
+
+_ROWS_CHUNK_BYTES = 16 << 20
+
+
+def _rows_to_cpu(corr: torch.Tensor, counts):
+    """The first counts[e] rows of corr[e] (B,P,4) for every edit, on the CPU.  Consecutive edits are copied together in chunks
+    of up to 16 MB: one large copy runs at a higher rate than many small ones, while a host buffer above glibc's largest mmap
+    threshold (32 MB) is mapped and faulted in anew on every call."""
+    out, e = [], 0
+    while e < len(counts):
+        k, n = e + 1, counts[e]
+        while k < len(counts) and (n + counts[k]) * 32 <= _ROWS_CHUNK_BYTES:
+            n += counts[k]
+            k += 1
+        rows = corr[e, :counts[e]] if k == e + 1 else torch.cat([corr[j, :counts[j]] for j in range(e, k)])
+        if k == e + 1:
+            out.append(rows.cpu())
+        else:                                                               # each edit owns its rows
+            out += [r.clone() for r in torch.split(rows.cpu(), counts[e:k])]
+        e = k
+    return out
+
+
+def _gather_planes(planes: torch.Tensor, index) -> torch.Tensor:
+    """planes[index] as one contiguous (len(index),...) tensor; the edits of a single scene expand it (no copy for one edit)."""
+    if len(set(index)) == 1:
+        s = index[0]
+        return planes[s:s + 1].expand(len(index), *planes.shape[1:]).contiguous()
+    return planes.index_select(0, torch.tensor(index, device=planes.device))
+
+
+def _scene_masks_present(fg_masks: torch.Tensor, index):
+    """Which scenes have a foreground, read with one synchronisation (scenes no edit references are not read)."""
+    used = sorted(set(index))
+    masks = fg_masks if len(used) == fg_masks.shape[0] else fg_masks[torch.tensor(used, device=fg_masks.device)]
+    present = masks.flatten(1).any(1).tolist()
+    return dict(zip(used, present))
+
+
+def _empty_mask_edits(depths, index, edits, use_input_depth_normalization, disparity, correspondences):
+    """``_empty_mask_result`` of its scene for each edit in ``edits`` (computed once per scene)."""
+    done = {}
+    for b in edits:
+        s = index[b]
+        if s not in done:
+            done[s] = _empty_mask_result(depths[s:s + 1], use_input_depth_normalization)
+        disparity[b] = done[s][0][0]
+        correspondences[b] = done[s][1].clone()
+
+
+def transform_depth_pc_scenes(depths: torch.Tensor, bg_depths: torch.Tensor, fg_masks: torch.Tensor, intrinsics: torch.Tensor,
+                              scene_index, rot_angles, rot_axes, translations, use_input_depth_normalization=False,
+                              return_device_result: bool = False):
+    """``transform_depth_pc`` for B edits over S scenes as ONE ``EditEngine`` batch.  ``depths`` / ``bg_depths`` / ``fg_masks``
+    are (S,1,H,W) (or sequences of S (1,1,H,W) tensors of one size); edit b transforms scene ``scene_index[b]`` by
+    (``rot_angles[b]``, ``rot_axes[b]``, ``translations[b]``; ``None`` takes the defaults of the single call).  The scene planes
+    are gathered per edit on the device.  Returns ``(disparities (B,1,H,W) fp32, [correspondences (n_b,4) int64 CPU] * B)``,
+    entry b equal bit for bit to ``transform_depth_pc`` on its scene; an edit of a scene without foreground gets that scene's
+    empty-mask result.  With ``return_device_result=True`` the ``EditResult`` of the edits whose scene has a foreground (in edit
+    order; None when there is none) is appended."""
+    depths, bg_depths, fg_masks, index, B = _scene_args(depths, bg_depths, fg_masks, scene_index, rot_angles, rot_axes, translations)
+    H, W = depths.shape[-2:]
+    present = _scene_masks_present(fg_masks, index)
+    live = [b for b in range(B) if present[index[b]]]
+    if live:
+        if H != W:
+            raise RuntimeError(f"the 'pc' depth transform needs a square mask, got {H} x {W}")
+        _require_cuda(depths, "depths")
+    disparity, correspondences, res = [None] * B, [None] * B, None
+    if live:
+        # defaults of the reference: no rotation about +y, no translation (depth_transform.py:219-224)
+        rigids = [make_rigid(0.0 if rot_angles[b] is None else rot_angles[b],
+                             torch.tensor([0.0, 1.0, 0.0]) if rot_axes[b] is None else rot_axes[b],
+                             torch.zeros(3) if translations[b] is None else translations[b]) for b in live]
+        dev, f32 = depths.device, torch.float32
+        d, bg, m = (_gather_planes(t.reshape(-1, H, W).to(device=dev, dtype=f32), [index[b] for b in live])
+                    for t in (depths, bg_depths, fg_masks))
+        res = get_engine(dev, len(live), H, W).run(d, bg, m, intrinsics, rigids,
+                                                   use_input_depth_normalization=use_input_depth_normalization, poisson=True)
+        # one copy per edit: the engine's rows are small (at most one per foreground pixel), and separate copies measured faster
+        # than chunked ones here
+        rows = [res.correspondences(e).cpu() for e in range(len(live))]
+        if len(live) == B:                        # every edit has a foreground: rows are already in edit order
+            out = res.disparity[:, None].clone(), rows
+            return (*out, res) if return_device_result else out
+        for e, b in enumerate(live):
+            disparity[b] = res.disparity[e:e + 1]
+            correspondences[b] = rows[e]
+    _empty_mask_edits(depths, index, [b for b in range(B) if not present[index[b]]], use_input_depth_normalization, disparity,
+                      correspondences)
+    out = torch.stack(disparity), correspondences
+    return (*out, res) if return_device_result else out
 
 
 def transform_depth_pc(depth: torch.Tensor, bg_depth: torch.Tensor, fg_mask: torch.Tensor, intrinsics: torch.Tensor,
@@ -264,31 +390,15 @@ def transform_depth_pc(depth: torch.Tensor, bg_depth: torch.Tensor, fg_mask: tor
 def transform_depth_pc_batch(depth: torch.Tensor, bg_depth: torch.Tensor, fg_mask: torch.Tensor, intrinsics: torch.Tensor,
                              rot_angles, rot_axes, translations, use_input_depth_normalization=False,
                              return_device_result: bool = False):
-    """``transform_depth_pc`` for B transforms of one scene as ONE ``EditEngine`` batch.  ``rot_angles`` / ``rot_axes`` /
-    ``translations`` hold one entry per edit (``None`` takes the defaults of the single call).  Returns ``(disparities
-    (B,1,S,S) fp32 on depth.device, [correspondences (n_b,4) int64 CPU] * B)``, plus the ``EditResult`` (None for an empty
-    mask) with ``return_device_result=True``."""
+    """``transform_depth_pc`` for B transforms of one scene: ``transform_depth_pc_scenes`` with one scene.  ``rot_angles`` /
+    ``rot_axes`` / ``translations`` hold one entry per edit (``None`` takes the defaults of the single call).  Returns
+    ``(disparities (B,1,S,S) fp32 on depth.device, [correspondences (n_b,4) int64 CPU] * B)``, plus the ``EditResult`` (None for
+    an empty mask) with ``return_device_result=True``."""
     B = _edit_count(rot_angles, rot_axes, translations)
-    if not fg_mask.any():
-        res = _empty_mask_batch(depth, use_input_depth_normalization, B)
-        return (*res, None) if return_device_result else res
-    S = fg_mask.shape[-1]
-    if fg_mask.shape[-2] != S:
-        raise RuntimeError(f"the 'pc' depth transform needs a square mask, got {fg_mask.shape[-2]} x {S}")
-    if depth.shape[0] != 1:
-        raise ValueError(f"one image per call (batch size 1), got a batch of {depth.shape[0]}")
-    _require_cuda(depth, "depth")
-    # defaults of the reference: no rotation about +y, no translation (depth_transform.py:219-224)
-    rigids = [make_rigid(0.0 if a is None else a, torch.tensor([0.0, 1.0, 0.0]) if ax is None else ax,
-                         torch.zeros(3) if t is None else t) for a, ax, t in zip(rot_angles, rot_axes, translations)]
-    dev, f32 = depth.device, torch.float32
-    d = depth.reshape(1, S, S).to(f32).expand(B, S, S).contiguous()
-    b = bg_depth.reshape(1, S, S).to(device=dev, dtype=f32).expand(B, S, S).contiguous()
-    m = fg_mask.reshape(1, S, S).to(device=dev, dtype=f32).expand(B, S, S).contiguous()
-    res = get_engine(dev, B, S, S).run(d, b, m, intrinsics, rigids, use_input_depth_normalization=use_input_depth_normalization,
-                                       poisson=True)
-    out = res.disparity[:, None].clone(), [res.correspondences(e).cpu() for e in range(B)]
-    return (*out, res) if return_device_result else out
+    H, W = depth.shape[-2:]
+    scene = [[_as_scene(t, H, W)] for t in (depth, bg_depth, fg_mask)]
+    return transform_depth_pc_scenes(*scene, intrinsics, [0] * B, rot_angles, rot_axes, translations, use_input_depth_normalization,
+                                     return_device_result)
 
 
 def transform_depth_mesh(depth: torch.Tensor, bg_depth: torch.Tensor, fg_mask: torch.Tensor, intrinsics: torch.Tensor,
@@ -306,56 +416,96 @@ def transform_depth_mesh(depth: torch.Tensor, bg_depth: torch.Tensor, fg_mask: t
 
 def transform_depth_mesh_batch(depth: torch.Tensor, bg_depth: torch.Tensor, fg_mask: torch.Tensor, intrinsics: torch.Tensor,
                                rot_angles, rot_axes, translations, use_input_depth_normalization=False):
-    """``transform_depth_mesh`` for B transforms of one scene in one native call (``dh_edit_mesh_batch``).
+    """``transform_depth_mesh`` for B transforms of one scene in one native call: ``transform_depth_mesh_scenes`` with one scene.
 
     Both meshes are built once; the background mesh is rasterised once and every edit's moved foreground faces are rasterised
     over a copy of its z-buffer, which gives the z-buffer of the joined mesh bit for bit.  ``rot_angles`` / ``rot_axes`` /
     ``translations`` hold one entry per edit (``None`` takes the defaults of the single call).  Returns ``(disparities
     (B,1,H,W) fp32 on depth.device, [correspondences (n_b,4) int64 CPU] * B)``; entry b equals bit for bit what the
     renderer reads off the joined mesh [background, foreground moved by transform b]."""
-    from .renderer import MeshRenderer, fov_scales
     B = _edit_count(rot_angles, rot_axes, translations)
-    if not fg_mask.any():
-        return _empty_mask_batch(depth, use_input_depth_normalization, B)
-    _require_cuda(depth, "depth")
-    lib = N.load()
-    dev = depth.device
-    H, W = depth.shape[-2], depth.shape[-1]
-    f32 = torch.float32
-    background = depth_to_mesh(depth=bg_depth, intrinsics=intrinsics)
-    foreground = depth_to_mesh(depth=depth, intrinsics=intrinsics, mask=fg_mask[0, 0] > 0.5)
-    bg_verts = background.verts.to(f32).contiguous()
-    bg_faces = background.faces.to(torch.int32).contiguous()
-    fg_verts = foreground.verts.to(f32).contiguous()
-    fg_colors = foreground.vert_attributes["color"].to(f32).contiguous()
-    fg_faces = foreground.faces.to(torch.int32).contiguous()
-    V_bg, F_bg, V_fg, F_fg = bg_verts.shape[0], bg_faces.shape[0], fg_verts.shape[0], fg_faces.shape[0]
-    # the host values of the single call: the angle through an fp32 tensor, axis / translation as C floats
-    angles, axes, shifts = [], [], []
-    for a, ax, t in zip(rot_angles, rot_axes, translations):
-        angles.append(float(torch.tensor(0.0 if a is None else float(a), dtype=f32)))
-        axes += [float(v) for v in (torch.tensor([0.0, 1.0, 0.0]) if ax is None else ax).detach().cpu().reshape(-1)[:3]]
-        shifts += [float(v) for v in (torch.zeros(3) if t is None else t).detach().cpu().reshape(-1)[:3]]
-    # the camera of the single call: Camera(intrinsics) (identity extrinsics) through MeshRenderer, blur 1e-5, back faces culled
-    sx, sy = fov_scales(intrinsics[1, 1], H, W, MeshRenderer.z_near)
-    R = (C.c_float * 9)(1.0, 0.0, 0.0, 0.0, 1.0, 0.0, 0.0, 0.0, 1.0)
-    T = (C.c_float * 3)(0.0, 0.0, 0.0)
-    target_z = torch.empty((B, H, W), dtype=f32, device=dev)
-    corr = torch.empty((B, H * W, 4), dtype=torch.int64, device=dev)
-    n_corr = torch.empty(B, dtype=torch.int32, device=dev)
-    ws_bytes = int(lib.dh_edit_mesh_batch_workspace_bytes(B, V_bg, V_fg, H, W))
-    if ws_bytes == 0:
-        raise ValueError(f"dh_edit_mesh_batch: unsupported sizes (B={B}, {H}x{W}, {V_bg} + {V_fg} vertices)")
-    ws = torch.empty(ws_bytes, dtype=torch.uint8, device=dev)
-    N.check(lib.dh_edit_mesh_batch(N.ptr(bg_verts), V_bg, N.ptr(bg_faces), F_bg, N.ptr(fg_verts), N.ptr(fg_colors), V_fg,
-                                   N.ptr(fg_faces), F_fg, B, (C.c_float * B)(*angles), (C.c_float * (3 * B))(*axes),
-                                   (C.c_float * (3 * B))(*shifts), H, W, R, T, sx, sy, 1e-5, 1, 1, 1, N.ptr(target_z), N.ptr(corr),
-                                   N.ptr(n_corr), None, N.ptr(ws), ws_bytes, N.stream_handle(dev)), "dh_edit_mesh_batch")
-    counts = n_corr.tolist()                                                 # the one synchronisation
-    rows = corr[:, :max(counts)].cpu()
-    correspondences = [rows[b, :n].clone() for b, n in enumerate(counts)]
-    bounds = normalize_depth(1.0 / depth, return_bounds=True)[1] if use_input_depth_normalization else None
-    return normalize_depth(1.0 / target_z[:, None], bounds=bounds), correspondences
+    H, W = depth.shape[-2:]
+    scene = [[_as_scene(t, H, W)] for t in (depth, bg_depth, fg_mask)]
+    return transform_depth_mesh_scenes(*scene, intrinsics, [0] * B, rot_angles, rot_axes, translations, use_input_depth_normalization)
+
+
+def transform_depth_mesh_scenes(depths: torch.Tensor, bg_depths: torch.Tensor, fg_masks: torch.Tensor, intrinsics: torch.Tensor,
+                                scene_index, rot_angles, rot_axes, translations, use_input_depth_normalization=False):
+    """``transform_depth_mesh`` for B edits over S scenes in one native call (``dh_edit_mesh_scenes``).  Arguments and result
+    as ``transform_depth_pc_scenes``: edit b moves the foreground of scene ``scene_index[b]``, entry b equals bit for bit
+    ``transform_depth_mesh_batch`` on its scene.  The meshes of each scene an edit uses are built once and its background is
+    rasterised once; scenes without foreground give their edits the empty-mask result and are not sent to the kernels."""
+    from .renderer import MeshRenderer, fov_scales
+    depths, bg_depths, fg_masks, index, B = _scene_args(depths, bg_depths, fg_masks, scene_index, rot_angles, rot_axes, translations)
+    H, W = depths.shape[-2:]
+    present = _scene_masks_present(fg_masks, index)
+    live = [b for b in range(B) if present[index[b]]]
+    disparity, correspondences = [None] * B, [None] * B
+    if live:
+        _require_cuda(depths, "depths")
+        lib = N.load()
+        dev = depths.device
+        f32, i32 = torch.float32, torch.int32
+        scenes = sorted({index[b] for b in live})
+        slot = {s: k for k, s in enumerate(scenes)}
+        bg_v, bg_f, fg_v, fg_c, fg_f = [], [], [], [], []
+        for s in scenes:
+            background = depth_to_mesh(depth=bg_depths[s:s + 1], intrinsics=intrinsics)
+            foreground = depth_to_mesh(depth=depths[s:s + 1], intrinsics=intrinsics, mask=fg_masks[s, 0] > 0.5)
+            bg_v.append(background.verts.to(f32))
+            bg_f.append(background.faces.to(i32))
+            fg_v.append(foreground.verts.to(f32))
+            fg_c.append(foreground.vert_attributes["color"].to(f32))
+            fg_f.append(foreground.faces.to(i32))
+        counts = [(C.c_int32 * len(scenes))(*[t.shape[0] for t in ts]) for ts in (bg_v, bg_f, fg_v, fg_f)]
+        bg_verts, bg_faces, fg_verts, fg_colors, fg_faces = (torch.cat(ts).contiguous() for ts in (bg_v, bg_f, fg_v, fg_c, fg_f))
+        n = len(live)
+        table = (C.c_int32 * n)(*[slot[index[b]] for b in live])
+        # the host values of the single call: the angle through an fp32 tensor, axis / translation as C floats
+        angles, axes, shifts = [], [], []
+        for b in live:
+            a, ax, t = rot_angles[b], rot_axes[b], translations[b]
+            angles.append(float(torch.tensor(0.0 if a is None else float(a), dtype=f32)))
+            axes += [float(v) for v in (torch.tensor([0.0, 1.0, 0.0]) if ax is None else ax).detach().cpu().reshape(-1)[:3]]
+            shifts += [float(v) for v in (torch.zeros(3) if t is None else t).detach().cpu().reshape(-1)[:3]]
+        # the camera of the single call: Camera(intrinsics) (identity extrinsics) through MeshRenderer, blur 1e-5, back faces culled
+        sx, sy = fov_scales(intrinsics[1, 1], H, W, MeshRenderer.z_near)
+        R = (C.c_float * 9)(1.0, 0.0, 0.0, 0.0, 1.0, 0.0, 0.0, 0.0, 1.0)
+        T = (C.c_float * 3)(0.0, 0.0, 0.0)
+        target_z = torch.empty((n, H, W), dtype=f32, device=dev)
+        corr = torch.empty((n, H * W, 4), dtype=torch.int64, device=dev)
+        n_corr = torch.empty(n, dtype=i32, device=dev)
+        host = ((C.c_float * n)(*angles), (C.c_float * (3 * n))(*axes), (C.c_float * (3 * n))(*shifts), H, W, R, T, sx, sy, 1e-5, 1, 1, 1,
+                N.ptr(target_z), N.ptr(corr), N.ptr(n_corr), None)
+        if len(scenes) == 1:        # one scene: dh_edit_mesh_batch, whose kernels are faster for it than the scene-table ones
+            ws_bytes = int(lib.dh_edit_mesh_batch_workspace_bytes(n, counts[0][0], counts[2][0], H, W))
+        else:
+            ws_bytes = int(lib.dh_edit_mesh_scenes_workspace_bytes(len(scenes), *counts, n, table, H, W))
+        if ws_bytes == 0:
+            raise ValueError(f"mesh mode: unsupported sizes ({len(scenes)} scenes, {n} edits, {H}x{W}, "
+                             f"{bg_verts.shape[0]} + {fg_verts.shape[0]} vertices)")
+        ws = torch.empty(ws_bytes, dtype=torch.uint8, device=dev)
+        if len(scenes) == 1:
+            N.check(lib.dh_edit_mesh_batch(N.ptr(bg_verts), counts[0][0], N.ptr(bg_faces), counts[1][0], N.ptr(fg_verts), N.ptr(fg_colors),
+                                           counts[2][0], N.ptr(fg_faces), counts[3][0], n, *host, N.ptr(ws), ws_bytes,
+                                           N.stream_handle(dev)), "dh_edit_mesh_batch")
+        else:
+            N.check(lib.dh_edit_mesh_scenes(len(scenes), N.ptr(bg_verts), N.ptr(bg_faces), counts[0], counts[1], N.ptr(fg_verts),
+                                            N.ptr(fg_colors), N.ptr(fg_faces), counts[2], counts[3], n, table, *host, N.ptr(ws), ws_bytes,
+                                            N.stream_handle(dev)), "dh_edit_mesh_scenes")
+        rows_per_edit = n_corr.tolist()                                          # the one synchronisation
+        rows = _rows_to_cpu(corr, rows_per_edit)
+        bounds = (normalize_depth(1.0 / _gather_planes(depths, [index[b] for b in live]), return_bounds=True)[1]
+                  if use_input_depth_normalization else None)
+        disp = normalize_depth(1.0 / target_z[:, None], bounds=bounds)
+        if len(live) == B:                        # every edit has a foreground: rows are already in edit order
+            return disp, rows
+        for e, b in enumerate(live):
+            disparity[b] = disp[e]
+            correspondences[b] = rows[e]
+    _empty_mask_edits(depths, index, [b for b in range(B) if not present[index[b]]], use_input_depth_normalization, disparity,
+                      correspondences)
+    return torch.stack(disparity), correspondences
 
 
 def transform_depth(depth: torch.Tensor, bg_depth: torch.Tensor, fg_mask: torch.Tensor, intrinsics: torch.Tensor,

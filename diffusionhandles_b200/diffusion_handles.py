@@ -11,7 +11,7 @@ from types import SimpleNamespace
 
 import torch
 
-from .depth_transform import normalize_depth, transform_depth, transform_depth_mesh_batch, transform_depth_pc_batch
+from .depth_transform import (_as_scene, _scene_planes, normalize_depth, transform_depth, transform_depth_mesh_scenes, transform_depth_pc_scenes)
 from .guided_stable_diffuser import GuidedStableDiffuser
 
 DEFAULT_CONF = SimpleNamespace(   # diffhandles/config/default.yaml
@@ -59,21 +59,33 @@ class DiffusionHandles:
     def set_foreground(self, depth: torch.Tensor, fg_mask: torch.Tensor, bg_depth: torch.Tensor) -> torch.Tensor:
         """diffusion_handles.py:88-110: background depth = input depth with the (15 px dilated) foreground hole filled by
         a Poisson problem driven by the Laplacian of ``bg_depth``.  Entirely on the device: the dilation is one pass of the
-        bit-packed morphology kernel with the 31 x 31 diamond that 15 iterations of SciPy's cross element amount to."""
+        bit-packed morphology kernel with the 31 x 31 diamond that 15 iterations of SciPy's cross element amount to.  Runs as
+        ``set_foreground_scenes`` with one scene."""
+        H, W = depth.shape[-2:]
+        return self.set_foreground_scenes(_as_scene(depth, H, W), _as_scene(fg_mask, H, W), _as_scene(bg_depth, H, W))
+
+    def set_foreground_scenes(self, depths: torch.Tensor, fg_masks: torch.Tensor, bg_depths: torch.Tensor) -> torch.Tensor:
+        """``set_foreground`` for S scenes of one size ((S,1,H,W) tensors or sequences of S (1,1,H,W) tensors): one dilation launch
+        and one Poisson launch for all of them (the S systems are independent).  Returns (S,1,H,W); entry s equals
+        ``set_foreground`` of scene s bit for bit."""
         from . import _native as N
         from .depth_transform import _pack_mask, _poisson_device
+        depths, fg_masks, bg_depths = (_scene_planes(x, n) for x, n in ((depths, "depths"), (fg_masks, "fg_masks"), (bg_depths, "bg_depths")))
+        S, H, W = depths.shape[0], depths.shape[-2], depths.shape[-1]
+        for name, t in (("fg_masks", fg_masks), ("bg_depths", bg_depths)):
+            if tuple(t.shape) != (S, 1, H, W):
+                raise ValueError(f"{name} must be {(S, 1, H, W)} like depths, got {tuple(t.shape)}")
         lib = N.load()
-        dev = depth.device
-        H, W = depth.shape[-2:]
-        d = depth.reshape(1, H, W).to(torch.float32).contiguous()
-        b = bg_depth.reshape(1, H, W).to(device=dev, dtype=torch.float32).contiguous()
-        bits = _pack_mask((fg_mask.reshape(1, H, W).to(dev) != 0).to(torch.float32).contiguous())
+        dev = depths.device
+        d = depths.reshape(S, H, W).to(torch.float32).contiguous()
+        b = bg_depths.reshape(S, H, W).to(device=dev, dtype=torch.float32).contiguous()
+        bits = _pack_mask((fg_masks.reshape(S, H, W).to(dev) != 0).to(torch.float32).contiguous())
         r = 15
         rows = N.u32_array([((1 << (2 * (r - abs(i - r)) + 1)) - 1) << abs(i - r) for i in range(2 * r + 1)])
         dil = torch.empty_like(bits)
-        N.check(lib.dh_morph_pass(N.ptr(bits), N.ptr(dil), 1, H, W, rows, 2 * r + 1, 2 * r + 1, 1, N.stream_handle(dev)), "dh_morph_pass")
+        N.check(lib.dh_morph_pass(N.ptr(bits), N.ptr(dil), S, H, W, rows, 2 * r + 1, 2 * r + 1, 1, N.stream_handle(dev)), "dh_morph_pass")
         # (the reference's set_foreground is synchronous CPU code: the convergence check's small read-back costs nothing extra)
-        return _poisson_device(d, dil, lap_source=b, check=True, what="set_foreground")[None]
+        return _poisson_device(d, dil, lap_source=b, check=True, what="set_foreground")[:, None]
 
     def edit_geometry(self, depth: torch.Tensor, fg_mask: torch.Tensor, bg_depth: torch.Tensor, rot_angle: float = None,
                       rot_axis: torch.Tensor = None, translation: torch.Tensor = None, use_input_depth_normalization=False):
@@ -106,30 +118,68 @@ class DiffusionHandles:
 
     def edit_geometry_batch(self, depth: torch.Tensor, fg_mask: torch.Tensor, bg_depth: torch.Tensor, rot_angles, rot_axes,
                             translations, use_input_depth_normalization=False):
-        """B transforms of one scene: edited disparities (B,1,H,W) and a list of B correspondence lists, each equal bit for bit
-        to ``edit_geometry`` with that transform.  In 'pc' mode the B edits are ONE ``EditEngine`` batch
-        (``transform_depth_pc_batch``); in 'mesh' mode they are ONE ``transform_depth_mesh_batch`` call (the background mesh
-        rasterised once)."""
-        batch = {"pc": transform_depth_pc_batch, "mesh": transform_depth_mesh_batch}.get(self.conf.depth_transform_mode)
-        if batch is None:
+        """B transforms of one scene: ``edit_geometry_scenes`` with one scene.  Edited disparities (B,1,H,W) and a list of B
+        correspondence lists, each equal bit for bit to ``edit_geometry`` with that transform."""
+        H, W = depth.shape[-2:]
+        return self.edit_geometry_scenes([_as_scene(depth, H, W)], [_as_scene(fg_mask, H, W)], [_as_scene(bg_depth, H, W)], [0] * len(rot_angles),
+                                         rot_angles, rot_axes, translations, use_input_depth_normalization)
+
+    def edit_geometry_scenes(self, depths, fg_masks, bg_depths, scene_index, rot_angles, rot_axes, translations,
+                             use_input_depth_normalization=False):
+        """B edits over S scenes of one size (``depths`` / ``fg_masks`` / ``bg_depths`` (S,1,H,W) or sequences of S (1,1,H,W)
+        tensors; edit b transforms scene ``scene_index[b]``).  In 'pc' mode the edits are ONE ``EditEngine`` batch
+        (``transform_depth_pc_scenes``), in 'mesh' mode ONE ``dh_edit_mesh_scenes`` call (``transform_depth_mesh_scenes``).
+        Returns (disparities (B,1,H,W), [correspondences (n_b,4) int64 CPU] * B), entry b equal bit for bit to ``edit_geometry``
+        of its scene with its transform."""
+        scenes = {"pc": transform_depth_pc_scenes, "mesh": transform_depth_mesh_scenes}.get(self.conf.depth_transform_mode)
+        if scenes is None:
             raise ValueError(f"Unknown depth transform mode '{self.conf.depth_transform_mode}'.")
+        dev = (depths if isinstance(depths, torch.Tensor) else depths[0]).device
         with torch.no_grad():
-            return batch(depth, bg_depth, fg_mask, self.diffuser.get_depth_intrinsics(device=depth.device), rot_angles, rot_axes,
-                         translations, use_input_depth_normalization)
+            return scenes(depths, bg_depths, fg_masks, self.diffuser.get_depth_intrinsics(device=dev), scene_index, rot_angles, rot_axes,
+                          translations, use_input_depth_normalization)
 
     def transform_foreground_batch(self, depth: torch.Tensor, prompt: str, fg_mask: torch.Tensor, bg_depth: torch.Tensor,
                                    null_text_emb: torch.Tensor, init_noise: torch.Tensor, activations: list, rot_angles, rot_axes,
                                    translations, fg_weight: float = None, bg_weight: float = None, use_input_depth_normalization=False):
-        """``transform_foreground`` for B transforms of one scene: the geometry of all B edits in one batch
-        (``edit_geometry_batch``), then the injected diffuser's ``guided_inference_batch`` with ``init_noise`` and the identity
-        ``activations`` shared by every edit; the geometry is batched in both depth transform modes ('pc' and 'mesh').  Returns
-        (edited images (B,...), edited disparities (B,1,H,W)).  Saving the denoising steps is not supported in batch mode."""
+        """``transform_foreground`` for B transforms of one scene: ``transform_foreground_scenes`` with one scene, whose prompt,
+        ``init_noise`` and identity ``activations`` every edit shares.  Returns (edited images (B,...), edited disparities
+        (B,1,H,W)).  Saving the denoising steps is not supported in batch mode."""
+        H, W = depth.shape[-2:]
+        return self.transform_foreground_scenes([_as_scene(depth, H, W)], [prompt], [_as_scene(fg_mask, H, W)], [_as_scene(bg_depth, H, W)],
+                                                [null_text_emb], [init_noise], [activations], [0] * len(rot_angles), rot_angles, rot_axes,
+                                                translations, fg_weight, bg_weight, use_input_depth_normalization)
+
+    def transform_foreground_scenes(self, depths, prompts, fg_masks, bg_depths, null_text_embs, init_noises, identities, scene_index,
+                                    rot_angles, rot_axes, translations, fg_weight: float = None, bg_weight: float = None,
+                                    use_input_depth_normalization=False):
+        """``transform_foreground`` for B edits over S scenes: the geometry of all edits in one batch (``edit_geometry_scenes``),
+        then ONE ``guided_inference_batch`` in which edit b takes the prompt, null-text sequence, initial noise and identity of
+        its scene ``scene_index[b]`` (``prompts``, ``null_text_embs``, ``init_noises``, ``identities``: one entry per scene; the
+        identities are referenced, never copied).  When every edit is of one scene, that scene's values are passed as shared
+        ones.  Returns (edited images (B,...), edited disparities (B,1,H,W)).  Saving the denoising steps is not supported in
+        batch mode."""
         guided = self._need(self.diffuser, "guided_inference_batch")
         if self.conf.guided_diffuser.save_denoising_steps:
             raise NotImplementedError("transform_foreground_batch does not save the denoising steps; use transform_foreground per edit")
-        disparities, correspondences = self.edit_geometry_batch(depth, fg_mask, bg_depth, rot_angles, rot_axes, translations,
-                                                                use_input_depth_normalization)
+        S = len(depths)
+        for name, v in (("prompts", prompts), ("null_text_embs", null_text_embs), ("init_noises", init_noises), ("identities", identities)):
+            if len(v) != S:
+                raise ValueError(f"{name} must have one entry per scene ({S}), got {len(v)}")
+        disparities, correspondences = self.edit_geometry_scenes(depths, fg_masks, bg_depths, scene_index, rot_angles, rot_axes,
+                                                                 translations, use_input_depth_normalization)
+        index = [int(i) for i in scene_index]
+        if len(set(index)) == 1:
+            s = index[0]
+            prompt, uncond, latents, acts = prompts[s], null_text_embs[s], init_noises[s], identities[s]
+        else:
+            prompt = [prompts[s] for s in index]
+            if not all(isinstance(p, str) for p in prompt):
+                prompt = torch.cat([prompts[s] for s in index])              # per-edit embedding rows (B,L,D)
+            uncond = [null_text_embs[s] for s in index]
+            latents = torch.cat([init_noises[s] for s in index])
+            acts = [identities[s] for s in index]
         with torch.no_grad():
-            images = guided(latents=init_noise, depth=disparities, uncond_embeddings=null_text_emb, prompt=prompt,
-                            activations_orig=activations, correspondences=correspondences, fg_weight=fg_weight, bg_weight=bg_weight)
+            images = guided(latents=latents, depth=disparities, uncond_embeddings=uncond, prompt=prompt, activations_orig=acts,
+                            correspondences=correspondences, fg_weight=fg_weight, bg_weight=bg_weight)
         return images, disparities

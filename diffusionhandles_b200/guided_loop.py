@@ -203,7 +203,8 @@ def _denoise(batch, latents, timesteps, unet, scheduler_step, activations_orig, 
         raise ValueError("either scheduler_step or (ddim, cfg_pair) is required")
     if fused_update:           # the timestep values index the coefficient table on the host: one read-back for the whole loop
         t_host = [int(v) for v in (timesteps.tolist() if isinstance(timesteps, (torch.Tensor, np.ndarray)) else timesteps)]
-    # batch mode: one identity shared by every edit, or one identity per edit (its per-step slices are stacked to (B,C,h,w))
+    # batch mode: one identity shared by every edit, or one identity per edit (the loss kernel reads each edit's per-step slice in
+    # place; edits of one scene may share an identity)
     per_edit_orig = batch and not isinstance(activations_orig[0], torch.Tensor)
     ident = activations_orig[0] if per_edit_orig else activations_orig
     for t_idx, t in enumerate(timesteps):
@@ -216,7 +217,7 @@ def _denoise(batch, latents, timesteps, unet, scheduler_step, activations_orig, 
                 fgw, bgw = schedule(t_idx, iteration)
                 acts = list(activations) if batch else [a[0] for a in activations]
                 if per_edit_orig:
-                    origs = [torch.stack([ao[l][t_idx] for ao in activations_orig]) for l in range(len(acts))]
+                    origs = [[ao[l][t_idx] for ao in activations_orig] for l in range(len(acts))]
                 else:
                     origs = [a[t_idx] for a in activations_orig]
                 activations_size = (ident[2][t_idx].shape[-2], ident[2][t_idx].shape[-1])

@@ -209,13 +209,15 @@ class GuidedStableDiffuser:
         return self._guided_inference(False, latents, depth, uncond_embeddings, prompt, activations_orig, correspondences, fg_weight,
                                       bg_weight, save_denoising_steps)
 
-    def guided_inference_batch(self, latents: torch.Tensor, depth: torch.Tensor, uncond_embeddings: torch.Tensor, prompt: str,
+    def guided_inference_batch(self, latents: torch.Tensor, depth: torch.Tensor, uncond_embeddings, prompt,
                                activations_orig, correspondences, fg_weight: float = None, bg_weight: float = None):
         """``guided_inference`` for B edits at once (``guided_denoise_batch``): the U-Net runs at batch B, each guided step
         evaluates the losses of all edits in one K4 launch.  ``depth`` is (B,1,H,W), ``correspondences`` a list of B (N,4)
         lists; ``latents`` (1,4,h,w) is shared by every edit, or (B,4,h,w); ``activations_orig`` is one identity shared by every
-        edit, or a list of B identities.  Returns the B decoded images.  The saved denoising steps of ``save_denoising_steps``
-        are not supported here."""
+        edit, or a list of B identities.  ``prompt`` is one prompt (string or embedding) shared by every edit, a list of B
+        strings or a (B,L,D) embedding; ``uncond_embeddings`` is one null-text sequence shared by every edit or a list of B
+        sequences, so edits of different images run in one batch.  Returns the B decoded images.  The saved denoising steps of
+        ``save_denoising_steps`` are not supported here."""
         return self._guided_inference(True, latents, depth, uncond_embeddings, prompt, activations_orig, correspondences, fg_weight,
                                       bg_weight, False)
 
@@ -238,6 +240,10 @@ class GuidedStableDiffuser:
                 raise ValueError(f"depth must be (B,1,H,W) with B = {B} edits, got {tuple(depth.shape)}")
             if latents.shape[0] not in (1, B):
                 raise ValueError(f"latents must be (1,4,h,w) or ({B},4,h,w), got {tuple(latents.shape)}")
+            if isinstance(uncond_embeddings, (list, tuple)) and len(uncond_embeddings) != B:
+                raise ValueError(f"uncond_embeddings must be one sequence or a list of B = {B} sequences, got {len(uncond_embeddings)}")
+            if isinstance(prompt, (list, tuple)) and len(prompt) != B:
+                raise ValueError(f"prompt must be one prompt or a list of B = {B} prompts, got {len(prompt)}")
         fg_weight = self._conf("fg_weight", 1.5) if fg_weight is None else fg_weight
         bg_weight = self._conf("bg_weight", 1.25) if bg_weight is None else bg_weight
         use_depth = self._conf("use_depth", True)
@@ -249,11 +255,22 @@ class GuidedStableDiffuser:
             pcs = [self.process_correspondences(c, img_res=depth.shape[-1], bg_erosion=self._conf("bg_erosion", 0)) for c in corrs]
             if use_depth:
                 depth = self.init_depth(depth)
-            cond = self._encode_prompt(prompt)
+            if batch and isinstance(prompt, (list, tuple)):
+                cond = torch.cat([self._encode_prompt(p) for p in prompt])
+            else:
+                cond = self._encode_prompt(prompt)
             extra = self.prepare_extra_step_kwargs(generator, 0.0)
             if batch:
+                if cond.shape[0] not in (1, B):
+                    raise ValueError(f"the prompt embedding must be (1,L,D) or ({B},L,D), got {tuple(cond.shape)}")
                 cond = cond.expand(B, *cond.shape[1:])
                 latents = latents.expand(B, *latents.shape[1:]).contiguous()
+
+        def uncond_at(t_idx):
+            """the null-text embedding of step t_idx: shared, or each edit's own stacked to (B,L,D)"""
+            if batch and isinstance(uncond_embeddings, (list, tuple)):
+                return torch.cat([u[t_idx].expand(1, *cond.shape[1:]) for u in uncond_embeddings])
+            return uncond_embeddings[t_idx]
 
         def unet_fn(model_in, t):
             if use_depth:
@@ -262,7 +279,7 @@ class GuidedStableDiffuser:
             return out[0], [out[4], out[5], out[6]]
 
         def cfg_pair(lat, t, t_idx):
-            return self._cfg_forward(lat, t, uncond_embeddings[t_idx], cond, depth if use_depth else None)
+            return self._cfg_forward(lat, t, uncond_at(t_idx), cond, depth if use_depth else None)
 
         def cfg_noise(lat, t, t_idx):
             n_uncond, n_text = cfg_pair(lat, t, t_idx)

@@ -327,7 +327,8 @@ def guidance_loss_and_grad_batch(activations: Sequence[torch.Tensor], activation
     """``guidance_loss_and_grad`` for B edits at once: ONE K4 launch per 16 edits (dh_guidance_loss_batch).
 
     ``activations[l]`` is (B,C_l,h_l,w_l), what a U-Net run at batch B returns; ``activations_orig[l]`` is (C_l,h_l,w_l), shared
-    by every edit (variants of one image), or (B,C_l,h_l,w_l); ``processed_correspondences`` holds B dicts.  The weights are
+    by every edit (variants of one image), (B,C_l,h_l,w_l), or a sequence of B (C_l,h_l,w_l) tensors - one identity per edit,
+    read in place (edits may share a tensor); ``processed_correspondences`` holds B dicts.  The weights are
     the same for every edit.  Returns (totals (B,), parts (B,2L), [grad_l (B,C_l,h_l,w_l)]): row / slice e is bit-identical to
     what ``guidance_loss_and_grad`` returns for edit e alone.  Inputs that the single-edit call sends to the general patch kernel
     (patch_size > 1, map areas that are not a multiple of 4, 'local_avg' on resized layers) run one such launch per edit.  A chunk
@@ -344,18 +345,23 @@ def guidance_loss_and_grad_batch(activations: Sequence[torch.Tensor], activation
     for a, o in zip(activations, activations_orig):
         if a.dim() != 4 or a.shape[0] != B:
             raise ValueError(f"activations must be (B,C,h,w) with B = {B} edits, got {tuple(a.shape)}")
-        if tuple(o.shape) not in (tuple(a.shape[1:]), tuple(a.shape)):
-            raise ValueError(f"recorded activations must be (C,h,w) or (B,C,h,w) of the activations' shape, got {tuple(o.shape)}")
+        if isinstance(o, torch.Tensor):
+            if tuple(o.shape) not in (tuple(a.shape[1:]), tuple(a.shape)):
+                raise ValueError(f"recorded activations must be (C,h,w) or (B,C,h,w) of the activations' shape, got {tuple(o.shape)}")
+        elif len(o) != B or any(tuple(t.shape) != tuple(a.shape[1:]) for t in o):
+            raise ValueError(f"a per-edit list of recorded activations must hold B = {B} tensors of shape {tuple(a.shape[1:])}")
     dev = activations[0].device
     if dev.type != "cuda":
         raise N.NativeLibraryError("guidance losses run on CUDA only; there is no CPU fallback")
+    # the recorded activations of every (layer, edit): views, no copy
+    orig_rows = [[o if isinstance(o, torch.Tensor) and o.dim() == 3 else o[e] for e in range(B)] for o in activations_orig]
     plans = [_plan_for(pc, grid, dev) for pc in pcs]
     shapes = tuple(tuple(a.shape[1:]) for a in activations)
     out = torch.empty(B, 1 + 2 * L, dtype=torch.float32, device=dev)
     if _needs_general(shapes, grid, patch, bg_kind):
         grads = [torch.empty((B,) + sh, dtype=torch.float32, device=dev) for sh in shapes]
         for e in range(B):
-            o, g = _launch([a[e] for a in activations], [o if o.dim() == 3 else o[e] for o in activations_orig], [True] * L,
+            o, g = _launch([a[e] for a in activations], [rows[e] for rows in orig_rows], [True] * L,
                            fg_weights, bg_weights, plans[e], _FG, bg_kind, patch)
             out[e] = o
             for l in range(L):
@@ -363,11 +369,16 @@ def guidance_loss_and_grad_batch(activations: Sequence[torch.Tensor], activation
         return out[:, 0], out[:, 1:], grads
     lib = N.load()
     curs = [_as_f32(a, dev) for a in activations]
-    origs = [_as_f32(o, dev) for o in activations_orig]
+    converted = {}                     # one conversion per distinct tensor (a shared identity is converted once)
+    for rows in orig_rows:
+        for t in rows:
+            if id(t) not in converted:
+                converted[id(t)] = _as_f32(t, dev)
+    origs = [[converted[id(t)] for t in rows] for rows in orig_rows]        # kept alive until the launches are enqueued
     grads = [torch.empty_like(c) for c in curs]
     plane = [4 * sh[0] * sh[1] * sh[2] for sh in shapes]        # bytes of one edit's slice of layer l
     cur_p, grad_p = [c.data_ptr() for c in curs], [g.data_ptr() for g in grads]
-    org_p = [(o.data_ptr(), 0 if o.dim() == 3 else plane[l]) for l, o in enumerate(origs)]
+    org_p = [[t.data_ptr() for t in rows] for rows in origs]
     st = N.stream_handle(dev)
     for b0 in range(0, B, MAX_BATCH_EDITS):
         chunk = plans[b0:b0 + MAX_BATCH_EDITS]
@@ -376,7 +387,7 @@ def guidance_loss_and_grad_batch(activations: Sequence[torch.Tensor], activation
             e = b0 + j
             for l in range(L):
                 layers[l].cur, layers[l].grad = cur_p[l] + e * plane[l], grad_p[l] + e * plane[l]
-                layers[l].orig = org_p[l][0] + e * org_p[l][1]
+                layers[l].orig = org_p[l][e]
                 layers[l].fg_weight, layers[l].bg_weight = float(fg_weights[l]), float(bg_weights[l])
             edits[j].loss_out = out.data_ptr() + 4 * e * (1 + 2 * L)
         N.check(lib.dh_guidance_loss_batch(edits, len(chunk), grid, _FG, bg_kind, ws.data_ptr(), ws_bytes, st), "dh_guidance_loss_batch")

@@ -368,6 +368,30 @@ int dh_edit_mesh_batch(const float* bg_verts, int V_bg, const int32_t* bg_faces,
                        float* target_z, int64_t* corr, int32_t* n_corr, int32_t* pix_to_face, void* ws, size_t ws_bytes,
                        void* stream);
 
+/* ---- mesh mode for B transforms over a table of scenes -------------------------------------------
+ * dh_edit_mesh_batch for edits of several images in one call.  All scenes share H, W and the camera.  Scene s has V_bg[s]
+ * background vertices and F_bg[s] faces, V_fg[s] foreground vertices (with colours) and F_fg[s] faces (the host int32 arrays
+ * V_bg_host, F_bg_host, V_fg_host, F_fg_host of n_scenes entries); the device arrays hold the scenes concatenated in order: bg_verts (sum V_bg,3), bg_faces (sum F_bg,3),
+ * fg_verts / fg_colors (sum V_fg,3), fg_faces (sum F_fg,3), faces with scene-local vertex ids.  Edit b moves the foreground of
+ * scene scene_index_host[b] by its transform (angles_deg_host[b], axes_host[3b..], translations_host[3b..]).  Outputs as for
+ * dh_edit_mesh_batch, one plane / row block per edit; pix_to_face holds the joined face index of the edit's scene.
+ * Contract: edit b equals, bit for bit, dh_edit_mesh_batch on scene scene_index_host[b] with that transform.  Each scene
+ * referenced by an edit is rasterised once; scenes no edit references are projected but not rasterised.  One upload of the
+ * descriptor tables, no allocation, no synchronisation; every check runs before any CUDA call: DH_ERR_INVALID_ARGUMENT for NULL
+ * required pointers, n_scenes < 1, B < 1, a scene index outside [0, n_scenes), V_bg < 1, negative counts, F_fg > 0 without
+ * vertices, a negative or NaN blur_radius, corr not 32-byte aligned; DH_ERR_UNSUPPORTED for B or n_scenes > 65535, H*W > 2^29,
+ * vertex or face totals, the moved-vertex total (sum over edits of V_fg) or a scene's F_bg + F_fg above 2^31 - 1.  The workspace
+ * query returns 0 for sizes the call rejects. */
+size_t dh_edit_mesh_scenes_workspace_bytes(int n_scenes, const int32_t* V_bg_host, const int32_t* F_bg_host, const int32_t* V_fg_host,
+                                           const int32_t* F_fg_host, int B, const int32_t* scene_index_host, int H, int W);
+int dh_edit_mesh_scenes(int n_scenes, const float* bg_verts, const int32_t* bg_faces, const int32_t* V_bg_host, const int32_t* F_bg_host,
+                        const float* fg_verts, const float* fg_colors, const int32_t* fg_faces, const int32_t* V_fg_host,
+                        const int32_t* F_fg_host, int B, const int32_t* scene_index_host, const float* angles_deg_host,
+                        const float* axes_host, const float* translations_host, int H, int W, const float* R_host9,
+                        const float* T_host3, float sx, float sy, float blur_radius, int cull_backfaces, int perspective_correct,
+                        int clip_barycentric, float* target_z, int64_t* corr, int32_t* n_corr, int32_t* pix_to_face, void* ws,
+                        size_t ws_bytes, void* stream);
+
 #if defined(__GNUC__)
 #pragma GCC visibility pop
 #endif
