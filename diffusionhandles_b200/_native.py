@@ -99,6 +99,9 @@ _SIGNATURES = {
     "dh_guidance_loss_patch_workspace_bytes": (c_size_t, [c_int, c_int]),
     "dh_guidance_loss_patch": (c_int, [C.POINTER(dh_loss_layer), c_int, c_int, c_int, c_void_p, c_int, c_int, c_int, c_int, c_int,
                                        c_int, c_void_p, c_void_p, c_size_t, c_void_p]),
+    "dh_guidance_loss_patch_batch_workspace_bytes": (c_size_t, [c_int, c_int, c_int]),
+    "dh_guidance_loss_patch_batch": (c_int, [C.POINTER(dh_loss_batch_edit), c_int, c_int, c_int, c_int, c_int, c_void_p, c_size_t,
+                                             c_void_p]),
     "dh_loss_resize_tables_bytes": (c_size_t, []),
     "dh_build_loss_resize_tables": (c_int, [c_void_p, c_int, c_int, c_int, c_int, c_int, c_int, c_void_p, c_void_p]),
     "dh_loss_plan_bytes": (c_size_t, [c_int, c_int]),

@@ -650,12 +650,8 @@ __device__ __forceinline__ void pair_term(float fm, float d, float& acc, float& 
 // kGroups: groups per CTA the kernel is compiled for.  3 (80 registers) is the general build; 4 (64 registers, 1024 threads) is
 // compiled WITHOUT the resized-layer path and is used for launches whose layers all have the loss-grid resolution - which is what
 // guided_inference issues with the reference's weight schedule (its only resized layer always has weight 0 and is skipped).
-// Where a CTA sits among the CTAs that serve its edit: the whole grid (loss_fused_kernel) or the edit's share of the grid
-// (loss_fused_batch_kernel).  The single-edit position reads blockIdx / gridDim where they are used, as a plain kernel would.
-struct WholeGrid {
-    __device__ __forceinline__ unsigned int index() const { return blockIdx.x; }
-    __device__ __forceinline__ unsigned int count() const { return gridDim.x; }
-};
+// Where a CTA sits among the CTAs that serve its edit: the whole grid (loss_fused_kernel; WholeGrid, dh_loss_plan.cuh) or the
+// edit's share of the grid (loss_fused_batch_kernel).  The single-edit position reads blockIdx / gridDim where they are used, as a plain kernel would.
 struct EditShare {
     // shared memory: first CTA of the edit, CTAs of the edit (read where used rather than held in registers: the 3-group body
     // runs at its 80-register cap, and two more live registers cost spills)
@@ -1058,7 +1054,6 @@ __global__ void __launch_bounds__(kLossThreads * kGroups, 1) loss_fused_kernel(c
 // loss_fused_kernel launch of cta_begin[e + 1] - cta_begin[e] CTAs would (own queue, ticket, partials and loss_out; the last
 // CTA of the edit reduces it and re-arms its counters).  Launch-wide: the instantiation, the group count and the shared-memory
 // carve-out (ell_floats / tab_floats / scratch_floats are the maxima over the edits, so that the group bases line up).
-constexpr int kMaxBatchEdits = 16;
 struct FusedBatchParams {
     FusedParams edit[kMaxBatchEdits];
     int cta_begin[kMaxBatchEdits + 1];

@@ -12,6 +12,9 @@
 // accumulates the sign terms of the pairs (associative -> the gradient is bit-reproducible), and the gradient, which is
 // brought back through the transposed box filter and the transposed bilinear resize in gather form (no float atomics).
 // The per-channel loss terms go to a partial array that a one-CTA kernel reduces in a fixed order.
+//
+// dh_guidance_loss_patch_batch runs up to 16 edits in one launch: every CTA serves one edit with that edit's parameters and
+// partial array, and the finish kernel reduces each edit in its own CTA, so every edit gets the bits of its own launch.
 #include "dh_common.cuh"
 #include "dh_loss_plan.cuh"
 
@@ -132,7 +135,10 @@ __device__ float local_term(const PatchParams& p, const PlanView& pv, const floa
     return acc;
 }
 
-__global__ void __launch_bounds__(kPatchThreads, 1) loss_patch_kernel(const __grid_constant__ PatchParams p) {
+// The work of CTA cta.index() of the cta.count() CTAs that serve one edit: the edit's weight maps and denominators, then the
+// planes index, index + count, ...  A plane's partial and gradient do not depend on which CTA computes them.
+template <class Cta>
+__device__ __forceinline__ void loss_patch_body(const PatchParams& p, Cta cta) {
     extern __shared__ __align__(16) float psm[];
     __shared__ float red[kPatchWarps];
     __shared__ int tap0[2][kMaxG], tap1[2][kMaxG];       // [0] rows, [1] columns of the current layer
@@ -172,7 +178,7 @@ __global__ void __launch_bounds__(kPatchThreads, 1) loss_patch_kernel(const __gr
     }
 
     int cur_layer = -1;
-    for (int gc = blockIdx.x; gc < p.total_channels; gc += gridDim.x) {
+    for (int gc = cta.index(); gc < p.total_channels; gc += cta.count()) {
         int l = 0;
         for (int i = 1; i < p.n_layers; ++i)
             if (gc >= p.lv[i].chan_begin) l = i;
@@ -287,8 +293,35 @@ __global__ void __launch_bounds__(kPatchThreads, 1) loss_patch_kernel(const __gr
     }
 }
 
+__global__ void __launch_bounds__(kPatchThreads, 1) loss_patch_kernel(const __grid_constant__ PatchParams p) {
+    loss_patch_body(p, WholeGrid{});
+}
+
+// Several edits in one launch: CTAs [cta_begin[e], cta_begin[e + 1]) serve edit e exactly as a loss_patch_kernel launch of
+// that many CTAs would.  Every edit writes its own partial array and gradients; grid and patch are launch-wide.
+struct PatchBatchParams {
+    PatchParams edit[kMaxBatchEdits];
+    int cta_begin[kMaxBatchEdits + 1];
+    int n_edits;
+};
+static_assert(sizeof(PatchBatchParams) <= 32764, "kernel parameters are limited to 32764 bytes");
+
+struct EditCtas {
+    int first, n;       // first CTA of the edit, CTAs of the edit
+    __device__ __forceinline__ int index() const { return (int)blockIdx.x - first; }
+    __device__ __forceinline__ int count() const { return n; }
+};
+
+__global__ void __launch_bounds__(kPatchThreads, 1) loss_patch_batch_kernel(const __grid_constant__ PatchBatchParams bp) {
+    int e = 0;
+#pragma unroll
+    for (int i = 1; i < kMaxBatchEdits; ++i)
+        if (i < bp.n_edits && (int)blockIdx.x >= bp.cta_begin[i]) e = i;
+    loss_patch_body(bp.edit[e], EditCtas{bp.cta_begin[e], bp.cta_begin[e + 1] - bp.cta_begin[e]});
+}
+
 // fixed-order reduction of the per-channel terms: loss_out[0] = total, [1+2l] = fg_l, [2+2l] = bg_l
-__global__ void __launch_bounds__(kPatchThreads) loss_patch_finish_kernel(const __grid_constant__ PatchParams p) {
+__device__ __forceinline__ void loss_patch_finish(const PatchParams& p) {
     __shared__ float red[kPatchWarps];
     float total = 0.0f;
     for (int l = 0; l < p.n_layers; ++l) {
@@ -309,9 +342,97 @@ __global__ void __launch_bounds__(kPatchThreads) loss_patch_finish_kernel(const 
     if (threadIdx.x == 0) p.loss_out[0] = total;
 }
 
+__global__ void __launch_bounds__(kPatchThreads) loss_patch_finish_kernel(const __grid_constant__ PatchParams p) {
+    loss_patch_finish(p);
+}
+
+// one CTA per edit, each the single-edit reduction of that edit
+__global__ void __launch_bounds__(kPatchThreads) loss_patch_finish_batch_kernel(const __grid_constant__ PatchBatchParams bp) {
+    loss_patch_finish(bp.edit[blockIdx.x]);
+}
+
 static size_t patch_smem_bytes(int grid) {
     const size_t cells = (size_t)grid * grid;
     return cells * 10 * sizeof(float) + ((cells + 15) / 16) * 16;
+}
+
+// Validates one edit and builds its PatchParams, with its partial array at the start of ws.  No CUDA call.
+static int prepare_patch_edit(const dh_loss_layer* layers_host, int n_layers, int grid, int patch_size, const void* plan, int n_fg,
+                              int n_bg_orig, int n_bg_trans, int n_bg_common, int fg_kind, int bg_kind, float* loss_out, void* ws,
+                              size_t ws_bytes, PatchParams& p) {
+    DH_REQUIRE(layers_host && plan && loss_out && ws);
+    DH_REQUIRE(n_layers >= 1 && n_layers <= kMaxLossLayers && grid >= 1 && grid <= kMaxG);
+    DH_REQUIRE(patch_size >= 1 && patch_size <= kMaxPatch);
+    DH_REQUIRE(n_fg >= 0 && n_bg_orig >= 0 && n_bg_trans >= 0 && n_bg_common >= 0);
+    DH_REQUIRE(fg_kind >= 0 && fg_kind <= 1 && bg_kind >= 0 && bg_kind <= 2);
+    memset(&p, 0, sizeof(p));
+    int total = 0;
+    for (int l = 0; l < n_layers; ++l) {
+        const dh_loss_layer& s = layers_host[l];
+        DH_REQUIRE(s.cur && s.orig && s.channels >= 1 && s.h >= 1 && s.w >= 1 && s.h <= grid && s.w <= grid);
+        DH_REQUIRE(s.h <= kMaxNative && s.w <= kMaxNative);
+        PatchLayer& d = p.lv[l];
+        d.cur = s.cur; d.orig = s.orig; d.grad = s.grad; d.C = s.channels; d.h = s.h; d.w = s.w;
+        d.fgw = s.fg_weight; d.bgw = s.bg_weight; d.chan_begin = total;
+        total += s.channels;
+    }
+    if (ws_bytes < (size_t)total * 2 * sizeof(float)) return DH_ERR_WORKSPACE;
+    p.n_layers = n_layers; p.total_channels = total; p.G = grid; p.patch = patch_size;
+    p.plan = plan; p.plan_cap = n_fg;
+    p.n_fg = n_fg; p.n_bg_orig = n_bg_orig; p.n_bg_trans = n_bg_trans; p.n_bg_common = n_bg_common;
+    p.fg_kind = fg_kind; p.bg_kind = bg_kind;
+    p.partial = static_cast<float*>(ws); p.loss_out = loss_out;
+    return DH_OK;
+}
+
+static int sm_count(int* sms) {
+    int dev = 0;
+    DH_CUDA_CHECK(cudaGetDevice(&dev));
+    DH_CUDA_CHECK(cudaDeviceGetAttribute(sms, cudaDevAttrMultiProcessorCount, dev));
+    return DH_OK;
+}
+
+// one edit: min(channels, SMs) CTAs of loss_patch_kernel, then the one-CTA reduction
+static int launch_patch_edit(const PatchParams& p, void* stream) {
+    int sms = 0;
+    const int rc = sm_count(&sms);
+    if (rc != DH_OK) return rc;
+    const size_t smem = patch_smem_bytes(p.G);
+    DH_CUDA_CHECK(cudaFuncSetAttribute(loss_patch_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    const int ctas = p.total_channels < sms ? p.total_channels : sms;
+    loss_patch_kernel<<<ctas, kPatchThreads, smem, as_stream(stream)>>>(p);
+    DH_LAUNCH_CHECK();
+    loss_patch_finish_kernel<<<1, kPatchThreads, 0, as_stream(stream)>>>(p);
+    DH_LAUNCH_CHECK();
+    return DH_OK;
+}
+
+// several edits of one grid: CTAs in proportion to the edits' channels, at least one per edit, none without a plane, and at
+// most the SM count in all (each CTA holds a whole SM: 512 threads and up to 160 KB of shared memory)
+static int launch_patch_batch(PatchBatchParams& bp, int n_edits, void* stream) {
+    int sms = 0;
+    const int rc = sm_count(&sms);
+    if (rc != DH_OK) return rc;
+    long long channels = 0;
+    for (int e = 0; e < n_edits; ++e) channels += bp.edit[e].total_channels;
+    const long long spare = sms > n_edits ? sms - n_edits : 0;
+    int n_ctas = 0;
+    for (int e = 0; e < n_edits; ++e) {
+        const int c = bp.edit[e].total_channels;
+        int share = 1 + (int)(spare * c / channels);
+        if (share > c) share = c;
+        bp.cta_begin[e] = n_ctas;
+        n_ctas += share;
+    }
+    bp.cta_begin[n_edits] = n_ctas;
+    bp.n_edits = n_edits;
+    const size_t smem = patch_smem_bytes(bp.edit[0].G);
+    DH_CUDA_CHECK(cudaFuncSetAttribute(loss_patch_batch_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    loss_patch_batch_kernel<<<n_ctas, kPatchThreads, smem, as_stream(stream)>>>(bp);
+    DH_LAUNCH_CHECK();
+    loss_patch_finish_batch_kernel<<<n_edits, kPatchThreads, 0, as_stream(stream)>>>(bp);
+    DH_LAUNCH_CHECK();
+    return DH_OK;
 }
 
 }  // namespace dh
@@ -328,41 +449,32 @@ size_t dh_guidance_loss_patch_workspace_bytes(int n_layers, int max_channels) {
 int dh_guidance_loss_patch(const dh_loss_layer* layers_host, int n_layers, int grid, int patch_size, const void* plan, int n_fg,
                            int n_bg_orig, int n_bg_trans, int n_bg_common, int fg_kind, int bg_kind, float* loss_out, void* ws,
                            size_t ws_bytes, void* stream) {
-    DH_REQUIRE(layers_host && plan && loss_out && ws);
-    DH_REQUIRE(n_layers >= 1 && n_layers <= kMaxLossLayers && grid >= 1 && grid <= kMaxG);
-    DH_REQUIRE(patch_size >= 1 && patch_size <= kMaxPatch);
-    DH_REQUIRE(n_fg >= 0 && n_bg_orig >= 0 && n_bg_trans >= 0 && n_bg_common >= 0);
-    DH_REQUIRE(fg_kind >= 0 && fg_kind <= 1 && bg_kind >= 0 && bg_kind <= 2);
     PatchParams p;
-    memset(&p, 0, sizeof(p));
-    int total = 0, max_c = 0;
-    for (int l = 0; l < n_layers; ++l) {
-        const dh_loss_layer& s = layers_host[l];
-        DH_REQUIRE(s.cur && s.orig && s.channels >= 1 && s.h >= 1 && s.w >= 1 && s.h <= grid && s.w <= grid);
-        DH_REQUIRE(s.h <= kMaxNative && s.w <= kMaxNative);
-        PatchLayer& d = p.lv[l];
-        d.cur = s.cur; d.orig = s.orig; d.grad = s.grad; d.C = s.channels; d.h = s.h; d.w = s.w;
-        d.fgw = s.fg_weight; d.bgw = s.bg_weight; d.chan_begin = total;
-        total += s.channels;
-        max_c = s.channels > max_c ? s.channels : max_c;
+    const int rc = prepare_patch_edit(layers_host, n_layers, grid, patch_size, plan, n_fg, n_bg_orig, n_bg_trans, n_bg_common, fg_kind,
+                                      bg_kind, loss_out, ws, ws_bytes, p);
+    return rc != DH_OK ? rc : launch_patch_edit(p, stream);
+}
+
+size_t dh_guidance_loss_patch_batch_workspace_bytes(int n_edits, int n_layers, int max_channels) {
+    if (n_edits < 1 || n_edits > kMaxBatchEdits) return 0;
+    return (size_t)n_edits * dh_guidance_loss_patch_workspace_bytes(n_layers, max_channels);
+}
+
+int dh_guidance_loss_patch_batch(const dh_loss_batch_edit* edits_host, int n_edits, int grid, int patch_size, int fg_kind, int bg_kind,
+                                 void* ws, size_t ws_bytes, void* stream) {
+    DH_REQUIRE(edits_host && ws && n_edits >= 1);
+    if (n_edits > kMaxBatchEdits) return DH_ERR_UNSUPPORTED;
+    PatchBatchParams bp;
+    memset(&bp, 0, sizeof(bp));
+    // edit e owns bytes [e * stride, (e + 1) * stride) of the workspace (a partial array is a multiple of 8 bytes)
+    const size_t stride = ws_bytes / (size_t)n_edits / 8 * 8;
+    for (int e = 0; e < n_edits; ++e) {
+        const dh_loss_batch_edit& E = edits_host[e];
+        const int rc = prepare_patch_edit(E.layers, E.n_layers, grid, patch_size, E.plan, E.n_fg, E.n_bg_orig, E.n_bg_trans, E.n_bg_common,
+                                          fg_kind, bg_kind, E.loss_out, static_cast<char*>(ws) + e * stride, stride, bp.edit[e]);
+        if (rc != DH_OK) return rc;
     }
-    if (ws_bytes < (size_t)total * 2 * sizeof(float)) return DH_ERR_WORKSPACE;
-    p.n_layers = n_layers; p.total_channels = total; p.G = grid; p.patch = patch_size;
-    p.plan = plan; p.plan_cap = n_fg;
-    p.n_fg = n_fg; p.n_bg_orig = n_bg_orig; p.n_bg_trans = n_bg_trans; p.n_bg_common = n_bg_common;
-    p.fg_kind = fg_kind; p.bg_kind = bg_kind;
-    p.partial = static_cast<float*>(ws); p.loss_out = loss_out;
-    int dev = 0, sms = 0;
-    DH_CUDA_CHECK(cudaGetDevice(&dev));
-    DH_CUDA_CHECK(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
-    const size_t smem = patch_smem_bytes(grid);
-    DH_CUDA_CHECK(cudaFuncSetAttribute(loss_patch_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    const int ctas = total < sms ? total : sms;
-    loss_patch_kernel<<<ctas, kPatchThreads, smem, as_stream(stream)>>>(p);
-    DH_LAUNCH_CHECK();
-    loss_patch_finish_kernel<<<1, kPatchThreads, 0, as_stream(stream)>>>(p);
-    DH_LAUNCH_CHECK();
-    return DH_OK;
+    return n_edits == 1 ? launch_patch_edit(bp.edit[0], stream) : launch_patch_batch(bp, n_edits, stream);
 }
 
 }  // extern "C"

@@ -7,6 +7,13 @@ namespace dh {
 constexpr int kMaxLossLayers = 8;
 constexpr int kMaxG = 64;
 constexpr int kMaxNative = 64;
+constexpr int kMaxBatchEdits = 16;       // edits of one batched K4 launch (dh_guidance_loss_batch, dh_guidance_loss_patch_batch)
+
+// The CTAs of a single-edit launch: the whole grid serves the edit (the batched kernels pass the CTA's share of its edit).
+struct WholeGrid {
+    __device__ __forceinline__ unsigned int index() const { return blockIdx.x; }
+    __device__ __forceinline__ unsigned int count() const { return gridDim.x; }
+};
 
 struct PlanHeader {
     int32_t n_pairs, n_fg, n_bg_orig, n_bg_trans, n_bg_common, grid, cap, reserved;

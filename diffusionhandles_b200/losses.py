@@ -292,13 +292,14 @@ def guidance_loss_and_grad(activations: Sequence[torch.Tensor], activations_orig
     return out[0], out[1:], grads
 
 
-MAX_BATCH_EDITS = 16        # edits per dh_guidance_loss_batch launch; larger batches run in chunks of this size
+MAX_BATCH_EDITS = 16        # edits per batched K4 launch; larger batches run in chunks of this size
 
 
-def _batch_runner(plans: Sequence[LossPlan], shapes, bg_kind: int):
+def _batch_runner(plans: Sequence[LossPlan], shapes, bg_kind: int, general: bool):
     """The ctypes edit and layer arrays, the workspace and the resize tables of one chunk of edits, created once per (plans,
-    shapes) and cached on the first plan (the entry keeps the plans alive, so their ids stay unique)."""
-    key = ("batch", tuple(id(p) for p in plans), shapes, bg_kind)
+    shapes, kernel) and cached on the first plan (the entry keeps the plans alive, so their ids stay unique).  ``general``:
+    the chunk goes to the general patch kernel (dh_guidance_loss_patch_batch), which takes no resize tables."""
+    key = ("batch", tuple(id(p) for p in plans), shapes, bg_kind, general)
     runner = plans[0]._runners.get(key)
     if runner is None:
         lib = N.load()
@@ -306,7 +307,7 @@ def _batch_runner(plans: Sequence[LossPlan], shapes, bg_kind: int):
         edits = (N.dh_loss_batch_edit * n)()
         layer_arrays, tabs = [], []
         for e, plan in enumerate(plans):
-            layers, t = _layers(plan, shapes, _FG, bg_kind, False)
+            layers, t = _layers(plan, shapes, _FG, bg_kind, general)
             layer_arrays.append(layers)
             tabs += t
             edits[e].layers = C.cast(layers, C.POINTER(N.dh_loss_layer))
@@ -314,8 +315,9 @@ def _batch_runner(plans: Sequence[LossPlan], shapes, bg_kind: int):
             edits[e].plan = plan.buf.data_ptr()
             edits[e].desc = plan.desc
             edits[e].n_fg, edits[e].n_bg_orig, edits[e].n_bg_trans, edits[e].n_bg_common = plan.n
-        ws_bytes = int(lib.dh_guidance_loss_batch_workspace_bytes(n, L, max(sh[0] for sh in shapes)))
-        # zeroed once: the launch re-arms every edit's queue counters
+        ws_fn = lib.dh_guidance_loss_patch_batch_workspace_bytes if general else lib.dh_guidance_loss_batch_workspace_bytes
+        ws_bytes = int(ws_fn(n, L, max(sh[0] for sh in shapes)))
+        # zeroed once: the patch-1 launch re-arms every edit's queue counters
         runner = (tuple(plans), edits, layer_arrays, torch.zeros(ws_bytes, dtype=torch.uint8, device=plans[0].buf.device), ws_bytes, tabs)
         plans[0]._runners[key] = runner
     return runner
@@ -324,15 +326,16 @@ def _batch_runner(plans: Sequence[LossPlan], shapes, bg_kind: int):
 def guidance_loss_and_grad_batch(activations: Sequence[torch.Tensor], activations_orig: Sequence[torch.Tensor],
                                  processed_correspondences: Sequence, fg_weights: Sequence[float], bg_weights: Sequence[float],
                                  bg_loss_type: str = 'global_avg', activations_size=(64, 64), patch_size: int = 1):
-    """``guidance_loss_and_grad`` for B edits at once: ONE K4 launch per 16 edits (dh_guidance_loss_batch).
+    """``guidance_loss_and_grad`` for B edits at once: ONE K4 launch per 16 edits (dh_guidance_loss_batch, or
+    dh_guidance_loss_patch_batch for the inputs that the single-edit call sends to the general patch kernel: patch_size > 1,
+    map areas that are not a multiple of 4 or below grid/8, 'local_avg' on resized layers).
 
     ``activations[l]`` is (B,C_l,h_l,w_l), what a U-Net run at batch B returns; ``activations_orig[l]`` is (C_l,h_l,w_l), shared
     by every edit (variants of one image), (B,C_l,h_l,w_l), or a sequence of B (C_l,h_l,w_l) tensors - one identity per edit,
     read in place (edits may share a tensor); ``processed_correspondences`` holds B dicts.  The weights are
     the same for every edit.  Returns (totals (B,), parts (B,2L), [grad_l (B,C_l,h_l,w_l)]): row / slice e is bit-identical to
-    what ``guidance_loss_and_grad`` returns for edit e alone.  Inputs that the single-edit call sends to the general patch kernel
-    (patch_size > 1, map areas that are not a multiple of 4, 'local_avg' on resized layers) run one such launch per edit.  A chunk
-    of one edit runs the single-edit kernel (dh_guidance_loss_batch picks it)."""
+    what ``guidance_loss_and_grad`` returns for edit e alone.  A chunk of one edit runs the single-edit kernels (the library picks
+    them)."""
     if bg_loss_type not in ('global_avg', 'local_avg'):
         raise ValueError(f'Unknown background loss type: {bg_loss_type}')
     grid = _grid_of(activations_size)
@@ -358,15 +361,7 @@ def guidance_loss_and_grad_batch(activations: Sequence[torch.Tensor], activation
     plans = [_plan_for(pc, grid, dev) for pc in pcs]
     shapes = tuple(tuple(a.shape[1:]) for a in activations)
     out = torch.empty(B, 1 + 2 * L, dtype=torch.float32, device=dev)
-    if _needs_general(shapes, grid, patch, bg_kind):
-        grads = [torch.empty((B,) + sh, dtype=torch.float32, device=dev) for sh in shapes]
-        for e in range(B):
-            o, g = _launch([a[e] for a in activations], [rows[e] for rows in orig_rows], [True] * L,
-                           fg_weights, bg_weights, plans[e], _FG, bg_kind, patch)
-            out[e] = o
-            for l in range(L):
-                grads[l][e] = g[l]
-        return out[:, 0], out[:, 1:], grads
+    general = _needs_general(shapes, grid, patch, bg_kind)
     lib = N.load()
     curs = [_as_f32(a, dev) for a in activations]
     converted = {}                     # one conversion per distinct tensor (a shared identity is converted once)
@@ -382,7 +377,7 @@ def guidance_loss_and_grad_batch(activations: Sequence[torch.Tensor], activation
     st = N.stream_handle(dev)
     for b0 in range(0, B, MAX_BATCH_EDITS):
         chunk = plans[b0:b0 + MAX_BATCH_EDITS]
-        _, edits, layer_arrays, ws, ws_bytes, _ = _batch_runner(chunk, shapes, bg_kind)
+        _, edits, layer_arrays, ws, ws_bytes, _ = _batch_runner(chunk, shapes, bg_kind, general)
         for j, layers in enumerate(layer_arrays):
             e = b0 + j
             for l in range(L):
@@ -390,7 +385,11 @@ def guidance_loss_and_grad_batch(activations: Sequence[torch.Tensor], activation
                 layers[l].orig = org_p[l][e]
                 layers[l].fg_weight, layers[l].bg_weight = float(fg_weights[l]), float(bg_weights[l])
             edits[j].loss_out = out.data_ptr() + 4 * e * (1 + 2 * L)
-        N.check(lib.dh_guidance_loss_batch(edits, len(chunk), grid, _FG, bg_kind, ws.data_ptr(), ws_bytes, st), "dh_guidance_loss_batch")
+        if general:
+            N.check(lib.dh_guidance_loss_patch_batch(edits, len(chunk), grid, patch, _FG, bg_kind, ws.data_ptr(), ws_bytes, st),
+                    "dh_guidance_loss_patch_batch")
+        else:
+            N.check(lib.dh_guidance_loss_batch(edits, len(chunk), grid, _FG, bg_kind, ws.data_ptr(), ws_bytes, st), "dh_guidance_loss_batch")
     return out[:, 0], out[:, 1:], grads
 
 

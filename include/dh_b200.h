@@ -287,6 +287,17 @@ size_t dh_guidance_loss_patch_workspace_bytes(int n_layers, int max_channels);
 int dh_guidance_loss_patch(const dh_loss_layer* layers_host, int n_layers, int grid, int patch_size, const void* plan,
                            int n_fg, int n_bg_orig, int n_bg_trans, int n_bg_common, int fg_kind, int bg_kind,
                            float* loss_out, void* ws, size_t ws_bytes, void* stream);
+/* Workspace of a patch batch: n_edits times dh_guidance_loss_patch_workspace_bytes (0 outside 1 <= n_edits <= 16). */
+size_t dh_guidance_loss_patch_batch_workspace_bytes(int n_edits, int n_layers, int max_channels);
+/* dh_guidance_loss_patch for each of the n_edits edits of the HOST array edits_host: one main launch and one finish launch for
+ * all of them.  grid, patch_size, fg_kind and bg_kind are the same for every edit (the descriptors' desc and the layers'
+ * resize_tables are unused); every edit's results are bit-identical to a dh_guidance_loss_patch call on that edit alone, and a
+ * batch of one edit runs exactly that call's kernels.  Edit e owns bytes [e s, (e+1) s) of `ws`, s = ws_bytes / n_edits
+ * rounded down to 8, which must hold that edit's partial array.  Every check runs before any CUDA call: each edit is validated as
+ * dh_guidance_loss_patch validates one and is rejected with the same code; DH_ERR_INVALID_ARGUMENT for n_edits < 1 or NULL
+ * arrays, DH_ERR_UNSUPPORTED for n_edits above 16 (callers split larger batches).  No allocation, no synchronisation. */
+int dh_guidance_loss_patch_batch(const dh_loss_batch_edit* edits_host, int n_edits, int grid, int patch_size, int fg_kind,
+                                 int bg_kind, void* ws, size_t ws_bytes, void* stream);
 /* grads *= *scale (device scalar) for up to 8 tensors in one launch (HOST arrays of device pointers and element counts); exits
  * early on the device when *scale == 1. */
 int dh_scale_inplace_many(float* const* data_host, const size_t* n_host, int count, const float* scale, void* stream);
