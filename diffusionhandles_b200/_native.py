@@ -71,6 +71,11 @@ _SIGNATURES = {
     "dh_edit_splat": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, C.POINTER(dh_camera), C.POINTER(dh_rigid), c_void_p,
                               c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,
                               c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_size_t, c_void_p]),
+    "dh_edit_objects_workspace_bytes": (c_size_t, [c_int, c_int, c_int]),
+    "dh_edit_splat_objects": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_int, C.POINTER(dh_camera),
+                                      C.POINTER(dh_rigid), c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,
+                                      c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_size_t,
+                                      c_void_p]),
     "dh_transform_point_cloud_workspace_bytes": (c_size_t, [c_int]),
     "dh_transform_point_cloud": (c_int, [c_void_p, c_void_p, c_int, C.POINTER(dh_rigid), c_void_p, c_void_p, c_void_p, c_void_p,
                                          c_size_t, c_void_p]),

@@ -232,6 +232,63 @@ __global__ void __launch_bounds__(96) fg_centroid_kernel(const float* __restrict
     if (lane == 0) centroid[e * 3 + comp] = __fdiv_rn(s, (float)n);
 }
 
+constexpr int kSeqTileF = 512, kSeqBuf = 4;                      // floats per tile, ring depth
+using SeqRing = float[3][kSeqBuf][kSeqTileF];
+
+// The FADD chain of fg_centroid_kernel as a function of its own (fg_centroid_kernel keeps its inline copy, and with it its exact
+// instruction schedule): the sequential fp32 sum of a[0..n) by warp `comp`, staged in ring[comp], every lane holding the sum.
+__device__ __forceinline__ float seq_sum_warp(const float* __restrict__ a, int n, int comp, int lane, SeqRing& ring) {
+    constexpr int kTileF = kSeqTileF, kBuf = kSeqBuf, kGroup = 8;   // float4 per register group
+    const unsigned full = 0xFFFFFFFFu;
+    float s = 0.0f;
+    const int n_tiles = (reinterpret_cast<uintptr_t>(a) & 15) == 0 ? n / kTileF : 0;
+    auto issue = [&](int t) {
+        if (t < n_tiles) {
+            const float* src = a + (size_t)t * kTileF + lane * 4;
+            float* dst = &ring[comp][t % kBuf][lane * 4];
+#pragma unroll
+            for (int q = 0; q < kTileF / 128; ++q)
+                asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"((uint32_t)__cvta_generic_to_shared(dst + 128 * q)),
+                             "l"(src + 128 * q) : "memory");
+        }
+        asm volatile("cp.async.commit_group;" ::: "memory");       // (empty groups keep the wait count uniform)
+    };
+#pragma unroll
+    for (int t = 0; t < kBuf - 1; ++t) issue(t);
+    for (int t = 0; t < n_tiles; ++t) {
+        issue(t + kBuf - 1);                                        // refills the slot consumed in iteration t - 1
+        asm volatile("cp.async.wait_group %0;" ::"n"(kBuf - 1) : "memory");
+        __syncwarp();
+        const float4* tile = reinterpret_cast<const float4*>(ring[comp][t % kBuf]);
+        float4 cur[kGroup], nxt[kGroup];
+#pragma unroll
+        for (int j = 0; j < kGroup; ++j) cur[j] = tile[j];          // same address in every lane: broadcast
+#pragma unroll
+        for (int g = 0; g < kTileF / 4 / kGroup; ++g) {
+            if (g + 1 < kTileF / 4 / kGroup) {
+#pragma unroll
+                for (int j = 0; j < kGroup; ++j) nxt[j] = tile[(g + 1) * kGroup + j];
+            }
+#pragma unroll
+            for (int j = 0; j < kGroup; ++j) {
+                s = __fadd_rn(s, cur[j].x);
+                s = __fadd_rn(s, cur[j].y);
+                s = __fadd_rn(s, cur[j].z);
+                s = __fadd_rn(s, cur[j].w);
+            }
+#pragma unroll
+            for (int j = 0; j < kGroup; ++j) cur[j] = nxt[j];
+        }
+        __syncwarp();                                               // every lane is done with the slot before it is refilled
+    }
+    for (int base = n_tiles * kTileF; base < n; base += 32) {
+        const float v = base + lane < n ? a[base + lane] : 0.0f;
+        const int cnt = min(32, n - base);
+        for (int j = 0; j < cnt; ++j) s = __fadd_rn(s, __shfl_sync(full, v, j));
+    }
+    return s;
+}
+
 // depth_transform.py:512-531 for one point: Rodrigues about the centroid + translation, fp32 -> fp64 in the
 // reference's operation order (SURVEY.md A.2).
 __device__ __forceinline__ void rigid_point(float px, float py, float pz, float cx, float cy, float cz, const dh_rigid& rg,
@@ -567,6 +624,184 @@ __global__ void __launch_bounds__(256) edit_points_publish_kernel(
     }
 }
 
+// ------------------------------------------------------------------------------------------------
+// Multi-object edits (dh_edit_splat_objects): the foreground is the union of K <= 16 disjoint objects, labels[p] = k + 1 for
+// a pixel of object k.  The compaction of the union also records each foreground point's object; every point then moves about
+// the sequential centroid of its own object with its object's rigid transform.  The z-buffer, masks and winners do not depend on
+// which object a point came from: kernels A, E, F and G run unchanged.
+// ------------------------------------------------------------------------------------------------
+constexpr int kMaxObjects = 16;
+
+struct ObjWs {
+    int32_t* tile_hist;         // [B][ntiles][16]: foreground pixels of each object in each compaction tile
+    float *objX, *objY, *objZ;  // [B][stride]: the points of each object compacted, object k from a 16-byte aligned offset
+    size_t stride;
+};
+
+// B: the union compaction of fg_compact_kernel, plus the object of every foreground point and per-tile object counts.
+__global__ void __launch_bounds__(kTileThreads) fg_compact_objects_kernel(
+    const float* __restrict__ depth, const float* __restrict__ mask, const uint8_t* __restrict__ labels, int P, int W, int ntiles,
+    int K, CamDev cam, const float* __restrict__ xs, const float* __restrict__ ys, const int32_t* __restrict__ tile_counts,
+    int32_t* __restrict__ fg_index, uint8_t* __restrict__ fg_object, float* __restrict__ fgX, float* __restrict__ fgY,
+    float* __restrict__ fgZ, int32_t* __restrict__ n_fg, int32_t* __restrict__ tile_hist) {
+    __shared__ int scan_smem[33];
+    __shared__ int base_smem;
+    __shared__ int hist[kMaxObjects];
+    const int e = blockIdx.y, tile = blockIdx.x;
+    if (threadIdx.x < kMaxObjects) hist[threadIdx.x] = 0;
+    int part = 0;
+    for (int t = threadIdx.x; t < tile; t += blockDim.x) part += tile_counts[e * ntiles + t];
+    int tot;
+    block_exclusive_scan(part, scan_smem, tot);
+    if (threadIdx.x == 0) base_smem = tot;
+    __syncthreads();
+    const int base = base_smem;
+
+    const int p0 = tile * kTile + threadIdx.x * 4;
+    const float* m = mask + (size_t)e * P;
+    bool f[4];
+    int c = 0;
+#pragma unroll
+    for (int i = 0; i < 4; ++i) {
+        f[i] = (p0 + i < P) && (m[p0 + i] != 0.0f);
+        c += f[i];
+    }
+    int total;
+    int pos = base + block_exclusive_scan(c, scan_smem, total);
+    const size_t eo = (size_t)e * P;
+#pragma unroll
+    for (int i = 0; i < 4; ++i) {
+        if (!f[i]) continue;
+        const int p = p0 + i;
+        const int row = p / W, col = p - row * W;
+        float X, Y, Z;
+        unproject(cam, depth[eo + p], xs[col], ys[row], X, Y, Z);
+        // (a foreground pixel whose label is 0 or above K - the caller broke the contract - is taken as object K - 1)
+        const int k = min((int)(uint8_t)(labels[eo + p] - 1u), K - 1);
+        fg_index[eo + pos] = p;
+        fg_object[eo + pos] = (uint8_t)k;
+        fgX[eo + pos] = X; fgY[eo + pos] = Y; fgZ[eo + pos] = Z;
+        atomicAdd(&hist[k], 1);
+        ++pos;
+    }
+    __syncthreads();
+    if (threadIdx.x < kMaxObjects) tile_hist[((size_t)e * ntiles + tile) * kMaxObjects + threadIdx.x] = hist[threadIdx.x];
+    if (tile == ntiles - 1 && threadIdx.x == 0) n_fg[e] = base + total;
+}
+
+// C: the sequential centroid of object k = blockIdx.x of edit e = blockIdx.y.  The block first copies the object's points out
+// of the compacted union (a raster-ordered subsequence, found by a block scan over the object ids), then three warps run the
+// FADD chain of fg_centroid_kernel over that object alone: the chain is as long as the object, not the union.
+__global__ void __launch_bounds__(256) fg_centroid_objects_kernel(const float* __restrict__ fgX, const float* __restrict__ fgY,
+                                                                  const float* __restrict__ fgZ, const uint8_t* __restrict__ fg_object,
+                                                                  const int32_t* __restrict__ n_fg, int P, int ntiles, int K, ObjWs ow,
+                                                                  float* __restrict__ centroid) {
+    __shared__ __align__(16) float ring[3][kSeqBuf][kSeqTileF];
+    __shared__ int counts[8][kMaxObjects];
+    __shared__ int scan_smem[33];
+    const int k = blockIdx.x, e = blockIdx.y;
+    // points per object of this edit: the sums of the tile histograms (64-byte rows)
+    int c[kMaxObjects];
+#pragma unroll
+    for (int j = 0; j < kMaxObjects; ++j) c[j] = 0;
+    for (int t = threadIdx.x; t < ntiles; t += blockDim.x) {
+        const int4* h = reinterpret_cast<const int4*>(ow.tile_hist + ((size_t)e * ntiles + t) * kMaxObjects);
+#pragma unroll
+        for (int q = 0; q < kMaxObjects / 4; ++q) {
+            const int4 v = h[q];
+            c[4 * q] += v.x; c[4 * q + 1] += v.y; c[4 * q + 2] += v.z; c[4 * q + 3] += v.w;
+        }
+    }
+#pragma unroll
+    for (int j = 0; j < kMaxObjects; ++j) {
+        const int s = __reduce_add_sync(0xFFFFFFFFu, c[j]);
+        if (lane_id() == 0) counts[warp_id()][j] = s;
+    }
+    __syncthreads();
+    int n_k = 0, off = 0;                       // object k's count and its 16-byte aligned offset in the object arrays
+    for (int j = 0; j <= k; ++j) {
+        int nj = 0;
+        for (int w = 0; w < 8; ++w) nj += counts[w][j];
+        if (j < k) off += (nj + 3) & ~3;
+        else n_k = nj;
+    }
+    const size_t eo = (size_t)e * P;
+    float* dx = ow.objX + e * ow.stride + off;
+    float* dy = ow.objY + e * ow.stride + off;
+    float* dz = ow.objZ + e * ow.stride + off;
+    const int n = n_fg[e];
+    // stable compaction of the object's points, 4096 union points per step (16 id loads in flight per thread), until all n_k are found
+    constexpr int kPer = 16;
+    for (int base = 0, found = 0; found < n_k && base < n; base += kPer * 256) {
+        const int j0 = base + threadIdx.x * kPer;
+        uint32_t f = 0;
+#pragma unroll
+        for (int i = 0; i < kPer; ++i)
+            if (j0 + i < n && fg_object[eo + j0 + i] == k) f |= 1u << i;
+        int total;
+        int q = found + block_exclusive_scan(__popc(f), scan_smem, total);
+        for (; f; f &= f - 1) {
+            const size_t j = eo + j0 + __ffs(f) - 1;
+            dx[q] = fgX[j]; dy[q] = fgY[j]; dz[q] = fgZ[j];
+            ++q;
+        }
+        found += total;
+    }
+    __syncthreads();                            // the block's global writes are visible to its own warps
+    const int comp = warp_id();
+    if (comp < 3) {
+        const float s = seq_sum_warp(comp == 0 ? dx : comp == 1 ? dy : dz, n_k, comp, lane_id(), ring);
+        if (lane_id() == 0) centroid[((size_t)e * K + k) * 3 + comp] = __fdiv_rn(s, (float)n_k);
+    }
+}
+
+// a generic point of a multi-object edit: a foreground point moves with its own object's centroid and transform
+__device__ __forceinline__ EditPoint edit_point_objects(int e, int slot, int P, int W, int K, const CamDev& cam,
+                                                        const dh_rigid* __restrict__ rigid, const float* __restrict__ xs,
+                                                        const float* __restrict__ ys, const float* __restrict__ bg_depth,
+                                                        const int32_t* __restrict__ n_fg, const uint8_t* __restrict__ fg_object,
+                                                        const float* __restrict__ centroid, const EditWs& ws) {
+    if (slot < n_fg[e]) {
+        EditPoint pt;
+        const size_t eo = (size_t)e * P + slot;
+        const int ek = e * K + fg_object[eo];
+        rigid_point(ws.fgX[eo], ws.fgY[eo], ws.fgZ[eo], centroid[ek * 3 + 0], centroid[ek * 3 + 1], centroid[ek * 3 + 2], rigid[ek],
+                    pt.X, pt.Y, pt.Z);
+        pt.live = true; pt.index = P + slot;
+        return pt;
+    }
+    return edit_point(e, slot, P, W, cam, rigid, xs, ys, bg_depth, n_fg, centroid, ws);     // odd background point, or none
+}
+
+// D of a multi-object edit: edit_points_splat_kernel with the point's object transform
+__global__ void __launch_bounds__(256) edit_points_splat_objects_kernel(
+    const float* __restrict__ bg_depth, int P, int H, int W, int K, CamDev cam, const dh_rigid* __restrict__ rigid,
+    const float* __restrict__ xs, const float* __restrict__ ys, const int32_t* __restrict__ n_fg, const uint8_t* __restrict__ fg_object,
+    const float* __restrict__ centroid, EditWs ws, int32_t* __restrict__ pix, uint64_t* __restrict__ zkey, double* __restrict__ dbg_points,
+    uint64_t* zbuf) {
+    const int e = blockIdx.y;
+    const int n = n_fg[e] + ws.odd_count[e];
+    uint64_t* zb = zbuf + (size_t)e * P;
+    for (int base = blockIdx.x * blockDim.x; base < n; base += gridDim.x * blockDim.x) {
+        const int slot = base + threadIdx.x;
+        const EditPoint pt = edit_point_objects(e, slot, P, W, K, cam, rigid, xs, ys, bg_depth, n_fg, fg_object, centroid, ws);
+        int q = -1;
+        uint64_t key = kEmptyZ;
+        if (pt.live) {
+            int u, v;
+            const bool ok = project(cam, pt.X, pt.Y, pt.Z, H, W, u, v, key);
+            q = ok ? v * W + u : -1;
+            const size_t po = (size_t)e * 2 * P + pt.index;
+            pix[po] = q; zkey[po] = key;
+            if (dbg_points) {
+                double* o = dbg_points + po * 3;
+                o[0] = pt.X; o[1] = pt.Y; o[2] = pt.Z;
+            }
+        }
+        zbuf_atomic_min_warp(zb, q, key);
+    }
+}
+
 __global__ void __launch_bounds__(256) project_points_kernel(const double* __restrict__ points, int N, int H, int W,
                                                              CamDev cam, int32_t* __restrict__ pix, uint64_t* __restrict__ zkey,
                                                              int32_t* __restrict__ uo, int32_t* __restrict__ vo) {
@@ -863,6 +1098,105 @@ int dh_edit_splat(const float* depth, const float* bg_depth, const float* fg_mas
     edit_points_splat_kernel<<<ggrid, 256, 0, st>>>(bg_depth, P, H, W, cam, ew.rigid, xs, ys, n_fg, centroid, ew, pix, zkey, points_out, zbuf);
     DH_LAUNCH_CHECK();
     int gr = (16 * sms + B - 1) / B;            // block-stride over the 32-pixel words of an edit
+    if (gr < 16) gr = 16;
+    if (gr > (H * wpr + 7) / 8) gr = (H * wpr + 7) / 8;
+    edit_resolve_kernel<<<dim3(gr, B), 256, 0, st>>>(zbuf, bg_depth, H, W, wpr, cam_nice ? 1 : 0, winner, depth_map, target_mask,
+                                                                   target_bits, winner_src, ew);
+    DH_LAUNCH_CHECK();
+    edit_points_winner_kernel<<<ggrid, 256, 0, st>>>(pix, zkey, n_fg, P, zbuf, winner, ew);
+    DH_LAUNCH_CHECK();
+    edit_points_publish_kernel<<<ggrid, 256, 0, st>>>(pix, n_fg, fg_index, P, W, wpr, winner, winner_src, target_mask, target_bits, ew,
+                                                      inv_minmax);
+    DH_LAUNCH_CHECK();
+    return DH_OK;
+}
+
+// workspace of a multi-object edit: the dh_edit_splat layout, then [tile_hist int32 B*ntiles*16][rigid B*16]
+// [objX][objY][objZ float B*stride each]; stride holds the union plus 3 alignment floats per object
+struct ObjWsOffsets { size_t tile_hist, rigid, x, y, z, stride, total; };
+static ObjWsOffsets objects_ws_layout(int B, int P, size_t edit_bytes) {
+    ObjWsOffsets L;
+    const int ntiles = (P + kTile - 1) / kTile;
+    L.stride = align_up((size_t)P + 4 * kMaxObjects, 64);
+    size_t o = edit_bytes;
+    L.tile_hist = o; o = align_up(o + sizeof(int32_t) * (size_t)B * ntiles * kMaxObjects, 256);
+    L.rigid = o;     o = align_up(o + sizeof(dh_rigid) * (size_t)B * kMaxObjects, 256);
+    L.x = o;         o = align_up(o + sizeof(float) * (size_t)B * L.stride, 256);
+    L.y = o;         o = align_up(o + sizeof(float) * (size_t)B * L.stride, 256);
+    L.z = o;         o = align_up(o + sizeof(float) * (size_t)B * L.stride, 256);
+    L.total = o;
+    return L;
+}
+
+size_t dh_edit_objects_workspace_bytes(int B, int H, int W) {
+    if (B < 1 || H < 1 || W < 1) return 0;
+    return objects_ws_layout(B, H * W, dh_edit_workspace_bytes(B, H, W)).total;
+}
+
+int dh_edit_splat_objects(const float* depth, const float* bg_depth, const float* fg_mask, const uint8_t* labels, int B, int K, int H,
+                          int W, const dh_camera* cam_host, const dh_rigid* rigid_host, const float* xs, const float* ys, int32_t* pix,
+                          uint64_t* zkey, int32_t* fg_index, uint8_t* fg_object, int32_t* n_fg, float* centroid, double* points_out,
+                          uint64_t* zbuf, uint32_t* winner, float* depth_map, uint8_t* target_mask, uint32_t* target_bits,
+                          int32_t* winner_src, float* inv_minmax, void* ws, size_t ws_bytes, void* stream) {
+    DH_REQUIRE(depth && bg_depth && fg_mask && labels && cam_host && rigid_host && xs && ys && pix && zkey && fg_index && fg_object &&
+               n_fg && centroid && ws);
+    DH_REQUIRE(zbuf && winner && depth_map && target_bits);
+    DH_REQUIRE(B >= 1 && H >= 2 && W >= 2 && K >= 1 && K <= kMaxObjects);
+    DH_REQUIRE((long long)H * W <= (1ll << 29));
+    const int P = H * W;
+    size_t oc, orr, ox, oy, oz;
+    const size_t k1 = k1_ws_layout(B, P, &oc, &orr, &ox, &oy, &oz);
+    const EditWsOffsets L = edit_ws_layout(B, P, k1);
+    const ObjWsOffsets O = objects_ws_layout(B, P, L.total);
+    if (ws_bytes < O.total) return DH_ERR_WORKSPACE;
+    char* w = static_cast<char*>(ws);
+    EditWs ew;
+    ew.tile_counts = reinterpret_cast<int32_t*>(w + oc);
+    ew.rigid = reinterpret_cast<dh_rigid*>(w + O.rigid);          // [B][K]
+    ew.fgX = reinterpret_cast<float*>(w + ox);
+    ew.fgY = reinterpret_cast<float*>(w + oy);
+    ew.fgZ = reinterpret_cast<float*>(w + oz);
+    ew.odd_list = reinterpret_cast<int32_t*>(w + L.odd_list);
+    ew.odd_count = reinterpret_cast<int32_t*>(w + L.odd_count);
+    ew.minmax_keys = reinterpret_cast<uint32_t*>(w + L.minmax);
+    ObjWs ow;
+    ow.tile_hist = reinterpret_cast<int32_t*>(w + O.tile_hist);
+    ow.objX = reinterpret_cast<float*>(w + O.x);
+    ow.objY = reinterpret_cast<float*>(w + O.y);
+    ow.objZ = reinterpret_cast<float*>(w + O.z);
+    ow.stride = O.stride;
+    cudaStream_t st = as_stream(stream);
+    const CamDev cam = make_cam(cam_host);
+    // the camera / image class of dh_edit_splat in which a background point provably keeps its pixel
+    const bool cam_nice = cam.diag && H == W && cam.k[8] == 1.0f && cam.kinv[8] == 1.0f && cam.k[0] > 0.0f && cam.k[4] > 0.0f &&
+                          fabsf(cam.k[0] * cam.kinv[0] - 1.0f) < 1e-5f && fabsf(cam.k[4] * cam.kinv[4] - 1.0f) < 1e-5f && H <= 16384;
+    const int ntiles = (P + kTile - 1) / kTile;
+    const int wpr = (W + 31) / 32;
+    DH_CUDA_CHECK(cudaMemcpyAsync(ew.rigid, rigid_host, sizeof(dh_rigid) * (size_t)B * K, cudaMemcpyHostToDevice, st));
+    DH_CUDA_CHECK(cudaMemsetAsync(ew.odd_count, 0, sizeof(int32_t) * (size_t)B, st));
+    dim3 tgrid(ntiles, B);
+    edit_prepare_kernel<<<tgrid, kTileThreads, 0, st>>>(fg_mask, bg_depth, P, W, H, ntiles, cam_nice ? 1 : 0, cam, xs, ys, ew.tile_counts,
+                                                        zbuf, ew, points_out ? pix : nullptr, points_out ? zkey : nullptr, points_out);
+    DH_LAUNCH_CHECK();
+    fg_compact_objects_kernel<<<tgrid, kTileThreads, 0, st>>>(depth, fg_mask, labels, P, W, ntiles, K, cam, xs, ys, ew.tile_counts, fg_index,
+                                                              fg_object, ew.fgX, ew.fgY, ew.fgZ, n_fg, ow.tile_hist);
+    DH_LAUNCH_CHECK();
+    fg_centroid_objects_kernel<<<dim3(K, B), 256, 0, st>>>(ew.fgX, ew.fgY, ew.fgZ, fg_object, n_fg, P, ntiles, K, ow, centroid);
+    DH_LAUNCH_CHECK();
+    // the grids of dh_edit_splat
+    int sms = 148;
+    {
+        int dev = 0;
+        if (cudaGetDevice(&dev) == cudaSuccess) cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+    }
+    int gx = (8 * sms + B - 1) / B;
+    if (gx < 8) gx = 8;
+    if (gx > (2 * P + 255) / 256) gx = (2 * P + 255) / 256;
+    dim3 ggrid(gx, B);
+    edit_points_splat_objects_kernel<<<ggrid, 256, 0, st>>>(bg_depth, P, H, W, K, cam, ew.rigid, xs, ys, n_fg, fg_object, centroid, ew, pix,
+                                                           zkey, points_out, zbuf);
+    DH_LAUNCH_CHECK();
+    int gr = (16 * sms + B - 1) / B;
     if (gr < 16) gr = 16;
     if (gr > (H * wpr + 7) / 8) gr = (H * wpr + 7) / 8;
     edit_resolve_kernel<<<dim3(gr, B), 256, 0, st>>>(zbuf, bg_depth, H, W, wpr, cam_nice ? 1 : 0, winner, depth_map, target_mask,

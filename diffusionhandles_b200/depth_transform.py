@@ -401,6 +401,93 @@ def transform_depth_pc_batch(depth: torch.Tensor, bg_depth: torch.Tensor, fg_mas
                                      return_device_result)
 
 
+def _object_masks(fg_masks) -> torch.Tensor:
+    """K object masks as one (K,H,W) tensor: a (K,1,H,W) tensor, or a sequence of K (1,1,H,W) tensors."""
+    if isinstance(fg_masks, torch.Tensor):
+        if fg_masks.dim() != 4 or fg_masks.shape[1] != 1 or fg_masks.shape[0] < 1:
+            raise ValueError(f"fg_masks must be (K,1,H,W) with at least one object, got {tuple(fg_masks.shape)}")
+        return fg_masks[:, 0]
+    masks = list(fg_masks)
+    if not masks:
+        raise ValueError("fg_masks must hold at least one object mask")
+    if len({tuple(t.shape) for t in masks}) != 1 or masks[0].dim() != 4 or tuple(masks[0].shape[:2]) != (1, 1):
+        raise ValueError(f"the object masks must all be (1,1,H,W) of one size, got {[tuple(t.shape) for t in masks]}")
+    return torch.cat(masks)[:, 0]
+
+
+def _object_transforms(K: int, rot_angles, rot_axes, translations):
+    """B edits of K objects: ``rot_angles[b][k]`` etc. move object k in edit b.  Returns B."""
+    B = _edit_count(rot_angles, rot_axes, translations)
+    for b in range(B):
+        n = (len(rot_angles[b]), len(rot_axes[b]), len(translations[b]))
+        if n != (K, K, K):
+            raise ValueError(f"edit {b} must have one transform per object ({K}), got {n[0]} angles, {n[1]} axes, {n[2]} translations")
+    return B
+
+
+MAX_OBJECTS = 16
+
+
+def transform_depth_pc_objects_batch(depth: torch.Tensor, bg_depth: torch.Tensor, fg_masks, intrinsics: torch.Tensor, rot_angles,
+                                     rot_axes, translations, use_input_depth_normalization=False, return_device_result: bool = False):
+    """B edits of one scene whose foreground is K disjoint objects, each object with its own rigid transform, as ONE
+    ``EditEngine`` batch (``dh_edit_splat_objects``).
+
+    ``fg_masks``: K masks of the scene, a (K,1,H,W) tensor or a sequence of K (1,1,H,W) tensors (non-zero = in the object,
+    1 <= K <= 16); they must not overlap, and their union is the foreground.  ``rot_angles`` / ``rot_axes`` / ``translations``
+    are (B,K) nested sequences: entry [b][k] moves object k in edit b (``None`` takes the single call's default).  Every object
+    rotates about the sequential centroid of its own pixels; the z-buffer sees all moved objects together, so they occlude one
+    another (an exact z tie goes to the lower source raster index).  An object without pixels is allowed and its transform is
+    ignored.  With K = 1 every result equals ``transform_depth_pc_batch`` bit for bit.  Returns what ``transform_depth_pc_batch``
+    returns: ``(disparities (B,1,S,S) fp32, [correspondences (n_b,4) int64 CPU] * B)``, plus the ``EditResult`` (None for an
+    empty union) with ``return_device_result=True``."""
+    masks = _object_masks(fg_masks)
+    K = masks.shape[0]
+    if K > MAX_OBJECTS:
+        raise ValueError(f"at most {MAX_OBJECTS} objects per edit are supported, got {K}")
+    B = _object_transforms(K, rot_angles, rot_axes, translations)
+    H, W = masks.shape[-2:]
+    if depth.numel() != H * W or bg_depth.numel() != H * W:
+        raise ValueError(f"depth and bg_depth must be one {H} x {W} image like the masks, got {tuple(depth.shape)} and "
+                         f"{tuple(bg_depth.shape)}")
+    inside = masks != 0
+    count = inside.sum(0)
+    overlap, present = torch.stack([(count > 1).any(), (count > 0).any()]).tolist()     # the one synchronisation
+    if overlap:
+        raise ValueError("the object masks overlap: every pixel may belong to one object at most")
+    if not present:
+        disparity, corr = _empty_mask_result(depth.reshape(1, 1, H, W), use_input_depth_normalization)
+        out = disparity.expand(B, 1, H, W).clone(), [corr.clone() for _ in range(B)]
+        return (*out, None) if return_device_result else out
+    if H != W:
+        raise RuntimeError(f"the 'pc' depth transform needs a square mask, got {H} x {W}")
+    _require_cuda(depth, "depth")
+    dev, f32 = depth.device, torch.float32
+    ids = torch.arange(1, K + 1, dtype=torch.uint8, device=inside.device).view(K, 1, 1)
+    labels = (inside.to(torch.uint8) * ids).amax(0)                    # k + 1 on object k (the masks are disjoint)
+    planes = [t.reshape(1, H, W).to(device=dev, dtype=f32) for t in (depth, bg_depth)] + [(count > 0).to(device=dev, dtype=f32)[None],
+                                                                                           labels.to(dev)[None]]
+    d, bg, m, lab = (t.expand(B, H, W).contiguous() for t in planes)
+    rigids = [make_rigid(0.0 if rot_angles[b][k] is None else rot_angles[b][k],
+                         torch.tensor([0.0, 1.0, 0.0]) if rot_axes[b][k] is None else rot_axes[b][k],
+                         torch.zeros(3) if translations[b][k] is None else translations[b][k]) for b in range(B) for k in range(K)]
+    res = get_engine(dev, B, H, W).run_objects(d, bg, m, lab, K, intrinsics, rigids,
+                                               use_input_depth_normalization=use_input_depth_normalization, poisson=True)
+    rows = [res.correspondences(e).cpu() for e in range(B)]
+    out = res.disparity[:, None].clone(), rows
+    return (*out, res) if return_device_result else out
+
+
+def transform_depth_pc_objects(depth: torch.Tensor, bg_depth: torch.Tensor, fg_masks, intrinsics: torch.Tensor, rot_angles, rot_axes,
+                               translations, use_input_depth_normalization=False, return_device_result: bool = False):
+    """One 'pc' edit of K disjoint objects of a square scene, object k moved by (``rot_angles[k]``, ``rot_axes[k]``,
+    ``translations[k]``): ``transform_depth_pc_objects_batch`` with one edit.  Returns ``(edited disparity (1,1,S,S) fp32,
+    correspondences (N,4) int64 CPU)`` like ``transform_depth_pc`` (plus the ``EditResult`` with ``return_device_result=True``)."""
+    disparity, corrs, res = transform_depth_pc_objects_batch(depth, bg_depth, fg_masks, intrinsics, [rot_angles], [rot_axes],
+                                                             [translations], use_input_depth_normalization, return_device_result=True)
+    return (disparity, corrs[0], res) if return_device_result else (disparity, corrs[0])
+
+
 def transform_depth_mesh(depth: torch.Tensor, bg_depth: torch.Tensor, fg_mask: torch.Tensor, intrinsics: torch.Tensor,
                          rot_angle: float = None, rot_axis: torch.Tensor = None, translation: torch.Tensor = None,
                          use_input_depth_normalization=False):

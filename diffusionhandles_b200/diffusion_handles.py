@@ -11,7 +11,8 @@ from types import SimpleNamespace
 
 import torch
 
-from .depth_transform import (_as_scene, _scene_planes, normalize_depth, transform_depth, transform_depth_mesh_scenes, transform_depth_pc_scenes)
+from .depth_transform import (_as_scene, _scene_planes, normalize_depth, transform_depth, transform_depth_mesh_scenes, transform_depth_pc_objects,
+                              transform_depth_pc_scenes)
 from .guided_stable_diffuser import GuidedStableDiffuser
 
 DEFAULT_CONF = SimpleNamespace(   # diffhandles/config/default.yaml
@@ -60,7 +61,8 @@ class DiffusionHandles:
         """diffusion_handles.py:88-110: background depth = input depth with the (15 px dilated) foreground hole filled by
         a Poisson problem driven by the Laplacian of ``bg_depth``.  Entirely on the device: the dilation is one pass of the
         bit-packed morphology kernel with the 31 x 31 diamond that 15 iterations of SciPy's cross element amount to.  Runs as
-        ``set_foreground_scenes`` with one scene."""
+        ``set_foreground_scenes`` with one scene.  For a multi-object edit (``transform_foreground_objects``) pass the union of
+        the object masks: the background is filled under every object at once."""
         H, W = depth.shape[-2:]
         return self.set_foreground_scenes(_as_scene(depth, H, W), _as_scene(fg_mask, H, W), _as_scene(bg_depth, H, W))
 
@@ -183,3 +185,34 @@ class DiffusionHandles:
             images = guided(latents=latents, depth=disparities, uncond_embeddings=uncond, prompt=prompt, activations_orig=acts,
                             correspondences=correspondences, fg_weight=fg_weight, bg_weight=bg_weight)
         return images, disparities
+
+    def edit_geometry_objects(self, depth: torch.Tensor, fg_masks, bg_depth: torch.Tensor, rot_angles, rot_axes, translations,
+                              use_input_depth_normalization=False):
+        """The geometry of one edit that moves K disjoint objects of the image, each by its own transform
+        (``transform_depth_pc_objects``; ``fg_masks`` (K,1,H,W) or K (1,1,H,W) masks, ``rot_angles`` etc. of length K).  Returns
+        (edited disparity (1,1,H,W), correspondences (N,4) int64).  'pc' mode only."""
+        if self.conf.depth_transform_mode != "pc":
+            raise NotImplementedError(f"multi-object edits run in 'pc' mode only, not '{self.conf.depth_transform_mode}'")
+        with torch.no_grad():
+            return transform_depth_pc_objects(depth, bg_depth, fg_masks, self.diffuser.get_depth_intrinsics(device=depth.device),
+                                              rot_angles, rot_axes, translations, use_input_depth_normalization)
+
+    def transform_foreground_objects(self, depth: torch.Tensor, prompt: str, fg_masks, bg_depth: torch.Tensor, null_text_emb: torch.Tensor,
+                                     init_noise: torch.Tensor, activations: list, rot_angles, rot_axes, translations,
+                                     fg_weight: float = None, bg_weight: float = None, use_input_depth_normalization=False):
+        """``transform_foreground`` for K objects moved at once: the geometry of ``edit_geometry_objects``, then ONE guided
+        denoising pass of the injected diffuser over the joint correspondences (the losses see one list, as for a single
+        object).  ``bg_depth`` is ``set_foreground`` of the union of the masks.  Returns (edited_img, edited_disparity) plus the
+        saved denoising steps when the configuration asks for them.  'pc' mode only."""
+        guided = self._need(self.diffuser, "guided_inference")
+        disparity, correspondences = self.edit_geometry_objects(depth, fg_masks, bg_depth, rot_angles, rot_axes, translations,
+                                                                use_input_depth_normalization)
+        keep_steps = bool(self.conf.guided_diffuser.save_denoising_steps)
+        with torch.no_grad():
+            out = guided(latents=init_noise, depth=disparity, uncond_embeddings=null_text_emb, prompt=prompt,
+                         activations_orig=activations, correspondences=correspondences, fg_weight=fg_weight,
+                         bg_weight=bg_weight, save_denoising_steps=keep_steps)
+        if keep_steps:
+            image, steps = out
+            return image, disparity, steps
+        return out, disparity

@@ -15,6 +15,8 @@ import torch
 
 from . import _native as N
 
+MAX_OBJECTS = 16      # objects per multi-object edit (dh_edit_splat_objects)
+
 
 def ellipse_rows(k: int) -> List[int]:
     """Rows of ``cv2.getStructuringElement(cv2.MORPH_ELLIPSE, (k, k))`` as bit masks (bit j = column j).
@@ -82,7 +84,7 @@ class EditResult:
     W: int
     n_fg: torch.Tensor            # (B,) int32
     n_corr: torch.Tensor          # (B,) int32
-    centroid: torch.Tensor        # (B,3) fp32
+    centroid: torch.Tensor        # (B,3) fp32; (B,K,3) for a multi-object edit
     pix: torch.Tensor             # (B,2P) int32
     zkey: torch.Tensor            # (B,2P) int64 view of the uint64 keys
     fg_index: torch.Tensor        # (B,P) int32
@@ -103,6 +105,7 @@ class EditResult:
 
     n_corr_host: Optional[np.ndarray] = None
     n_fg_host: Optional[np.ndarray] = None
+    object_id: Optional[torch.Tensor] = None  # (B,P) uint8: object of foreground point j (multi-object edits only)
 
 
 class EditEngine:
@@ -154,6 +157,7 @@ class EditEngine:
         # the transforms are uploaded from this (pageable, engine-owned) array: it outlives the call, so a CUDA graph that captured
         # the launch chain re-reads the transforms stored here at every replay
         self._rigids = (N.dh_rigid * B)()
+        self.obj_ws = None                # scratch of multi-object edits (run_objects)
         self.xs, self.ys = pixel_grid(H, W, dev)
         S = max(H, W)
         # depth_transform.py:311-313: MORPH_ELLIPSE elements of size img_res//250 (open) and img_res//50 (close)
@@ -184,6 +188,49 @@ class EditEngine:
             N.ptr(self.n_fg), N.ptr(self.centroid), N.ptr(self.points) if self.points is not None else None,
             N.ptr(self.zbuf), N.ptr(self.winner), N.ptr(self.depth_map), N.ptr(self.target_mask), N.ptr(self.target_bits),
             N.ptr(self.winner_src), N.ptr(self.inv_minmax), N.ptr(self.ws), self.ws_bytes, st), "dh_edit_splat")
+        return self._finish(depth, self.centroid, None, use_input_depth_normalization, poisson, sync_counts)
+
+    def run_objects(self, depth: torch.Tensor, bg_depth: torch.Tensor, fg_mask: torch.Tensor, labels: torch.Tensor, K: int,
+                    intrinsics: torch.Tensor, rigids: Sequence[N.dh_rigid], use_input_depth_normalization: bool = False,
+                    poisson: bool = True, sync_counts: bool = True) -> EditResult:
+        """``run`` for edits of K disjoint objects (``dh_edit_splat_objects``).  fg_mask (B,H,W) fp32 is the union of the objects,
+        labels (B,H,W) uint8 holds k + 1 on the pixels of object k (0 elsewhere), rigids B*K host structs, edit-major.  The
+        result's ``centroid`` is (B,K,3) and ``object_id`` (B,P) uint8 gives the object of each foreground point."""
+        lib, B, H, W, P = self.lib, self.B, self.H, self.W, self.P
+        if not 1 <= K <= MAX_OBJECTS:
+            raise ValueError(f"between 1 and {MAX_OBJECTS} objects per edit are supported, got {K}")
+        if len(rigids) != B * K:
+            raise ValueError(f"expected {B * K} rigid transforms ({B} edits of {K} objects), got {len(rigids)}")
+        for name, t in (("depth", depth), ("bg_depth", bg_depth), ("fg_mask", fg_mask), ("labels", labels)):
+            if tuple(t.shape) != (B, H, W):
+                raise ValueError(f"{name} must have shape {(B, H, W)}, got {tuple(t.shape)}")
+        if self.obj_ws is None:           # allocated on first use: the single-object path never needs it
+            self.obj_ws_bytes = int(lib.dh_edit_objects_workspace_bytes(B, H, W))
+            self.obj_ws = torch.empty(self.obj_ws_bytes, dtype=torch.uint8, device=self.device)
+            self.object_id = torch.empty((B, P), dtype=torch.uint8, device=self.device)
+            self.obj_centroid = torch.empty((B * MAX_OBJECTS * 3,), dtype=torch.float32, device=self.device)
+            self._obj_rigids = (N.dh_rigid * (B * MAX_OBJECTS))()
+        st = N.stream_handle(self.device)
+        cam = N.make_camera(intrinsics)
+        rg = self._obj_rigids
+        for i, r in enumerate(rigids):
+            rg[i] = r
+        f32 = torch.float32
+        N.check(lib.dh_edit_splat_objects(
+            N.ptr(depth, f32, "depth"), N.ptr(bg_depth, f32, "bg_depth"), N.ptr(fg_mask, f32, "fg_mask"),
+            N.ptr(labels, torch.uint8, "labels"), B, K, H, W, C.byref(cam), rg, N.ptr(self.xs), N.ptr(self.ys), N.ptr(self.pix),
+            N.ptr(self.zkey), N.ptr(self.fg_index), N.ptr(self.object_id), N.ptr(self.n_fg), N.ptr(self.obj_centroid),
+            N.ptr(self.points) if self.points is not None else None, N.ptr(self.zbuf), N.ptr(self.winner), N.ptr(self.depth_map),
+            N.ptr(self.target_mask), N.ptr(self.target_bits), N.ptr(self.winner_src), N.ptr(self.inv_minmax), N.ptr(self.obj_ws),
+            self.obj_ws_bytes, st), "dh_edit_splat_objects")
+        centroid = self.obj_centroid[: B * K * 3].view(B, K, 3)
+        return self._finish(depth, centroid, self.object_id, use_input_depth_normalization, poisson, sync_counts)
+
+    def _finish(self, depth: torch.Tensor, centroid: torch.Tensor, object_id: Optional[torch.Tensor],
+                use_input_depth_normalization: bool, poisson: bool, sync_counts: bool) -> EditResult:
+        """Everything after the splat: mask cleaning, correspondences, disparity, hole fill, and the count read-back."""
+        lib, B, H, W, P = self.lib, self.B, self.H, self.W, self.P
+        st = N.stream_handle(self.device)
         N.check(lib.dh_mask_clean(N.ptr(self.target_bits), N.ptr(self.cleaned_bits), N.ptr(self.tmp_bits), B, H, W,
                                   self.close_rows, self.close_k, self.open_rows, self.open_k, st), "dh_mask_clean")
         N.check(lib.dh_correspondences(N.ptr(self.pix), N.ptr(self.winner), N.ptr(self.fg_index), N.ptr(self.n_fg),
@@ -200,11 +247,11 @@ class EditEngine:
                                         N.ptr(self.disparity), 0, self.poisson_rel_tol, N.ptr(self.poisson_iters),
                                         N.ptr(self.poisson_ws), self.poisson_ws_bytes, st), "dh_poisson_fill")
             disparity = self.disparity
-        res = EditResult(B=B, H=H, W=W, n_fg=self.n_fg, n_corr=self.n_corr, centroid=self.centroid, pix=self.pix,
+        res = EditResult(B=B, H=H, W=W, n_fg=self.n_fg, n_corr=self.n_corr, centroid=centroid, pix=self.pix,
                          zkey=self.zkey, fg_index=self.fg_index, winner=self.winner, winner_src=self.winner_src,
                          depth_map=self.depth_map, target_mask=self.target_mask, target_bits=self.target_bits,
                          cleaned_bits=self.cleaned_bits, corr=self.corr, disparity_raw=self.disparity_raw,
-                         disparity=disparity, points=self.points)
+                         disparity=disparity, points=self.points, object_id=object_id)
         if sync_counts:
             self.n_pinned[0].copy_(self.n_corr, non_blocking=True)
             self.n_pinned[1].copy_(self.n_fg, non_blocking=True)

@@ -126,6 +126,21 @@ int dh_edit_splat(const float* depth, const float* bg_depth, const float* fg_mas
                   uint64_t* zbuf, uint32_t* winner, float* depth_map, uint8_t* target_mask, uint32_t* target_bits,
                   int32_t* winner_src, float* inv_minmax, void* ws, size_t ws_bytes, void* stream);
 
+/* ---- multi-object edits: dh_edit_splat with K disjoint foreground objects, each with its own rigid transform -------------
+ * labels uint8[B][P]: 0 = background, k + 1 = object k (1 <= K <= 16); it must be non-zero exactly where fg_mask is, which
+ * stays the union of the objects.  The points are those of dh_edit_splat over the union (foreground point j = the j-th union
+ * pixel in raster order); point j belongs to the object of its pixel, fg_object uint8[B][P] records it (0..K-1), and it is
+ * rotated about the fp32 sequential centroid of ITS object's points (raster order) and moved by its object's transform.
+ * rigid_host: B*K structs on the host, edit-major (rigid_host[b*K + k]), uploaded with one copy; centroid float[B][K][3]
+ * (NaN for an object without pixels, whose transform is then unused).  Everything else as dh_edit_splat; with K = 1 the
+ * outputs are those of dh_edit_splat bit for bit.  ws: dh_edit_objects_workspace_bytes(B, H, W) (any K). */
+size_t dh_edit_objects_workspace_bytes(int B, int H, int W);
+int dh_edit_splat_objects(const float* depth, const float* bg_depth, const float* fg_mask, const uint8_t* labels, int B, int K,
+                          int H, int W, const dh_camera* cam_host, const dh_rigid* rigid_host, const float* xs, const float* ys,
+                          int32_t* pix, uint64_t* zkey, int32_t* fg_index, uint8_t* fg_object, int32_t* n_fg, float* centroid,
+                          double* points_out, uint64_t* zbuf, uint32_t* winner, float* depth_map, uint8_t* target_mask,
+                          uint32_t* target_bits, int32_t* winner_src, float* inv_minmax, void* ws, size_t ws_bytes, void* stream);
+
 /* ---- K2, row 5: deterministic z-buffer splat, depth_transform.py:689-712 ---------------------------
  * winner[q] = argmin over {i : pix_i = q} of (z_i, i).  Two 64/32-bit atomicMin passes (z bits, then
  * point index among the points that tie on z) - exact for fp64 depths.
