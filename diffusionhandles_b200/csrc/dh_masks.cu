@@ -257,7 +257,7 @@ __global__ void __launch_bounds__(256) dense_maps_scatter_kernel(const int64_t* 
                                                                  int corr_stride_rows, const __grid_constant__ MapLevels lv,
                                                                  int32_t* __restrict__ maps) {
     const int e = blockIdx.y;
-    const int n_e = n_corr[e];
+    const int n_e = min(n_corr[e], corr_stride_rows);     // a count above the capacity would read the next edit's rows
     for (int n = blockIdx.x * blockDim.x + threadIdx.x; n < n_e; n += gridDim.x * blockDim.x) {
         const longlong4 v = *reinterpret_cast<const longlong4*>(corr + ((size_t)e * corr_stride_rows + n) * 4);
         // rows with a coordinate outside the image (never produced by dh_correspondences; a caller's own list might) are ignored

@@ -145,15 +145,17 @@ __global__ void __launch_bounds__(kWarpThreads) warp_dense_tma_kernel(const __gr
                 v[k].z = off[k][2] >= 0 ? sm[off[k][2]] : 0.0f;
                 v[k].w = off[k][3] >= 0 ? sm[off[k][3]] : 0.0f;
             }
-            // all reads of this stage are done (values are in registers): hand it back to the producer
-            __syncwarp();
-            if ((t & 31) == 0) mbar_arrive(empty + stage);
             float* o = dst + (size_t)c * kStageFloats;
 #pragma unroll
             for (int k = 0; k < kSlotsPerThread; ++k) {
                 const int el = 4 * (t + kConsumerThreads * k);
                 if (el < floats) st_stream_f4(o + el, v[k]);
             }
+            // hand the stage back to the producer only after the stores: a store cannot issue before the shared loads
+            // it reads have returned, while the mbarrier arrive does not wait for loads still in flight - arriving
+            // right after the loads let the next TMA copy overwrite the stage under a few late loads
+            __syncwarp();
+            if ((t & 31) == 0) mbar_arrive(empty + stage);
             if (++stage == kStages) { stage = 0; phase ^= 1; }
         }
     }
@@ -162,14 +164,17 @@ __global__ void __launch_bounds__(kWarpThreads) warp_dense_tma_kernel(const __gr
 // ---- generic gather: out[c][i] = idx[i] >= 0 ? in[c][idx[i]] : 0 ------------------------------------
 constexpr int kGenChannels = 8;
 
+// out_aligned: `out` is 16-byte aligned.  Only then (and with n % 4 == 0) is every row group a float4 slot; a caller's
+// view at an odd float offset takes the scalar stores.
 __global__ void __launch_bounds__(256) gather_generic_kernel(const float* __restrict__ in, int C, int hw_in,
-                                                             const int32_t* __restrict__ idx, int n, float* __restrict__ out) {
+                                                             const int32_t* __restrict__ idx, int n, float* __restrict__ out,
+                                                             int out_aligned) {
     const int g = blockIdx.x * blockDim.x + threadIdx.x;       // group of 4 consecutive outputs
     const int i0 = g * 4;
     if (i0 >= n) return;
     const int c0 = blockIdx.y * kGenChannels;
     const int c1 = min(C, c0 + kGenChannels);
-    const bool vec = (i0 + 3 < n) && ((n & 3) == 0);
+    const bool vec = out_aligned && (i0 + 3 < n) && ((n & 3) == 0);
     int id[4];
 #pragma unroll
     for (int j = 0; j < 4; ++j) id[j] = (i0 + j < n) ? idx[i0 + j] : -1;
@@ -236,7 +241,8 @@ int dh_warp_gather_list(const float* in, int C, int hw, const int32_t* idx, int 
     DH_REQUIRE(in && out && C >= 1 && hw >= 1 && n >= 0 && (idx || n == 0));
     if (n == 0) return DH_OK;
     dim3 grid(((n + 3) / 4 + 255) / 256, (C + kGenChannels - 1) / kGenChannels);
-    gather_generic_kernel<<<grid, 256, 0, as_stream(stream)>>>(in, C, hw, idx, n, out);
+    const int out_aligned = (reinterpret_cast<uintptr_t>(out) & 15) == 0;
+    gather_generic_kernel<<<grid, 256, 0, as_stream(stream)>>>(in, C, hw, idx, n, out, out_aligned);
     DH_LAUNCH_CHECK();
     return DH_OK;
 }
@@ -253,12 +259,16 @@ int dh_warp_gather_dense(const dh_warp_level* levels_host, int n_levels, int B, 
     int seg_chunks_cfg = eb ? atoi(eb) : kSegChunksDefault;
     if (ctas_per_sm < 1 || ctas_per_sm > 8) ctas_per_sm = kCtasPerSmDefault;
     if (seg_chunks_cfg < 1) seg_chunks_cfg = kSegChunksDefault;
+    // every level is checked before the first launch: a rejected call writes no output
+    for (int i = 0; i < n_levels; ++i) {
+        const dh_warp_level& l = levels_host[i];
+        DH_REQUIRE(l.in && l.out && l.src_map && l.channels >= 1 && l.hw >= 1 && l.in != l.out);
+    }
     WarpParams p;
     memset(&p, 0, sizeof(p));
     int nfast = 0, seg = 0;
     for (int i = 0; i < n_levels; ++i) {
         const dh_warp_level& l = levels_host[i];
-        DH_REQUIRE(l.in && l.out && l.src_map && l.channels >= 1 && l.hw >= 1 && l.in != l.out);
         if (!fast_path_ok(l)) {
             // generic path, one launch per edit
             for (int e = 0; e < B; ++e) {

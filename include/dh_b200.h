@@ -205,7 +205,9 @@ int dh_process_correspondences(const int64_t* corr, int n_corr, int img_res, int
  * a splat winner; else -1.
  * All levels of a stack in one pass (the correspondences are read once): sides_host[l] = cells per side of level l
  * (HOST array); maps = one buffer of B * sum(side_l^2) ints, level-major (level l starts at B * sum_{k<l} side_k^2,
- * inside it edit-major: B maps of side_l^2 cells). */
+ * inside it edit-major: B maps of side_l^2 cells).
+ * corr = B lists of corr_stride_rows rows; n_corr[e] above corr_stride_rows counts as corr_stride_rows.  Rows with a
+ * coordinate outside [0, img_res) are ignored. */
 int dh_dense_source_maps(const int64_t* corr, const int32_t* n_corr, int corr_stride_rows, const int32_t* winner_src,
                          int B, int img_res, const int* sides_host, int n_levels, int32_t* maps, void* stream);
 
@@ -215,7 +217,9 @@ int dh_dense_source_maps(const int64_t* corr, const int32_t* n_corr, int corr_st
  * The dense kernel stages 16 KB chunks of the source planes in shared memory with TMA bulk copies
  * (cp.async.bulk + mbarrier) and writes 128-bit rows.
  * Indices outside [0, hw) - negative or too large - give 0 and are never dereferenced (the reference's tensor indexing
- * would raise IndexError for them; a kernel cannot, so it stays memory safe instead). */
+ * would raise IndexError for them; a kernel cannot, so it stays memory safe instead).
+ * Pointers need only fp32 / int32 alignment; a level whose pointers are not 16-byte aligned takes the generic path.
+ * The dense form checks every level before its first launch, so a rejected call writes no output. */
 int dh_warp_gather_list(const float* in, int C, int hw, const int32_t* idx, int n, float* out, void* stream);
 int dh_warp_gather_dense(const dh_warp_level* levels_host, int n_levels, int B, void* stream);
 
